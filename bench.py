@@ -33,11 +33,15 @@ over 8 GPUs), outcomes drawn on the device (Philox4x32-10 + Box-Muller), 10
 leverages, WITH the 12 statistics per leverage and the growth-rate summaries
 (valid-run count, mean / median / 5th percentile) over all shards.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line.  `--impl reference` times the reference's own CPU
 implementation of the same path (torch-CPU port, all host threads) on a bounded
-sample of the same workload.
+sample of the same workload.  `--dump-outputs DIR` writes what the last timed step
+returned to its caller as DIR/<name>.npy (float64, non-finite entries 0) and
+DIR/<name>_nonfinite.npy (which entries were inf / nan): `stats` [G,12], and for
+`--workload gbm` also `growth`.  The inputs depend only on the arguments, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -220,6 +224,23 @@ class ClockSampler(threading.Thread):
             "note": "sampled every 5 ms from the last warm-up steps (same kernels, same load) to the end of the "
                     "timed region",
         }
+
+
+def dump_outputs(out_dir, **arrays):
+    """
+    --dump-outputs: each array as <out_dir>/<name>.npy in float64 with its non-finite entries set to 0, and
+    <name>_nonfinite.npy saying what stood there: 0 finite, 1 +inf, 2 -inf, 3 nan.  The statistics follow
+    the reference's fp32 arithmetic, so wealth that overflows fp32 turns means into inf and std_mean into nan;
+    split like this every file is finite and two runs compare entry by entry (nan never equals nan).
+    """
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        code = np.select([np.isposinf(a), np.isneginf(a), np.isnan(a)], [1.0, 2.0, 3.0], 0.0)
+        np.save(os.path.join(out_dir, name + ".npy"), np.where(code == 0, a, 0.0))
+        np.save(os.path.join(out_dir, name + "_nonfinite.npy"), code)
 
 
 def physical_gpu_index(local_rank):
@@ -496,6 +517,8 @@ def run_gpu(args):
     elapsed, sweep_s = _max_over_ranks(torch, dist, dev, world, [elapsed, sweep_s])
     value = n_total * h * args.steps / elapsed
     stats = stats_holder["s"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats=stats)
 
     # the other statistics path on the same outcomes, once: the two must agree
     other = engine.FinalSweepPipeline("discrete", table, V0, top_total, device=dev, group=group, n_total=n_total,
@@ -796,6 +819,8 @@ def run_gpu_gbm(args):
     value = n_total * h * args.steps / elapsed
     stats = holder["stats"].cpu().numpy()
     growth = holder["growth"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats=stats, growth=growth)
 
     # e2e: the entry point with Philox-drawn outcomes has no host input; the host-facing call is the on-disk
     # script contract (lev_scripts.gbm): statistics and growth summaries read back to the host every step
@@ -859,7 +884,7 @@ def run_gpu_gbm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 2000; 10 for --workload gbm)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="dice", choices=["dice", "gbm"],
@@ -883,9 +908,16 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the GBM-Philox / replay / collector side numbers")
     ap.add_argument("--cpu-sample", type=int, default=60_000, help="investors in the cpu_baseline sample")
     ap.add_argument("--ref-sample", type=int, default=4_000, help="investors per step of --impl reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
-    if args.workload == "gbm" and args.steps == 2000:
-        args.steps = 10          # a GBM step is ~100 ms
+    if args.steps is None:
+        args.steps = 10 if args.workload == "gbm" else 2000          # a GBM step is ~100 ms
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm sizes its sample from a timing probe: its inputs differ from run to run
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)

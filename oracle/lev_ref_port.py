@@ -12,8 +12,8 @@ the mean absolute deviation of the three groups - all torch CPU ops on all host
 threads, as the reference runs with VRAM=False (lev/dice_roll.py:63,137).
 
 Pinned against the unmodified reference in tests/test_oracle_ref_port.py
-(identical printed statistics on the same outcomes; runs where the reference
-tree is present).
+(identical printed statistics on the same outcomes as the reference's text in
+tests/golden/final_text.json).
 """
 import torch as T
 

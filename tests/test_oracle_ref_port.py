@@ -1,37 +1,35 @@
-"""The torch-CPU baseline port prints exactly what the unmodified reference prints."""
+"""The torch-CPU baseline port prints exactly what the unmodified reference prints
+(tests/golden/final_text.json, written by tests/golden/gen_golden_final_text.py)."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch as T
 
 import golden_io
 from oracle import lev_ref_port as port
-from oracle import ref_shim
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+FINAL_TEXT = os.path.join(golden_io.GOLDEN_DIR, "final_text.json")
 
 
-@pytest.mark.parametrize("name", ["coin_top7", "dice_top5", "dicesh_top3", "gbm_snp_top4"])
+@pytest.mark.parametrize("name", [c["name"] for c in golden_io.LEV_CASES])
 def test_port_prints_reference_text(name):
     case = golden_io.lev_case(name)
     oc = golden_io.draw_outcomes(case)
-    lx = ref_shim.load("lev.lev_exp")
-    dev, v0, top, grid = T.device("cpu"), T.tensor(case["v0"]), case["top"], case["grid"]
-    with ref_shim.quiet() as buf:
-        if case["kind"] == "coin":
-            t = T.tensor(oc.astype(np.float32))
-            lx.coin_fixed_final_lev(dev, t, top, v0, case["up_r"], case["down_r"], *grid)
-            rows, levs = port.fixed_final("coin", t, top, v0, (case["up_r"], case["down_r"]), grid)
-        elif case["kind"] == "dice":
-            t = T.tensor(oc.astype(np.int64))
-            lx.dice_fixed_final_lev(dev, t, top, v0, case["up_r"], case["down_r"], case["mid_r"], *grid)
-            rows, levs = port.fixed_final("dice", t, top, v0, (case["up_r"], case["down_r"], case["mid_r"]), grid)
-        elif case["kind"] == "dice_sh":
-            t = T.tensor(oc.astype(np.int64))
-            lx.dice_sh_fixed_final_lev(dev, t, top, v0, case["up_r"], case["down_r"], case["mid_r"], *case["sh"], *grid)
-            rows, levs = port.fixed_final("dice_sh", t, top, v0, (case["up_r"], case["down_r"], case["mid_r"]), grid,
-                                          sh=case["sh"])
-        else:
-            t = T.tensor(oc)
-            lx.gbm_fixed_final_lev(dev, t, top, v0, *grid)
-            rows, levs = port.fixed_final("gbm", t, top, v0, None, grid)
-    assert buf.getvalue().rstrip("\n") == port.format_rows(rows, levs)
+    want = json.load(open(FINAL_TEXT))[name]
+    v0, top, grid = T.tensor(case["v0"]), case["top"], case["grid"]
+    if case["kind"] == "coin":
+        t = T.tensor(oc.astype(np.float32))
+        rows, levs = port.fixed_final("coin", t, top, v0, (case["up_r"], case["down_r"]), grid)
+    elif case["kind"] == "dice":
+        t = T.tensor(oc.astype(np.int64))
+        rows, levs = port.fixed_final("dice", t, top, v0, (case["up_r"], case["down_r"], case["mid_r"]), grid)
+    elif case["kind"] == "dice_sh":
+        t = T.tensor(oc.astype(np.int64))
+        rows, levs = port.fixed_final("dice_sh", t, top, v0, (case["up_r"], case["down_r"], case["mid_r"]), grid,
+                                      sh=case["sh"])
+    else:
+        t = T.tensor(oc)
+        rows, levs = port.fixed_final("gbm", t, top, v0, None, grid)
+    assert want == port.format_rows(rows, levs)
