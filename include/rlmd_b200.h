@@ -120,6 +120,10 @@ typedef struct b200_lev_desc {
  * select kernel then takes two CTAs per leverage instead of six - slower alone (more bins per CTA), but it
  * leaves the sweep its SMs (measured at 2 GPUs, statistics beside the next sweep: 0.448 against 0.469 ms per step). */
 #define B200_LEV_FLAG_BESIDE_SWEEP 4
+/* b200_tally_stats: every grid point takes the radix route (three histogram levels over the fp32 key)
+ * instead of the log-wealth route - the route the kernel takes by itself for K = 4, non-finite log
+ * factors, or a grid point whose log-wealth bins fail a check.  For comparing the two. */
+#define B200_LEV_FLAG_RADIX_SELECT 8
 
 /*
  * outcomes : STREAM: uint8 [N,ld] (discrete, codes < K; or packed 2-bit codes,
@@ -220,7 +224,9 @@ int64_t b200_tally_exchange_bytes(const b200_tally_plan* plan);
  *   2 outcomes outside {0..K-1} met by b200_lev_ingest (dice: the reference would
  *     use such a value as the factor itself, lev/lev_exp.py:541; not supported)
  *   3 peer time-out (a rank's bins never arrived: statistics are NaN)
- *   4 sum of the bin counts seen by the last b200_tally_stats != n_total */
+ *   4 sum of the bin counts seen by the last b200_tally_stats != n_total
+ *   5 grid points whose statistics took the radix route (B200_LEV_FLAG_RADIX_SELECT)
+ *     since the last finalize */
 #define B200_TALLY_INFO_WORDS 8
 int b200_tally_reset(const b200_tally_plan* plan, void* workspace, void* stream);
 

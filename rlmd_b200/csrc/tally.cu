@@ -11,9 +11,11 @@
 //                             rank ends with the identical list
 //   statistics             -> wealth of every (grid point, tuple) with the count
 //                             kernels' own expressions (bit-identical data_T
-//                             values), then one block per grid point: weighted
-//                             3-level radix select (11+11+10 bits of the fp32 key)
-//                             for the four target ranks, exact top / rest split with
+//                             values), then one cluster per grid point: the four
+//                             target ranks from a histogram of log wealth and an
+//                             exact sort of one bin (checked; else a weighted 3-level
+//                             radix select, 11+11+10 bits of the fp32 key), exact
+//                             top / rest split with
 //                             tie apportioning, two-pass fp64 moments.  The block
 //                             owns its row: no atomics on fp64, so the result does
 //                             not depend on scheduling, only on the list order.
@@ -143,6 +145,27 @@ struct PeerView {
   uint32_t epoch;
 };
 
+// the (n_1, n_2) box of the keys a thread met, as the running maxima of TH_BOX_ACC
+__device__ __forceinline__ void box_add(uint32_t (&b)[4], unsigned long long key) {
+  int n1, n2, n3;
+  tally_unkey(key, n1, n2, n3);
+  b[0] = max(b[0], (uint32_t)(TALLY_MAX_HORIZON - n1)); b[1] = max(b[1], (uint32_t)n1);
+  b[2] = max(b[2], (uint32_t)(TALLY_MAX_HORIZON - n2)); b[3] = max(b[3], (uint32_t)n2);
+}
+// the block's maxima -> one global atomicMax per word into dst[0..3]; every thread of the block calls
+__device__ __forceinline__ void box_flush(const uint32_t (&b)[4], long long* dst, uint32_t* s /* shared [4] */) {
+  if (threadIdx.x < 4) s[threadIdx.x] = 0;
+  __syncthreads();
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const uint32_t m = __reduce_max_sync(0xffffffffu, b[q]);
+    if ((threadIdx.x & 31) == 0 && m != 0u) atomicMax(s + q, m);
+  }
+  __syncthreads();
+  if (threadIdx.x < 4 && s[threadIdx.x] != 0u)
+    atomicMax(reinterpret_cast<unsigned long long*>(dst) + threadIdx.x, (unsigned long long)s[threadIdx.x]);
+}
+
 constexpr int COMPACT_PER = 8;                    // slots per thread
 constexpr int COMPACT_CHUNK = 256 * COMPACT_PER;  // slots per block (the table holds a multiple: capacity >= 2048... see layout)
 
@@ -153,6 +176,8 @@ tally_compact_kernel(TallyDev t, unsigned long long* __restrict__ ukeys, uint32_
   __shared__ BinEntry stage[COMPACT_CHUNK];
   __shared__ int n_s;
   __shared__ long long base_s;
+  __shared__ uint32_t box_s[4];
+  uint32_t box[4] = {0, 0, 0, 0};
   const uint64_t cap = t.mask + 1;
   const uint64_t base = (uint64_t)blockIdx.x * COMPACT_CHUNK;
   if (threadIdx.x == 0) n_s = 0;
@@ -173,12 +198,14 @@ tally_compact_kernel(TallyDev t, unsigned long long* __restrict__ ukeys, uint32_
     const uint64_t i = base + (uint64_t)u * 256 + threadIdx.x;
     t.keys[i] = TALLY_EMPTY;
     t.counts[i] = 0;
+    if (!MULTI) box_add(box, key[u]);   // (across GPUs the merged list's box is taken by the unique kernel)
     const int p = atomicAdd(&n_s, 1);
     stage[p].key = key[u];
     stage[p].count = cnt[u];
   }
   __syncthreads();
   const int n = n_s;
+  if (!MULTI && n > 0) box_flush(box, t.header + TH_BOX_ACC, box_s);
   if (n > 0) {   // one reservation per block
     if (threadIdx.x == 0)
       base_s = (long long)atomicAdd(reinterpret_cast<unsigned long long*>(t.header + TH_LISTPOS), (unsigned long long)n);
@@ -211,7 +238,14 @@ tally_compact_kernel(TallyDev t, unsigned long long* __restrict__ ukeys, uint32_
     t.header[TH_LISTPOS] = 0;
     t.header[TH_TICKET] = 0;
     if (MULTI) *P.list_count[P.rank] = m;
-    else t.header[TH_NBINS] = m;
+    else {
+      t.header[TH_NBINS] = m;
+      t.header[TH_RADIX] = 0;
+      for (int q = 0; q < 4; ++q) {
+        t.header[TH_BOX + q] = *reinterpret_cast<volatile long long*>(t.header + TH_BOX_ACC + q);
+        t.header[TH_BOX_ACC + q] = 0;
+      }
+    }
   }
   if (MULTI) {
     __syncthreads();
@@ -271,7 +305,11 @@ tally_merge_kernel(const __grid_constant__ PeerView P, long long* __restrict__ h
   __syncthreads();
   long long total = off_s[P.world];
   if (total > concat_cap) total = concat_cap;   // cannot happen: every list is <= list_cap
-  if (blockIdx.x == 0 && threadIdx.x == 0) header[TH_CONCAT] = total;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    header[TH_CONCAT] = total;
+    header[TH_RADIX] = 0;
+    for (int q = 0; q < 4; ++q) header[TH_BOX + q] = 0;   // filled by tally_unique_kernel (stream order)
+  }
   // the part of table B this merge uses: a power of two >= 2 * total (every slot of B is empty between merges)
   uint64_t used = 1024;
   while (used < 2 * (uint64_t)total && used < capB) used <<= 1;
@@ -343,6 +381,8 @@ tally_unique_kernel(long long* __restrict__ header, const BinEntry* __restrict__
   __shared__ long long red[32];
   __shared__ long long warp_tot[8];
   __shared__ long long base_s;
+  __shared__ uint32_t box_s[4];
+  uint32_t box[4] = {0, 0, 0, 0};
   const long long total = header[TH_CONCAT];
   const long long nchunks = (total + MERGE_CHUNK - 1) / MERGE_CHUNK;
   if (total == 0 && blockIdx.x == 0 && threadIdx.x == 0) header[TH_NBINS] = 0;
@@ -389,6 +429,7 @@ tally_unique_kernel(long long* __restrict__ header, const BinEntry* __restrict__
       if (!rep[u]) continue;
       const long long p = base + (long long)threadIdx.x * PER + u;
       if (outp < bins_cap) {
+        box_add(box, concat[p].key);
         ukeys[outp] = concat[p].key;
         ucnt[outp] = (uint32_t)__ldcg(countsB + slot[u]);
       } else {
@@ -405,6 +446,7 @@ tally_unique_kernel(long long* __restrict__ header, const BinEntry* __restrict__
     }
     __syncthreads();
   }
+  box_flush(box, header + TH_BOX, box_s);
 }
 
 // ----------------------------------------------------------------- select
@@ -467,15 +509,27 @@ __device__ __forceinline__ void push_hist(uint32_t* mine, uint32_t* leaders, int
     }
 }
 
+// Log-wealth route: the candidates of a target (the bins of its log-wealth bin) in the leader's `hist`
+constexpr int CAND = 512;                           // per target; more sends the grid point to the radix route
+constexpr int CAND_CTA = 256;                       // per target and CTA; more counts as more than CAND
+
 struct SelShared {
-  uint32_t hist[4 * SL2];                 // leader: level 1 [0,2048); level 2: 4 x 2048; level 3: 4 x 1024
+  uint32_t hist[4 * SL2];                 // leader: level 1 [0,2048); level 2: 4 x 2048; level 3: 4 x 1024;
+                                          // log-wealth route: bin histogram, then candidates [key 4 x CAND |
+                                          // count 4 x CAND | the same sorted by (key, count)]
+  uint32_t ext[4][2];                     // leader, log-wealth route: max key below / min key above a target's bin
+  uint32_t ext_cta[4][2];                 // the same over this CTA's slice
+  uint32_t cand_cta[2][4][CAND_CTA];          // log-wealth route: this CTA's candidates (key, count) per target
+  int ncand_cta[4], base_cta[4];
+  uint32_t sel[4];                        // leader, log-wealth route: the targets' keys
+  int ncand[4], found[4], lat_ok;
   double part_d[SEL_MAX_CLUSTER][6];      // leader: the CTAs' partial sums of the running pass
-  long long part_i[SEL_MAX_CLUSTER][2];
+  long long part_i[SEL_MAX_CLUSTER][5];
   double res_d[4];                        // leader: mean_all, mean_top, mean_adj
   long long res_i[16];                    // leader: nonfinite[3], has_nan[3], ties_top, ties_adj, bins[4], rems[4]
   uint32_t warp_tot[32];
   double red_d[32];
-  double red_d2[32 * 6];
+  double red_d2[32 * 7];
   long long red_i[32];
 };
 
@@ -504,7 +558,8 @@ __global__ void __launch_bounds__(SEL_THREADS)
 tally_select_kernel(long long* __restrict__ header, const unsigned long long* __restrict__ ukeys,
                     const uint32_t* __restrict__ ucnt, float* __restrict__ wbuf, int64_t ldw, int32_t H,
                     const __grid_constant__ LogTable lf, double logV0, int64_t n_total, int64_t top,
-                    double* __restrict__ stats, int32_t SEL_CACHE /* bins per CTA kept in shared memory */) {
+                    double* __restrict__ stats, int32_t SEL_CACHE /* bins per CTA kept in shared memory */,
+                    int32_t force_radix) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   const int C = (int)cluster.num_blocks(), r = (int)cluster.block_rank();
@@ -512,6 +567,7 @@ tally_select_kernel(long long* __restrict__ header, const unsigned long long* __
   extern __shared__ __align__(16) uint8_t dyn[];
   float* cw = reinterpret_cast<float*>(dyn);                   // [SEL_CACHE] wealth of the slice's bins beyond the registers
   uint32_t* cc = reinterpret_cast<uint32_t*>(dyn) + SEL_CACHE; // [SEL_CACHE] their counts
+  uint16_t* cb = reinterpret_cast<uint16_t*>(cc + SEL_CACHE);  // [SEL_CACHE] their log-wealth bins
   SelShared* L = cluster.map_shared_rank(&sh, 0);              // the leader's copy
 
   const int g = blockIdx.x / C;
@@ -538,31 +594,79 @@ tally_select_kernel(long long* __restrict__ header, const unsigned long long* __
   float* __restrict__ w = wbuf + (int64_t)g * ldw + lo;      // spill space for bins beyond the shared-memory cache
   const uint32_t* __restrict__ cnt = ucnt + lo;
   constexpr int REGS = 0;
-  // The wealth of this grid point at every bin of the slice: the epilogue of the LOG count kernels
-  // (lev_sweep.cu) expression for expression, so a bin's wealth is bit-identical to the data_T entry of
-  // every investor in it.  It is formed once, here, and kept in shared memory for the four passes.
-  {
-    double lm[NK];
+  double lm[NK];
 #pragma unroll
-    for (int k = 0; k < NK; ++k) lm[k] = lf.lm[k][g];
-    for (int i = tid; i < m; i += SEL_THREADS) {
-      int n1, n2, n3;
-      tally_unkey(__ldg(ukeys + lo + i), n1, n2, n3);
-      int nk[4];
-      nk[1] = n1; nk[2] = NK >= 3 ? n2 : 0; nk[3] = NK >= 4 ? n3 : 0;
-      nk[0] = H - nk[1] - nk[2] - nk[3];
-      double lw = logV0;
+  for (int k = 0; k < NK; ++k) lm[k] = lf.lm[k][g];
+  // The log wealth of a bin: the epilogue of the LOG count kernels (lev_sweep.cu) expression for expression,
+  // so fl32(exp(lw)) is bit-identical to the data_T entry of every investor in the bin.
+  auto lw_of = [&](unsigned long long key) {
+    int n1, n2, n3;
+    tally_unkey(key, n1, n2, n3);
+    int nk[4];
+    nk[1] = n1; nk[2] = NK >= 3 ? n2 : 0; nk[3] = NK >= 4 ? n3 : 0;
+    nk[0] = H - nk[1] - nk[2] - nk[3];
+    double lw = logV0;
 #pragma unroll
-      for (int k = 0; k < NK; ++k)
-        if (nk[k] > 0) lw += (double)nk[k] * lm[k];
-      const float x = (float)exp(lw);
-      if (i < SEL_CACHE) { cw[i] = x; cc[i] = __ldg(cnt + i); }
-      else w[i] = x;
+    for (int k = 0; k < NK; ++k)
+      if (nk[k] > 0) lw += (double)nk[k] * lm[k];
+    return lw;
+  };
+  // Log-wealth route (K <= 3, finite log factors): log wealth is linear in the count tuple, so over the
+  // (n_1, n_2) box of the list it lies between the values at the box's corners.  SL1 equal bins of log wealth
+  // over that range take the place of the radix levels: fl32(exp(.)) is monotone, so the bins are ordered by
+  // wealth and a target lies in ONE bin of a few dozen tuples, which the leader then sorts exactly.  Every
+  // step is checked on the fp32 values; a grid point that fails a check takes the radix route.
+  bool lat = false;
+  double lw_lo = 0.0, lw_scale = 0.0;
+  if (NK <= 3 && !force_radix) {
+    const long long M = TALLY_MAX_HORIZON;
+    const long long a[2] = {M - header[TH_BOX + 0], header[TH_BOX + 1]}, b[2] = {M - header[TH_BOX + 2], header[TH_BOX + 3]};
+    bool fin = a[0] <= a[1] && b[0] <= b[1];
+#pragma unroll
+    for (int k = 0; k < NK; ++k) fin = fin && isfinite(lm[k]);
+    if (fin) {
+      double lo_ = INFINITY, hi_ = -INFINITY;
+      for (int u = 0; u < 4; ++u) {
+        const double n1 = (double)a[u & 1], n2 = NK >= 3 ? (double)b[u >> 1] : 0.0;
+        double v = logV0 + ((double)H - n1 - n2) * lm[0] + n1 * lm[1];
+        if (NK >= 3) v += n2 * lm[NK >= 3 ? 2 : 0];
+        lo_ = fmin(lo_, v);
+        hi_ = fmax(hi_, v);
+      }
+      if (hi_ > lo_ && isfinite(hi_ - lo_)) { lat = true; lw_lo = lo_; lw_scale = (double)SL1 / (hi_ - lo_); }
+    }
+  }
+  auto lw_bin = [&](double lw) -> uint32_t {   // monotone in lw; out-of-range rounding is clamped
+    const double t = (lw - lw_lo) * lw_scale;
+    return t >= (double)(SL1 - 1) ? (uint32_t)(SL1 - 1) : t > 0.0 ? (uint32_t)t : 0u;
+  };
+  if (lat) {
+    for (int i = tid; i < SL1; i += SEL_THREADS) sh.hist[i] = 0;
+    cluster.sync();
+  }
+  // The wealth of this grid point at every bin of the slice, formed once and kept in shared memory for the
+  // passes; on the log-wealth route the loop also takes pass 0's sums and the bin histogram.
+  double a0 = 0;
+  long long c0 = 0, pinf = 0;
+  for (int i = tid; i < m; i += SEL_THREADS) {
+    const double lw = lw_of(__ldg(ukeys + lo + i));
+    const float x = (float)exp(lw);
+    const uint32_t c = __ldg(cnt + i);
+    if (i < SEL_CACHE) { cw[i] = x; cc[i] = c; }
+    else w[i] = x;
+    if (lat) {
+      const uint32_t bn = lw_bin(lw);
+      if (i < SEL_CACHE) cb[i] = (uint16_t)bn;
+      atomicAdd(sh.hist + bn, c);
+      a0 += (double)c * (double)x;
+      c0 += c;
+      if (isinf(x)) pinf += c;
     }
   }
   __syncthreads();
   auto far_w = [&](int i) { return i < REGS + SEL_CACHE ? cw[i - REGS] : w[i]; };
   auto far_c = [&](int i) { return i < REGS + SEL_CACHE ? cc[i - REGS] : cnt[i]; };
+  auto far_b = [&](int i) { return i < SEL_CACHE ? (uint32_t)cb[i] : lw_bin(lw_of(__ldg(ukeys + lo + i))); };
   // f(x, c, in): called by every lane of a warp together (`in` = this lane holds an element)
   auto sweep = [&](auto&& f) {
     for (int base = (tid & ~31); base < m; base += SEL_THREADS) {
@@ -571,187 +675,397 @@ tally_select_kernel(long long* __restrict__ header, const unsigned long long* __
       f(in ? far_w(i) : 0.f, in ? far_c(i) : 0u, in);
     }
   };
+  const long long ranks[4] = {(n - 1) / 2, n - K, n - K + (K - 1) / 2, (n - K - 1) / 2};
+  uint32_t key_j[4];
+  bool radix = !lat;
 
-  // ---- pass 0: sum, count, level-1 histogram
-  for (int i = tid; i < SL1; i += SEL_THREADS) sh.hist[i] = 0;
-  cluster.sync();
-  STAMP();
-  {
-    double a0 = 0;
-    long long c0 = 0;
-    sweep([&](float x, uint32_t c, bool in) {
-      a0 += (double)c * (double)x;      // c = 0 where the lane holds nothing
-      c0 += c;
-      warp_hist_add(sh.hist, float_key(x) >> 21, c, in);
-    });
+  if (lat) {
     STAMP();
+    // ---- pass 0: sums and the log-wealth histogram are in; the leader finds the targets' bins
     push_hist(sh.hist, L->hist, SL1, r);
-    a0 = block_sum(a0, sh.red_d);
-    c0 = block_sum(c0, sh.red_i);
-    if (tid == 0) { L->part_d[r][0] = a0; L->part_i[r][0] = c0; }
-  }
-  cluster.sync();
-  STAMP();
-  if (r == 0) {
-    if (tid == 0) {
-      double sum_all = 0;
-      long long cnt_all = 0;
-      for (int q = 0; q < C; ++q) { sum_all += sh.part_d[q][0]; cnt_all += sh.part_i[q][0]; }
-      if (cnt_all != n) header[TH_MISMATCH] = 1;
-      // key bins that can only hold non-finite values: 3 = -inf, 2044 = +inf, 2047 = NaN
-      const long long ninf = sh.hist[3], pinf = sh.hist[2044], nan = sh.hist[2047];
-      const long long hi_ = pinf + nan;
-      sh.res_i[0] = (hi_ + ninf) > 0; sh.res_i[1] = hi_ > 0 || ninf > n - K; sh.res_i[2] = hi_ > K || ninf > 0;
-      sh.res_i[3] = nan > 0; sh.res_i[4] = nan > 0; sh.res_i[5] = nan > K;
-      sh.res_d[0] = sum_all / (double)n;
+    {
+      double v[3] = {a0, (double)c0, (double)pinf};   // (counts < 2^32: exact in fp64)
+      block_sum_n<3>(v, sh.red_d2);
+      if (tid == 0) { L->part_d[r][0] = v[0]; L->part_i[r][0] = (long long)v[1]; L->part_i[r][1] = (long long)v[2]; }
     }
-    scan_hists(sh.hist, SL1, 1, sh.warp_tot);   // (thread 0's reads above precede the scan's first barrier)
-    if (tid < 4) {
-      const long long ranks[4] = {(n - 1) / 2, n - K, n - K + (K - 1) / 2, (n - K - 1) / 2};
-      int bin; long long rem;
-      find_rank(sh.hist, SL1, ranks[tid], bin, rem);
-      sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+    if (tid < 4) { sh.ext_cta[tid][0] = 0u; sh.ext_cta[tid][1] = 0xffffffffu; sh.ncand_cta[tid] = 0; }
+    cluster.sync();
+    STAMP();
+    if (r == 0) {
+      if (tid == 0) {
+        double sum_all = 0;
+        long long cnt_all = 0, inf_all = 0;
+        for (int q = 0; q < C; ++q) { sum_all += sh.part_d[q][0]; cnt_all += sh.part_i[q][0]; inf_all += sh.part_i[q][1]; }
+        if (cnt_all != n) header[TH_MISMATCH] = 1;
+        // finite log factors: no NaN and no -inf wealth, +inf where exp overflows fp32
+        sh.res_i[0] = inf_all > 0; sh.res_i[1] = inf_all > 0; sh.res_i[2] = inf_all > K;
+        sh.res_i[3] = 0; sh.res_i[4] = 0; sh.res_i[5] = 0;
+        sh.res_d[0] = sum_all / (double)n;
+      }
+      if (tid < 4) { sh.ncand[tid] = 0; sh.found[tid] = 0; sh.ext[tid][0] = 0u; sh.ext[tid][1] = 0xffffffffu; }
+      scan_hists(sh.hist, SL1, 1, sh.warp_tot);
+      if (tid < 4) {
+        int bin; long long rem;
+        find_rank(sh.hist, SL1, ranks[tid], bin, rem);
+        sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+      }
     }
-  }
-  cluster.sync();
-  uint32_t pre[4];
-  long long rk[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) { pre[j] = (uint32_t)L->res_i[8 + j]; rk[j] = L->res_i[12 + j]; }
-  const double mean_a = L->res_d[0];
-  STAMP();
-  // targets that share a prefix share a histogram: only the first of them (its representative) is counted,
-  // the leader copies it for the others before it scans
-  int rep[4];
-  auto find_reps = [&]() {
+    cluster.sync();
+    STAMP();
+    // ---- gather: the tuples of the targets' bins go to the leader (once per distinct bin: targets that share
+    // a bin share its list); the sums on either side of thr's bin and the extreme keys on either side of every
+    // target's bin are taken on the way
+    int bq[4], rep[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
+      bq[j] = (int)L->res_i[8 + j];
       rep[j] = j;
 #pragma unroll
       for (int q = 3; q >= 0; --q)
-        if (q < j && pre[q] == pre[j]) rep[j] = q;
+        if (q < j && bq[q] == bq[j]) rep[j] = q;
     }
-  };
-  auto copy_reps = [&](int bins) {     // leader only
-    for (int j = 1; j < 4; ++j)
-      if (rep[j] != j)
-        for (int i = tid; i < bins; i += SEL_THREADS) sh.hist[j * bins + i] = sh.hist[rep[j] * bins + i];
-    __syncthreads();
-  };
-  find_reps();
+    {
+      // beside thr's bin the saturated values (+inf, 0) are counted apart: they are thr's ties if thr is one
+      double v[7] = {0, 0, 0, 0, 0, 0, 0};   // sum > , sum < thr's bin; count >; +inf >, 0 >, +inf <, 0 <
+      uint32_t ext_lo[4] = {0u, 0u, 0u, 0u}, ext_hi[4] = {~0u, ~0u, ~0u, ~0u};
+      for (int i = tid; i < m; i += SEL_THREADS) {
+        const int bn = (int)far_b(i);
+        const float x = far_w(i);
+        const uint32_t c = far_c(i), k = float_key(x);
+        if (bn > bq[1]) {
+          if (isinf(x)) v[3] += (double)c;
+          else if (x == 0.f) v[4] += (double)c;
+          else { v[0] += (double)c * (double)x; v[2] += (double)c; }
+        } else if (bn < bq[1]) {
+          if (isinf(x)) v[5] += (double)c;
+          else if (x == 0.f) v[6] += (double)c;
+          else v[1] += (double)c * (double)x;
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          if (bn < bq[j]) ext_lo[j] = max(ext_lo[j], k);
+          else if (bn > bq[j]) ext_hi[j] = min(ext_hi[j], k);
+          else if (rep[j] == j) {
+            const int p = atomicAdd(&sh.ncand_cta[j], 1);
+            if (p < CAND_CTA) { sh.cand_cta[0][j][p] = k; sh.cand_cta[1][j][p] = c; }
+          }
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const uint32_t a = __reduce_max_sync(0xffffffffu, ext_lo[j]), b = __reduce_min_sync(0xffffffffu, ext_hi[j]);
+        if (lane == 0) { atomicMax(&sh.ext_cta[j][0], a); atomicMin(&sh.ext_cta[j][1], b); }
+      }
+      STAMP();
+      block_sum_n<7>(v, sh.red_d2);      // (its barriers also close this CTA's extremes)
+      if (tid == 0) {
+        L->part_d[r][0] = v[0]; L->part_d[r][1] = v[1];
+#pragma unroll
+        for (int q = 0; q < 5; ++q) L->part_i[r][q] = (long long)v[2 + q];
+      }
+      if (tid < 8) {
+        const int j = tid >> 1;
+        if (tid & 1) atomicMin(&L->ext[j][1], sh.ext_cta[j][1]);
+        else atomicMax(&L->ext[j][0], sh.ext_cta[j][0]);
+      }
+      // one reservation per CTA and list in the leader's lists, then plain remote stores
+      if (tid < 4 && rep[tid] == tid)
+        sh.base_cta[tid] = atomicAdd(&L->ncand[tid], sh.ncand_cta[tid] <= CAND_CTA ? sh.ncand_cta[tid] : CAND + 1);
+      __syncthreads();
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        if (rep[j] != j) continue;
+        const int nl = min(sh.ncand_cta[j], CAND_CTA), b0 = sh.base_cta[j];
+        for (int p = tid; p < nl && b0 + p < CAND; p += SEL_THREADS) {
+          L->hist[j * CAND + b0 + p] = sh.cand_cta[0][j][p];
+          L->hist[4 * CAND + j * CAND + b0 + p] = sh.cand_cta[1][j][p];
+        }
+      }
+    }
+    cluster.sync();
+    STAMP();
+    if (r == 0) {
+      // The candidates of every distinct bin in (key, count) order, eight lanes per candidate: a target is the
+      // key whose run of weights covers the rank left inside its bin, and the sums over the sorted copy do not
+      // depend on the order in which the CTAs appended them.
+      int mq[4], off[5];
+      off[0] = 0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) { mq[j] = rep[j] == j ? min(sh.ncand[j], CAND) : 0; off[j + 1] = off[j] + mq[j]; }
+      const int gi = tid >> 3, sub = tid & 7;
+      for (int c0 = 0; c0 < off[4]; c0 += SEL_THREADS / 8) {     // the same trip count for every thread
+        const int idx = c0 + gi;
+        const bool in = idx < off[4];
+        int j = 0, oj = 0, mj = mq[0], pos = 0;   // the list of candidate idx (the last with off <= idx: not empty)
+#pragma unroll
+        for (int q = 1; q < 4; ++q)
+          if (idx >= off[q]) { j = q; oj = off[q]; mj = mq[q]; }
+        const int t = idx - oj;
+        uint32_t kt = 0, ct = 0;
+        long long below = 0, eq = 0;
+        if (in) {
+          const uint32_t* ck = sh.hist + j * CAND;
+          const uint32_t* ccn = sh.hist + 4 * CAND + j * CAND;
+          kt = ck[t]; ct = ccn[t];
+          for (int u = sub; u < mj; u += 8) {
+            const uint32_t ku = ck[u], cu = ccn[u];
+            if (ku < kt) below += cu;
+            else if (ku == kt) eq += cu;
+            pos += ku < kt || (ku == kt && (cu < ct || (cu == ct && u < t)));
+          }
+        }
+#pragma unroll
+        for (int o = 4; o > 0; o >>= 1) {
+          below += __shfl_xor_sync(0xffffffffu, below, o);
+          eq += __shfl_xor_sync(0xffffffffu, eq, o);
+          pos += __shfl_xor_sync(0xffffffffu, pos, o);
+        }
+        if (in && sub == 0) {
+          sh.hist[8 * CAND + j * CAND + pos] = kt;
+          sh.hist[12 * CAND + j * CAND + pos] = ct;
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            const long long rem = sh.res_i[12 + q];
+            if (rep[q] == j && below <= rem && rem < below + eq) { sh.sel[q] = kt; sh.found[q] = 1; }   // (ties write the same)
+          }
+        }
+      }
+      __syncthreads();
+      // thr's bin: the exact split of its tuples, as in the radix route's last level
+      const uint32_t thr_key = sh.sel[1];
+      const int m1 = rep[1] == 0 ? mq[0] : mq[1];
+      double f[5] = {0, 0, 0, 0, 0};      // sum > thr, sum < thr, count > thr, count < thr, count of the bin
+      for (int t = tid; t < m1; t += SEL_THREADS) {
+        const uint32_t k = sh.hist[8 * CAND + rep[1] * CAND + t];
+        const long long c = sh.hist[12 * CAND + rep[1] * CAND + t];
+        f[4] += (double)c;
+        if (k == thr_key) continue;
+        const double val = (double)c * (double)key_float(k);
+        if (k > thr_key) { f[0] += val; f[2] += (double)c; } else { f[1] += val; f[3] += (double)c; }
+      }
+      block_sum_n<5>(f, sh.red_d2);
+      if (tid == 0) {
+        // The bins are ordered by wealth if no key below a target's bin exceeds the target and none above it
+        // falls short.  thr's neighbours must be strictly apart (the sums beside its bin were taken as > thr /
+        // < thr) unless thr is a saturated value, whose copies beside its bin were counted apart.
+        constexpr uint32_t KEY_ZERO = 0x80000000u, KEY_INF = 0xff800000u;
+        const bool t_inf = thr_key == KEY_INF, t_zero = thr_key == KEY_ZERO;
+        bool ok = true;
+        for (int j = 0; j < 4; ++j)
+          ok = ok && sh.ncand[rep[j]] <= CAND && sh.found[j] && sh.ext[j][0] <= sh.sel[j] && sh.sel[j] <= sh.ext[j][1];
+        ok = ok && (t_inf || t_zero || (sh.ext[1][0] < thr_key && thr_key < sh.ext[1][1]));
+        sh.lat_ok = ok;
+        if (ok) {
+          const long long fc_gt = (long long)f[2], fc_lt = (long long)f[3], fc_all = (long long)f[4];
+          double coarse_gt = 0, coarse_lt = 0;
+          long long cnt_gt = 0, sat[4] = {0, 0, 0, 0};   // +inf above, 0 above, +inf below, 0 below
+          for (int q = 0; q < C; ++q) {
+            coarse_gt += sh.part_d[q][0]; coarse_lt += sh.part_d[q][1];
+            cnt_gt += sh.part_i[q][0];
+            for (int u = 0; u < 4; ++u) sat[u] += sh.part_i[q][1 + u];
+          }
+          const double thr = (double)key_float(thr_key);
+          const long long below = n - cnt_gt - sat[0] - sat[1] - fc_all;   // investors in the bins under thr's
+          const long long n_gt = cnt_gt + (t_inf ? 0 : sat[0]) + (t_zero ? 0 : sat[1]) + fc_gt;
+          const long long n_lt = below - (t_inf ? sat[2] : 0) - (t_zero ? sat[3] : 0) + fc_lt;
+          if (!t_inf && sat[0] > 0) coarse_gt += INFINITY;
+          const double sum_gt = fc_gt ? coarse_gt + f[0] : coarse_gt, sum_lt = fc_lt ? coarse_lt + f[1] : coarse_lt;
+          const long long n_eq = n - n_gt - n_lt;
+          const long long tt = K - n_gt;
+          sh.res_i[6] = tt;
+          sh.res_i[7] = n_eq - tt;
+          sh.res_d[1] = (sum_gt + (tt > 0 ? (double)tt * thr : 0.0)) / (double)K;
+          sh.res_d[2] = (sum_lt + (n_eq - tt > 0 ? (double)(n_eq - tt) * thr : 0.0)) / (double)(n - K);
+        }
+      }
+    }
+    cluster.sync();
+    STAMP();
+    radix = !L->lat_ok;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) key_j[j] = L->sel[j];
+  }
 
-  // ---- pass 1: level-2 histograms of the elements in the targets' level-1 bins
-  // (the leader next writes its results after the barrier that ends the pass: every read above is done by then)
-  for (int j = 0; j < 4; ++j)
-    if (rep[j] == j)
-      for (int i = tid; i < SL2; i += SEL_THREADS) sh.hist[j * SL2 + i] = 0;
-  cluster.sync();
-  {
-    sweep([&](float x, uint32_t c, bool in) {
-      const uint32_t k = float_key(x);
-      const uint32_t b1 = k >> 21, b2 = (k >> 10) & (SL2 - 1);
+  if (radix) {
+    if (r == 0 && tid == 0) atomicAdd(reinterpret_cast<unsigned long long*>(header + TH_RADIX), 1ull);
+    // ---- pass 0: sum, count, level-1 histogram
+    for (int i = tid; i < SL1; i += SEL_THREADS) sh.hist[i] = 0;
+    cluster.sync();
+    STAMP();
+    {
+      a0 = 0;
+      c0 = 0;
+      sweep([&](float x, uint32_t c, bool in) {
+        a0 += (double)c * (double)x;      // c = 0 where the lane holds nothing
+        c0 += c;
+        warp_hist_add(sh.hist, float_key(x) >> 21, c, in);
+      });
+      STAMP();
+      push_hist(sh.hist, L->hist, SL1, r);
+      a0 = block_sum(a0, sh.red_d);
+      c0 = block_sum(c0, sh.red_i);
+      if (tid == 0) { L->part_d[r][0] = a0; L->part_i[r][0] = c0; }
+    }
+    cluster.sync();
+    STAMP();
+    if (r == 0) {
+      if (tid == 0) {
+        double sum_all = 0;
+        long long cnt_all = 0;
+        for (int q = 0; q < C; ++q) { sum_all += sh.part_d[q][0]; cnt_all += sh.part_i[q][0]; }
+        if (cnt_all != n) header[TH_MISMATCH] = 1;
+        // key bins that can only hold non-finite values: 3 = -inf, 2044 = +inf, 2047 = NaN
+        const long long ninf = sh.hist[3], pinf = sh.hist[2044], nan = sh.hist[2047];
+        const long long hi_ = pinf + nan;
+        sh.res_i[0] = (hi_ + ninf) > 0; sh.res_i[1] = hi_ > 0 || ninf > n - K; sh.res_i[2] = hi_ > K || ninf > 0;
+        sh.res_i[3] = nan > 0; sh.res_i[4] = nan > 0; sh.res_i[5] = nan > K;
+        sh.res_d[0] = sum_all / (double)n;
+      }
+      scan_hists(sh.hist, SL1, 1, sh.warp_tot);   // (thread 0's reads above precede the scan's first barrier)
+      if (tid < 4) {
+        int bin; long long rem;
+        find_rank(sh.hist, SL1, ranks[tid], bin, rem);
+        sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+      }
+    }
+    cluster.sync();
+    uint32_t pre[4];
+    long long rk[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { pre[j] = (uint32_t)L->res_i[8 + j]; rk[j] = L->res_i[12 + j]; }
+    STAMP();
+    // targets that share a prefix share a histogram: only the first of them (its representative) is counted,
+    // the leader copies it for the others before it scans
+    int rep[4];
+    auto find_reps = [&]() {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        rep[j] = j;
+#pragma unroll
+        for (int q = 3; q >= 0; --q)
+          if (q < j && pre[q] == pre[j]) rep[j] = q;
+      }
+    };
+    auto copy_reps = [&](int bins) {     // leader only
+      for (int j = 1; j < 4; ++j)
+        if (rep[j] != j)
+          for (int i = tid; i < bins; i += SEL_THREADS) sh.hist[j * bins + i] = sh.hist[rep[j] * bins + i];
+      __syncthreads();
+    };
+    find_reps();
+
+    // ---- pass 1: level-2 histograms of the elements in the targets' level-1 bins
+    // (the leader next writes its results after the barrier that ends the pass: every read above is done by then)
+    for (int j = 0; j < 4; ++j)
+      if (rep[j] == j)
+        for (int i = tid; i < SL2; i += SEL_THREADS) sh.hist[j * SL2 + i] = 0;
+    cluster.sync();
+    {
+      sweep([&](float x, uint32_t c, bool in) {
+        const uint32_t k = float_key(x);
+        const uint32_t b1 = k >> 21, b2 = (k >> 10) & (SL2 - 1);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (rep[j] == j) warp_hist_add(sh.hist + j * SL2, b2, c, in && b1 == pre[j]);     // (rep is warp-uniform)
+      });
+      STAMP();
 #pragma unroll
       for (int j = 0; j < 4; ++j)
-        if (rep[j] == j) warp_hist_add(sh.hist + j * SL2, b2, c, in && b1 == pre[j]);     // (rep is warp-uniform)
-    });
-    STAMP();
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-      if (rep[j] == j) push_hist(sh.hist + j * SL2, L->hist + j * SL2, SL2, r);
-  }
-  STAMP();
-  cluster.sync();
-  STAMP();
-  if (r == 0) {
-    copy_reps(SL2);
-    scan_hists(sh.hist, SL2, 4, sh.warp_tot);
-    if (tid < 4) {
-      int bin; long long rem;
-      find_rank(sh.hist + tid * SL2, SL2, rk[tid], bin, rem);
-      sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+        if (rep[j] == j) push_hist(sh.hist + j * SL2, L->hist + j * SL2, SL2, r);
     }
-  }
-  cluster.sync();
+    STAMP();
+    cluster.sync();
+    STAMP();
+    if (r == 0) {
+      copy_reps(SL2);
+      scan_hists(sh.hist, SL2, 4, sh.warp_tot);
+      if (tid < 4) {
+        int bin; long long rem;
+        find_rank(sh.hist + tid * SL2, SL2, rk[tid], bin, rem);
+        sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+      }
+    }
+    cluster.sync();
 #pragma unroll
-  for (int j = 0; j < 4; ++j) { pre[j] = (pre[j] << 11) | (uint32_t)L->res_i[8 + j]; rk[j] = L->res_i[12 + j]; }   // 22 bits
-  find_reps();
-  STAMP();
+    for (int j = 0; j < 4; ++j) { pre[j] = (pre[j] << 11) | (uint32_t)L->res_i[8 + j]; rk[j] = L->res_i[12 + j]; }   // 22 bits
+    find_reps();
+    STAMP();
 
-  // ---- pass 2: level-3 histograms + the sums on either side of thr's 22-bit prefix
-  for (int j = 0; j < 4; ++j)
-    if (rep[j] == j)
-      for (int i = tid; i < SL3; i += SEL_THREADS) sh.hist[j * SL3 + i] = 0;
-  cluster.sync();
-  const uint32_t thr22 = pre[1];
-  {
-    double v[2] = {0, 0};
-    long long c_gt = 0;
-    sweep([&](float x, uint32_t c, bool in) {
-      const uint32_t k = float_key(x);
-      const uint32_t hi22 = k >> 10;
-      const double cx = (double)c * (double)x;
-      if (in && hi22 > thr22) { v[0] += cx; c_gt += c; }
-      else if (in && hi22 < thr22) v[1] += cx;
+    // ---- pass 2: level-3 histograms + the sums on either side of thr's 22-bit prefix
+    for (int j = 0; j < 4; ++j)
+      if (rep[j] == j)
+        for (int i = tid; i < SL3; i += SEL_THREADS) sh.hist[j * SL3 + i] = 0;
+    cluster.sync();
+    const uint32_t thr22 = pre[1];
+    {
+      double v[2] = {0, 0};
+      long long c_gt = 0;
+      sweep([&](float x, uint32_t c, bool in) {
+        const uint32_t k = float_key(x);
+        const uint32_t hi22 = k >> 10;
+        const double cx = (double)c * (double)x;
+        if (in && hi22 > thr22) { v[0] += cx; c_gt += c; }
+        else if (in && hi22 < thr22) v[1] += cx;
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (rep[j] == j) warp_hist_add(sh.hist + j * SL3, k & (SL3 - 1), c, in && hi22 == pre[j]);
+      });
+      STAMP();
 #pragma unroll
       for (int j = 0; j < 4; ++j)
-        if (rep[j] == j) warp_hist_add(sh.hist + j * SL3, k & (SL3 - 1), c, in && hi22 == pre[j]);
-    });
-    STAMP();
+        if (rep[j] == j) push_hist(sh.hist + j * SL3, L->hist + j * SL3, SL3, r);
+      STAMP();
+      block_sum_n<2>(v, sh.red_d2);
+      c_gt = block_sum(c_gt, sh.red_i);
+      if (tid == 0) { L->part_d[r][0] = v[0]; L->part_d[r][1] = v[1]; L->part_i[r][0] = c_gt; }
+    }
+    cluster.sync();
+    if (r == 0) {
+      // thr's level-3 histogram: bin `b3` holds the copies of the ONE fp32 value with key (prefix22 << 10 | b3).
+      // The scan overwrites the counts with prefixes; the per-bin counts are read back as differences.
+      copy_reps(SL3);
+      scan_hists(sh.hist, SL3, 4, sh.warp_tot);
+      if (tid < 4) {
+        int bin; long long rem;
+        find_rank(sh.hist + tid * SL3, SL3, rk[tid], bin, rem);
+        sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
+      }
+      __syncthreads();
+      const uint32_t thr_key = (pre[1] << 10) | (uint32_t)sh.res_i[8 + 1];
+      const uint32_t thr_lo = thr_key & (SL3 - 1), base = thr_key & ~(uint32_t)(SL3 - 1);
+      double f[5] = {0, 0, 0, 0, 0};      // sum > thr, sum < thr, count > thr, count < thr, count of the whole histogram
+      const uint32_t* h3 = sh.hist + 1 * SL3;
+      for (uint32_t b3 = tid; b3 < (uint32_t)SL3; b3 += SEL_THREADS) {
+        const long long c = (long long)h3[b3] - (b3 > 0 ? (long long)h3[b3 - 1] : 0);
+        f[4] += (double)c;                  // counts < 2^32: exact in fp64
+        if (c == 0 || b3 == thr_lo) continue;   // an empty bin must not contribute 0 * inf
+        const double val = (double)c * (double)key_float(base | b3);
+        if (b3 > thr_lo) { f[0] += val; f[2] += (double)c; } else { f[1] += val; f[3] += (double)c; }
+      }
+      block_sum_n<5>(f, sh.red_d2);
+      if (tid == 0) {
+        const long long fc_gt = (long long)f[2], fc_lt = (long long)f[3], fc_all = (long long)f[4];
+        double coarse_gt = 0, coarse_lt = 0;
+        long long cnt_gt = 0;
+        for (int q = 0; q < C; ++q) { coarse_gt += sh.part_d[q][0]; coarse_lt += sh.part_d[q][1]; cnt_gt += sh.part_i[q][0]; }
+        const double thr = (double)key_float(thr_key);
+        const long long n_gt = cnt_gt + fc_gt, n_lt = (n - cnt_gt - fc_all) + fc_lt;
+        const double sum_gt = fc_gt ? coarse_gt + f[0] : coarse_gt, sum_lt = fc_lt ? coarse_lt + f[1] : coarse_lt;
+        const long long n_eq = n - n_gt - n_lt;
+        const long long tt = K - n_gt;   // ties that belong to the top group
+        sh.res_i[6] = tt;
+        sh.res_i[7] = n_eq - tt;
+        sh.res_d[1] = (sum_gt + (tt > 0 ? (double)tt * thr : 0.0)) / (double)K;                       // mean_top
+        sh.res_d[2] = (sum_lt + (n_eq - tt > 0 ? (double)(n_eq - tt) * thr : 0.0)) / (double)(n - K);   // mean_adj
+      }
+    }
+    cluster.sync();
 #pragma unroll
-    for (int j = 0; j < 4; ++j)
-      if (rep[j] == j) push_hist(sh.hist + j * SL3, L->hist + j * SL3, SL3, r);
+    for (int j = 0; j < 4; ++j) key_j[j] = (pre[j] << 10) | (uint32_t)L->res_i[8 + j];
     STAMP();
-    block_sum_n<2>(v, sh.red_d2);
-    c_gt = block_sum(c_gt, sh.red_i);
-    if (tid == 0) { L->part_d[r][0] = v[0]; L->part_d[r][1] = v[1]; L->part_i[r][0] = c_gt; }
   }
-  cluster.sync();
-  if (r == 0) {
-    // thr's level-3 histogram: bin `b3` holds the copies of the ONE fp32 value with key (prefix22 << 10 | b3).
-    // The scan overwrites the counts with prefixes; the per-bin counts are read back as differences.
-    copy_reps(SL3);
-    scan_hists(sh.hist, SL3, 4, sh.warp_tot);
-    if (tid < 4) {
-      int bin; long long rem;
-      find_rank(sh.hist + tid * SL3, SL3, rk[tid], bin, rem);
-      sh.res_i[8 + tid] = bin; sh.res_i[12 + tid] = rem;
-    }
-    __syncthreads();
-    const uint32_t thr_key = (pre[1] << 10) | (uint32_t)sh.res_i[8 + 1];
-    const uint32_t thr_lo = thr_key & (SL3 - 1), base = thr_key & ~(uint32_t)(SL3 - 1);
-    double f[5] = {0, 0, 0, 0, 0};      // sum > thr, sum < thr, count > thr, count < thr, count of the whole histogram
-    const uint32_t* h3 = sh.hist + 1 * SL3;
-    for (uint32_t b3 = tid; b3 < (uint32_t)SL3; b3 += SEL_THREADS) {
-      const long long c = (long long)h3[b3] - (b3 > 0 ? (long long)h3[b3 - 1] : 0);
-      f[4] += (double)c;                  // counts < 2^32: exact in fp64
-      if (c == 0 || b3 == thr_lo) continue;   // an empty bin must not contribute 0 * inf
-      const double val = (double)c * (double)key_float(base | b3);
-      if (b3 > thr_lo) { f[0] += val; f[2] += (double)c; } else { f[1] += val; f[3] += (double)c; }
-    }
-    block_sum_n<5>(f, sh.red_d2);
-    if (tid == 0) {
-      const long long fc_gt = (long long)f[2], fc_lt = (long long)f[3], fc_all = (long long)f[4];
-      double coarse_gt = 0, coarse_lt = 0;
-      long long cnt_gt = 0;
-      for (int q = 0; q < C; ++q) { coarse_gt += sh.part_d[q][0]; coarse_lt += sh.part_d[q][1]; cnt_gt += sh.part_i[q][0]; }
-      const double thr = (double)key_float(thr_key);
-      const long long n_gt = cnt_gt + fc_gt, n_lt = (n - cnt_gt - fc_all) + fc_lt;
-      const double sum_gt = fc_gt ? coarse_gt + f[0] : coarse_gt, sum_lt = fc_lt ? coarse_lt + f[1] : coarse_lt;
-      const long long n_eq = n - n_gt - n_lt;
-      const long long tt = K - n_gt;   // ties that belong to the top group
-      sh.res_i[6] = tt;
-      sh.res_i[7] = n_eq - tt;
-      sh.res_d[1] = (sum_gt + (tt > 0 ? (double)tt * thr : 0.0)) / (double)K;                       // mean_top
-      sh.res_d[2] = (sum_lt + (n_eq - tt > 0 ? (double)(n_eq - tt) * thr : 0.0)) / (double)(n - K);   // mean_adj
-    }
-  }
-  cluster.sync();
-  uint32_t key_j[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) key_j[j] = (pre[j] << 10) | (uint32_t)L->res_i[8 + j];
   const uint32_t thr_key = key_j[1];
-  const double mean_t = L->res_d[1], mean_j = L->res_d[2];
-  STAMP();
+  const double mean_a = L->res_d[0], mean_t = L->res_d[1], mean_j = L->res_d[2];
 
   // ---- pass 3: deviations
   double d[6] = {0, 0, 0, 0, 0, 0};
@@ -823,7 +1137,7 @@ static void select_shape(int& cluster, int& cache) {
 template <int K>
 static int launch_select_k(int n_grid, long long* header, const unsigned long long* ukeys, const uint32_t* ucnt,
                            float* wbuf, int64_t ldw, int32_t H, const LogTable& lf, double logV0, int64_t n_total,
-                           int64_t top, double* stats, bool beside_sweep, cudaStream_t st) {
+                           int64_t top, double* stats, bool beside_sweep, bool force_radix, cudaStream_t st) {
   static bool attr_set[64] = {false};
   int dev = 0;
   B200_CUDA(cudaGetDevice(&dev));
@@ -831,7 +1145,7 @@ static int launch_select_k(int n_grid, long long* header, const unsigned long lo
   select_shape(C, cache);
   static const bool forced = getenv("B200_SELECT_CLUSTER") != nullptr;
   if (beside_sweep && !forced) C = 2;     // a small footprint beside a running sweep (B200_LEV_FLAG_BESIDE_SWEEP)
-  const size_t dyn = (size_t)cache * 8;
+  const size_t dyn = (size_t)cache * 10;   // wealth, count and log-wealth bin of the cached bins
   if (dev < 64 && !attr_set[dev]) {
     B200_CUDA(cudaFuncSetAttribute(tally_select_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
     if (C > 8) B200_CUDA(cudaFuncSetAttribute(tally_select_kernel<K>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
@@ -851,7 +1165,7 @@ static int launch_select_k(int n_grid, long long* header, const unsigned long lo
   cfg.attrs = at;
   cfg.numAttrs = 1;
   return check_cuda(cudaLaunchKernelEx(&cfg, tally_select_kernel<K>, header, ukeys, ucnt, wbuf, ldw, H, lf, logV0,
-                                       n_total, top, stats, (int32_t)cache),
+                                       n_total, top, stats, (int32_t)cache, (int32_t)force_radix),
                     "tally_select launch");
 }
 
@@ -961,9 +1275,10 @@ extern "C" int b200_tally_stats(const b200_tally_plan* plan, void* workspace, co
     }
   const double logV0 = log((double)desc->value_0);
   const bool beside = (desc->flags & B200_LEV_FLAG_BESIDE_SWEEP) != 0;
+  const bool radix = (desc->flags & B200_LEV_FLAG_RADIX_SELECT) != 0;
   switch (desc->n_outcomes) {
-    case 2: return launch_select_k<2>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, st);
-    case 3: return launch_select_k<3>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, st);
-    default: return launch_select_k<4>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, st);
+    case 2: return launch_select_k<2>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
+    case 3: return launch_select_k<3>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
+    default: return launch_select_k<4>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
   }
 }

@@ -33,11 +33,17 @@ enum {
   TH_BAD = 2,       // outcomes outside {0..K-1} met by an ingest kernel
   TH_TIMEOUT = 3,   // a peer's bins never arrived
   TH_MISMATCH = 4,  // sum of the bin counts != n_total at the last statistics call
+  TH_RADIX = 5,     // grid points whose statistics took the radix route since the last finalize
   TH_TICKET = 9,    // last-block-done ticket of the compaction kernel
   TH_LISTPOS = 10,  // append cursor of the compaction kernel
   TH_CONCAT = 11,   // bins of all ranks before the merge removes duplicates
   TH_DEBUG = 16,    // 48 words of per-phase clock stamps (B200_TALLY_DEBUG builds)
-  TH_WORDS = 64
+  // Bounding box of (n_1, n_2) over the bin list, as 4 running maxima (identity 0):
+  // TALLY_MAX_HORIZON - min n_1, max n_1, TALLY_MAX_HORIZON - min n_2, max n_2.
+  // One atomic per block and word, never one per tuple.
+  TH_BOX_ACC = 64,  // the single-GPU compaction's accumulators (published and cleared by its last block)
+  TH_BOX = 68,      // the box of the list the statistics read
+  TH_WORDS = 72
 };
 
 struct TallyDev {

@@ -242,9 +242,10 @@ class FinalTally:
         self.rows = 0
 
     def stats(self, factors: np.ndarray, value_0: float, horizon: int, *, n_total: int, top: int,
-              beside_sweep: bool = False) -> torch.Tensor:
+              beside_sweep: bool = False, radix_select: bool = False) -> torch.Tensor:
         """The 12 statistics (engine.STAT_NAMES order) of every grid point: float64 [G,12] on the GPU.
-        beside_sweep: the call runs beside another kernel (B200_LEV_FLAG_BESIDE_SWEEP: a smaller footprint)."""
+        beside_sweep: the call runs beside another kernel (B200_LEV_FLAG_BESIDE_SWEEP: a smaller footprint).
+        radix_select: every grid point takes the radix route (B200_LEV_FLAG_RADIX_SELECT), for comparisons."""
         f = np.ascontiguousarray(factors, dtype=np.float32)
         if f.ndim != 2:
             raise ValueError("factors must be [G,K]")
@@ -253,7 +254,7 @@ class FinalTally:
         d = LevDesc()
         d.kind, d.mode, d.source = _lib.LEV_DISCRETE, _lib.MODE_LOG, _lib.SRC_STREAM
         d.horizon, d.n_outcomes, d.value_0 = int(horizon), k, float(value_0)
-        d.flags = _lib.LEV_FLAG_BESIDE_SWEEP if beside_sweep else 0
+        d.flags = (_lib.LEV_FLAG_BESIDE_SWEEP if beside_sweep else 0) | (_lib.LEV_FLAG_RADIX_SELECT if radix_select else 0)
         with torch.cuda.device(self.dev):
             for g0 in range(0, g, self.plan.grid_cap):
                 tile = np.ascontiguousarray(f[g0:g0 + self.plan.grid_cap])
@@ -274,7 +275,7 @@ class FinalTally:
             dist.all_reduce(w, op=dist.ReduceOp.MAX, group=self.group)
         w = w.cpu().tolist()
         return {"bins": w[0], "overflow": bool(w[1]), "bad_outcomes": w[2], "timed_out": bool(w[3]),
-                "count_mismatch": bool(w[4])}
+                "count_mismatch": bool(w[4]), "radix_route": w[5]}
 
     def check(self) -> dict:
         """info() + raise on anything that invalidates the statistics (and reset the tally)."""

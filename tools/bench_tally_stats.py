@@ -10,12 +10,14 @@ f = lev_exp.dice_factor_table(lev, 0.5, -0.5, 0.05)
 oc = engine.lev_draw("discrete", n, h, seed=420, probs=(1/6, 1/6, 2/3), packed=True)
 t = tally.FinalTally(n)
 ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-tt = np.zeros(3)
 reps = 30
-for it in range(reps + 3):
-    ev[0].record(); t.add(oc, 3); ev[1].record(); t.finalize(); ev[2].record()
-    st = t.stats(f, 100.0, h, n_total=n, top=100); ev[3].record()
-    torch.cuda.synchronize()
-    if it >= 3:
-        tt += [ev[i].elapsed_time(ev[i + 1]) * 1e3 for i in range(3)]
-print(os.environ.get("B200_SELECT_CLUSTER"), os.environ.get("B200_SELECT_CACHE"), "count/finalize/stats us:", (tt / reps).round(1), t.info()["bins"])
+for radix in (False, True):      # the log-wealth route (default), then the radix route (B200_LEV_FLAG_RADIX_SELECT)
+    tt = np.zeros(3)
+    for it in range(reps + 3):
+        ev[0].record(); t.add(oc, 3); ev[1].record(); t.finalize(); ev[2].record()
+        st = t.stats(f, 100.0, h, n_total=n, top=100, radix_select=radix); ev[3].record()
+        torch.cuda.synchronize()
+        if it >= 3:
+            tt += [ev[i].elapsed_time(ev[i + 1]) * 1e3 for i in range(3)]
+    print(os.environ.get("B200_SELECT_CLUSTER"), os.environ.get("B200_SELECT_CACHE"), "radix" if radix else "log-wealth",
+          "count/finalize/stats us:", (tt / reps).round(1), t.info()["bins"], "radix-route grid points:", t.info()["radix_route"])
