@@ -704,13 +704,14 @@ class FinalSweepPipeline:
             self.sweep_stream.wait_stream(cur)        # the caller produced `outcomes` on its stream
             data = outcomes.data if isinstance(outcomes, PackedCodes) else outcomes
             data.record_stream(self.sweep_stream)
-            if tally and (self.tallies[b] is None or self.tallies[b].plan.rows_cap < n):
-                from . import tally as _tally
-
-                self.tallies[b] = _tally.FinalTally(n, device=self.dev, group=self.group)   # collective with a group
             with torch.cuda.stream(self.sweep_stream):
                 if self.free[b] is not None:
                     self.sweep_stream.wait_event(self.free[b])
+                if tally and (self.tallies[b] is None or self.tallies[b].plan.rows_cap < n):
+                    from . import tally as _tally
+
+                    # on the sweep stream: the reset of its table runs before the count kernel fills it
+                    self.tallies[b] = _tally.FinalTally(n, device=self.dev, group=self.group)   # collective with a group
                 if not tally and (self.data_T[b] is None or tuple(self.data_T[b].shape) != (g, n)):
                     self.data_T[b] = torch.empty((g, n), dtype=torch.float32, device=self.dev)
                     self.ws[b] = rowstats_workspace(g, self.dev)

@@ -13,6 +13,7 @@ import pytest
 import torch as T
 
 import golden_io
+import tally_sets
 from oracle import lev_oracle as lo
 
 pytestmark = pytest.mark.gpu
@@ -275,10 +276,7 @@ def test_merge_of_rank_tallies_on_one_gpu(world):
     queued behind it.  Every rank must end with the identical bin list (bit-identical
     statistics) and with the statistics of the undivided population.
     """
-    import ctypes as C
-
-    from rlmd_b200 import _lib, engine, tally
-    from rlmd_b200._lib import check, lib, ptr, stream_ptr
+    from rlmd_b200 import engine
 
     case = golden_io.lev_case("dice_top5")
     oc = golden_io.draw_outcomes(case)
@@ -287,40 +285,18 @@ def test_merge_of_rank_tallies_on_one_gpu(world):
     codes = engine.encode_codes(oc)
     want = engine.lev_final_stats(f, case["v0"], case["top"], codes).cpu().numpy()
     # uneven shards, one of them empty when there are enough ranks
-    cuts = np.linspace(0, n, world + 1).astype(int)
-    cuts[1:-1] += np.arange(1, world) * 7 % 50
-    if world >= 3:
-        cuts[2] = cuts[1]
-    ranks = []
-    for r in range(world):
-        t = tally.FinalTally.__new__(tally.FinalTally)
-        t.dev, t.group, t._staging, t.rows, t.horizon = T.device("cuda", 0), None, None, 0, None
-        t.plan = _lib.TallyPlan()
-        t.plan.rows_cap, t.plan.bins_cap, t.plan.grid_cap, t.plan.world = n, n, 64, world
-        t.ws = T.empty((lib.b200_tally_workspace_bytes(C.byref(t.plan)) // 8,), dtype=T.int64, device="cuda")
-        t.exchange = None
-        t.ex_buf = T.zeros((lib.b200_tally_exchange_bytes(C.byref(t.plan)) // 8 + 1,), dtype=T.int64, device="cuda")
-        check(lib.b200_tally_reset(C.byref(t.plan), ptr(t.ws), stream_ptr()))
-        ranks.append(t)
+    cuts = tally_sets.shard_cuts(n, world)
+    ranks = tally_sets.one_gpu_ranks(world, n, n)
     for epoch in (1, 2, 3):      # successive sweeps alternate between the two published lists
         sl = slice(None) if epoch != 2 else slice(0, h - 3)      # another horizon in between
         ref = want if epoch != 2 else engine.lev_final_stats(f, case["v0"], case["top"],
                                                              engine.encode_codes(oc[:, sl])).cpu().numpy()
         hh = oc[:, sl].shape[1]
-        peers = []
         for r, t in enumerate(ranks):
             t.rows = 0
             if cuts[r + 1] > cuts[r]:
                 t.add(engine.encode_codes(oc[cuts[r]:cuts[r + 1], sl]), 3)
-            p = _lib.TallyPeers()
-            p.world, p.rank, p.epoch = world, r, epoch
-            for q in range(world):
-                p.exchange[q] = ranks[q].ex_buf.data_ptr()
-            peers.append(p)
-        for r, t in enumerate(ranks):
-            check(lib.b200_tally_finalize(C.byref(t.plan), ptr(t.ws), C.byref(peers[r]), 0, stream_ptr()))
-        for r, t in enumerate(ranks):
-            check(lib.b200_tally_finalize(C.byref(t.plan), ptr(t.ws), C.byref(peers[r]), 1, stream_ptr()))
+        tally_sets.merge_on_one_gpu(ranks, epoch)
         got = [t.stats(f, case["v0"], hh, n_total=n, top=case["top"]).cpu().numpy() for t in ranks]
         for r, t in enumerate(ranks):
             i = t.info()
@@ -329,6 +305,42 @@ def test_merge_of_rank_tallies_on_one_gpu(world):
         assert_same_stats(got[0], ref, rtol=1e-13)
     distinct = len({tuple(c) for c in lo.counts_discrete(oc, 3)})
     assert ranks[0].info()["bins"] == distinct
+
+
+@pytest.mark.parametrize("world", [2, 3, 8])
+def test_merge_of_long_rank_lists_on_one_gpu(world):
+    """
+    The same merge on the 150 000 distinct tuples of tally_sets' wide K = 3 set, shuffled over uneven shards
+    (one empty): every rank's list is tens of thousands of bins long and shares tuples with the others, so
+    the mark / unique kernels walk many chunks of MERGE_CHUNK positions, each placed after the first
+    occurrences of all earlier chunks, and rebuild the (n_1, n_2) box.  The merged list (about 150 k bins,
+    spilling in both select shapes) gives every rank bit-identical statistics, equal to the reference and to
+    the undivided tally, with the six-CTA and the two-CTA (beside_sweep: 8-GPU depth 2) select.
+    """
+    s = tally_sets.get("wide3")
+    want = tally_sets.set_reference("wide3")
+    codes = tally_sets.rows(s)
+    single = tally_sets.tally_in_blocks(codes, 3)
+    whole = single.stats(s["f"], s["v0"], s["h"], n_total=s["n"], top=s["top"]).cpu().numpy()
+    del single
+    cuts = tally_sets.shard_cuts(s["n"], world)
+    ranks = tally_sets.one_gpu_ranks(world, int(np.diff(cuts).max()), len(s["tuples"]))
+    for r, t in enumerate(ranks):
+        if cuts[r + 1] > cuts[r]:
+            t.add(codes[cuts[r]:cuts[r + 1]], 3)
+    tally_sets.merge_on_one_gpu(ranks, 1)
+    box = tally_sets.box_of(s["tuples"])
+    for beside in (False, True):
+        got = [t.stats(s["f"], s["v0"], s["h"], n_total=s["n"], top=s["top"], beside_sweep=beside).cpu().numpy()
+               for t in ranks]
+        for r, t in enumerate(ranks):
+            i = t.info()
+            assert not (i["overflow"] or i["timed_out"] or i["count_mismatch"] or i["bad_outcomes"]), (r, i)
+            assert i["bins"] == len(s["tuples"]), (r, i)
+            assert tally_sets.box_words(t) == box, r
+            assert np.array_equal(got[r].view(np.uint64), got[0].view(np.uint64)), f"rank {r} differs from rank 0"
+        assert_same_stats(got[0], want, rtol=1e-12)
+        assert_same_stats(got[0], whole, rtol=1e-13)
 
 
 def test_pipeline_depths_agree():
