@@ -151,7 +151,9 @@ int b200_lev_sweep(const b200_lev_desc* desc, const void* outcomes,
  * statistics into data[G,13,H-1]; after the last chunk `state` holds data_T.
  *
  * state : discrete (CHAIN): float [G,N] wealth, in/out (ignored as input when
- *         t_begin == 0); GBM: double [3,N] = running sum of x, its max, its min.
+ *         t_begin == 0); GBM: double [5,N] = running sum of x, its max, its min,
+ *         then the bit patterns of two 64-bit masks: bit g set once grid point g's
+ *         wealth has overflowed / underflowed (sticky, the first one decides).
  * dump  : float [G, t_end - t_begin, N] or NULL (advance the state only).
  * t_begin must be a multiple of 4 (discrete Philox) / 32 (GBM).
  */

@@ -621,15 +621,23 @@ draw_gbm_kernel(uint64_t seed, int64_t investor_offset, float log_mean, float si
 // ------------------------------------------------ GBM series chunk
 // Steps [t_begin, t_end) (t_begin a multiple of 32 so that the fp32 partial sums
 // fold exactly where the final-time kernels fold them) with the wealth after
-// every step dumped: dump[(g*tc + t-t_begin)*N + row].  state = double [3,N].
-__device__ __forceinline__ float gbm_wealth(double l, double S, double Smax, double Smin, double logV0) {
+// every step dumped: dump[(g*tc + t-t_begin)*N + row].  state = double [5,N]:
+// S, its running max and min, then the bit patterns of two 64-bit masks (bit g:
+// grid point g's wealth has overflowed / underflowed).  The reference's fp32 chain
+// saturates for good in time order - inf once it passes FLT_MAX, 0 once it falls
+// below half the smallest denormal, whichever comes first - so the series keeps
+// that order per grid point instead of reading it off the running extremes (a path
+// that underflowed and later climbed past ln FLT_MAX stays 0).
+__device__ __forceinline__ float gbm_wealth(double lw, uint64_t bit, uint64_t& over, uint64_t& under) {
   const double LOG_FLT_MAX = 88.72283905206835;
   const double LOG_FLT_ZERO = -103.97207708399179;
-  const double hi = logV0 + (l >= 0 ? l * Smax : l * Smin);
-  const double lo = logV0 + (l >= 0 ? l * Smin : l * Smax);
-  if (hi > LOG_FLT_MAX) return __int_as_float(0x7f800000);
-  if (lo < LOG_FLT_ZERO) return 0.0f;
-  return (float)exp(logV0 + l * S);
+  if (!((over | under) & bit)) {
+    if (lw > LOG_FLT_MAX) over |= bit;
+    else if (lw < LOG_FLT_ZERO) under |= bit;
+  }
+  if (over & bit) return __int_as_float(0x7f800000);
+  if (under & bit) return 0.0f;
+  return (float)exp(lw);
 }
 
 template <bool PHILOX>
@@ -640,7 +648,12 @@ gbm_chunk_kernel(const float* __restrict__ x, int64_t ld, const __grid_constant_
   const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (row >= N) return;
   GbmAcc acc;
-  if (t_begin > 0) { acc.S = state[row]; acc.Smax = state[N + row]; acc.Smin = state[2 * N + row]; }
+  uint64_t over = 0, under = 0;
+  if (t_begin > 0) {
+    acc.S = state[row]; acc.Smax = state[N + row]; acc.Smin = state[2 * N + row];
+    over = (uint64_t)__double_as_longlong(state[3 * N + row]);
+    under = (uint64_t)__double_as_longlong(state[4 * N + row]);
+  }
   const int64_t tc = t_end - t_begin;
   const uint64_t id = (uint64_t)(row + investor_offset);
   float xb[4];
@@ -655,17 +668,17 @@ gbm_chunk_kernel(const float* __restrict__ x, int64_t ld, const __grid_constant_
       xt = __ldg(x + row * ld + t);
     }
     acc.step(xt);
-    if (dump != nullptr) {
-      const double S = acc.S + (double)acc.p;
-      const double Smax = fmax(acc.Smax, acc.S + (double)acc.pmax);
-      const double Smin = fmin(acc.Smin, acc.S + (double)acc.pmin);
-      for (int g = 0; g < G; ++g)
-        __stcs(dump + ((int64_t)g * tc + (t - t_begin)) * N + row, gbm_wealth((double)lv.lev[g], S, Smax, Smin, logV0));
+    const double S = acc.S + (double)acc.p;
+    for (int g = 0; g < G; ++g) {
+      const float w = gbm_wealth(logV0 + (double)lv.lev[g] * S, 1ull << g, over, under);
+      if (dump != nullptr) __stcs(dump + ((int64_t)g * tc + (t - t_begin)) * N + row, w);
     }
     if ((t & 31) == 31) acc.fold();
   }
   acc.fold();
   state[row] = acc.S; state[N + row] = acc.Smax; state[2 * N + row] = acc.Smin;
+  state[3 * N + row] = __longlong_as_double((long long)over);
+  state[4 * N + row] = __longlong_as_double((long long)under);
 }
 
 // ------------------------------------------------------------ host side

@@ -213,7 +213,10 @@ def lev_sweep(
               None -> Philox draws on device
     mode      "chain" (exact fp32 product; discrete only) or "log"
     final_only  GBM: data_T without the running-extremes saturation, i.e. what gbm_fixed_final_lev's
-              torch.prod holds (B200_LEV_FLAG_FINAL_ONLY); the default is gbm_smart_lev's chain
+              torch.prod holds (B200_LEV_FLAG_FINAL_ONLY); the default is gbm_smart_lev's chain, saturated
+              from the running extremes of S: inf if log wealth ever passed ln FLT_MAX, else 0 if it ever
+              fell below ln 2^-150 (the reference's chain keeps whichever came first; the two differ only
+              on a path that did both - lev_series follows the reference; DESIGN.md section 4)
     want_state  GBM: also return "state" = float64 [3,N] (S, running max, running min of the summed
               log-returns): the leverage-independent state every row's log wealth log V0 + l S follows
               from (B200_LEV_FLAG_STATE_OUT; excludes want_log_w) - see gbm_growth_summary
@@ -434,7 +437,7 @@ def lev_series(
         if kind == "discrete":
             state = torch.empty((g, n), dtype=torch.float32, device=dev)
         else:
-            state = torch.empty((3, n), dtype=torch.float64, device=dev)
+            state = torch.empty((5, n), dtype=torch.float64, device=dev)   # S, max, min, overflow / underflow masks
         if chunk_steps is None:
             n_ref = max(n, 1)
             if group is not None:   # every rank must walk the same chunks (one exchange per chunk)
