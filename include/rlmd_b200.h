@@ -124,6 +124,13 @@ typedef struct b200_lev_desc {
  * instead of the log-wealth route - the route the kernel takes by itself for K = 4, non-finite log
  * factors, or a grid point whose log-wealth bins fail a check.  For comparing the two. */
 #define B200_LEV_FLAG_RADIX_SELECT 8
+/* b200_lev_tally on packed (2-bit / 1-bit) outcomes: the count kernel may start while the stream's previous
+ * kernel still runs (programmatic dependent launch).  It streams the outcomes at once and waits for that kernel
+ * to complete only before its first tally insertion or `counts` store, so the flag is for a stream whose
+ * previous kernel writes nothing the sweep reads: FinalSweepPipeline sets it at depth 1, where that kernel is
+ * the previous step's select, and the next sweep then runs on the SMs the statistics leave free.  The
+ * environment variable B200_PDL=0 turns it (and the same launch mode of the compaction and the select) off. */
+#define B200_LEV_FLAG_EARLY_START 16
 
 /*
  * outcomes : STREAM: uint8 [N,ld] (discrete, codes < K; or packed 2-bit codes,

@@ -41,7 +41,7 @@ class LevDesc(C.Structure):
     ]
 
 
-LEV_FLAG_FINAL_ONLY, LEV_FLAG_STATE_OUT, LEV_FLAG_BESIDE_SWEEP, LEV_FLAG_RADIX_SELECT = 1, 2, 4, 8
+LEV_FLAG_FINAL_ONLY, LEV_FLAG_STATE_OUT, LEV_FLAG_BESIDE_SWEEP, LEV_FLAG_RADIX_SELECT, LEV_FLAG_EARLY_START = 1, 2, 4, 8, 16
 MAX_PEERS = 8
 
 

@@ -1,6 +1,7 @@
 // Error plumbing and device queries shared by every entry point.
 #include "common.cuh"
 
+#include <cstdlib>
 #include <cstring>
 
 namespace b200 {
@@ -18,6 +19,11 @@ int set_error(int code, const char* fmt, ...) {
 int check_cuda(cudaError_t e, const char* what) {
   if (e == cudaSuccess) return 0;
   return set_error(B200_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+}
+
+bool pdl_enabled() {
+  static const bool on = [] { const char* e = getenv("B200_PDL"); return e == nullptr || atoi(e) != 0; }();
+  return on;
 }
 
 int sm_count() {

@@ -28,6 +28,19 @@ int check_cuda(cudaError_t e, const char* what);
 
 int sm_count();
 
+// -------------------------------------------- programmatic dependent launch
+// A kernel launched with the programmatic-stream-serialization attribute may start once every block of the
+// stream's previous kernel has executed launch_dependents (or exited); its griddepcontrol.wait then blocks
+// until that kernel has completed and its memory is visible.  Both instructions are no-ops in a kernel
+// launched without the attribute.  B200_PDL=0 in the environment (read once) launches without it.
+bool pdl_enabled();
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+inline void set_pdl_attribute(cudaLaunchAttribute& a) {
+  a.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  a.val.programmaticStreamSerializationAllowed = 1;
+}
+
 // ------------------------------------------------------------ Philox4x32-10
 // Counter-based generator (Salmon et al., SC'11).  Words are consumed as
 //   counter = (investor_id lo, investor_id hi, block index, stream tag)

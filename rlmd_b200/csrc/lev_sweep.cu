@@ -296,6 +296,7 @@ log_discrete_packed_kernel(const uint8_t* __restrict__ outcomes, int64_t ldb, in
                            const __grid_constant__ LogFactorTable lf, double logV0, float* __restrict__ data_T,
                            double* __restrict__ log_w, int32_t* __restrict__ counts, int64_t ldT, const TallyDev tally,
                            int32_t task_rows) {
+  if (TALLY) pdl_launch_dependents();   // the compaction's blocks may queue up behind the last wave
   const int lane = threadIdx.x & 31;
   const int64_t warp_global = (int64_t)blockIdx.x * COUNT_WARPS + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * COUNT_WARPS;
@@ -387,6 +388,9 @@ log_discrete_packed_kernel(const uint8_t* __restrict__ outcomes, int64_t ldb, in
       if (lane == r) { m1 = s1; m2 = s2; m3 = s3; }
     }
     // ---- epilogue: one row per lane
+    // Launched early (B200_LEV_FLAG_EARLY_START), the kernel has only read the outcomes so far; the table and
+    // `counts` belong to the previous kernel (the last step's statistics) until it has completed.
+    if (TALLY) pdl_wait();
     if (lane < nr) {
       const int64_t row = row0 + lane;
       int n[4];
@@ -814,28 +818,41 @@ static int run_log_discrete(const b200_lev_desc& d, const uint8_t* outcomes, con
   // grid would give each warp 3.3 tasks at 1e6 rows: a fifth of the run spent in the tail)
   const int64_t cap = packed ? (int64_t)0x7fffffff : (int64_t)sm_count() * 8;
   if (blocks > cap) blocks = cap;
-#define B200_LOG_LAUNCH(KERNEL, ...)                                                                                     \
+  if (packed && tally.keys != nullptr) {   // the tally sink, launched early on request (B200_LEV_FLAG_EARLY_START)
+    const auto kern = d.outcome_bits == 1 ? log_discrete_packed_kernel<2, true, 1>
+                      : d.n_outcomes == 2 ? log_discrete_packed_kernel<2, true>
+                      : d.n_outcomes == 3 ? log_discrete_packed_kernel<3, true>
+                                          : log_discrete_packed_kernel<4, true>;
+    // All L1, no shared memory: launched early, the kernel's first blocks land on SMs the compaction and the
+    // select set up for shared memory, and without this preference the sweep kept that split - a small L1 for
+    // its loads in flight - to the end (on B200 the overlapped sweep took 436 us, 409 with it; 387-391 alone).
+    B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxL1));
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)blocks);
+    cfg.blockDim = dim3(COUNT_WARPS * 32);
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    set_pdl_attribute(at[0]);
+    cfg.attrs = at;
+    cfg.numAttrs = (d.flags & B200_LEV_FLAG_EARLY_START) != 0 && pdl_enabled() ? 1 : 0;
+    return check_cuda(cudaLaunchKernelEx(&cfg, kern, outcomes, d.ld_outcomes, d.horizon, N, d.n_grid, lf, logV0, data_T,
+                                         log_w, counts, out_ld(d), tally, (int32_t)task_rows),
+                      "log_discrete_packed (tally) launch");
+  }
+#define B200_LOG_LAUNCH(KERNEL, ...)                                                                                  \
   KERNEL<__VA_ARGS__><<<(unsigned)blocks, COUNT_WARPS * 32, 0, st>>>(outcomes, d.ld_outcomes, d.horizon, N, d.n_grid, lf, \
                                                                      logV0, data_T, log_w, counts, out_ld(d), tally B200_EXTRA)
   if (d.outcome_bits == 1) {
 #define B200_EXTRA , task_rows
-    if (tally.keys != nullptr) B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, true, 1);
-    else B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, false, 1);
+    B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, false, 1);
 #undef B200_EXTRA
   } else if (d.outcome_bits == 2) {
 #define B200_EXTRA , task_rows
-    if (tally.keys != nullptr) {
-      switch (d.n_outcomes) {
-        case 2: B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, true); break;
-        case 3: B200_LOG_LAUNCH(log_discrete_packed_kernel, 3, true); break;
-        default: B200_LOG_LAUNCH(log_discrete_packed_kernel, 4, true); break;
-      }
-    } else {
-      switch (d.n_outcomes) {
-        case 2: B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, false); break;
-        case 3: B200_LOG_LAUNCH(log_discrete_packed_kernel, 3, false); break;
-        default: B200_LOG_LAUNCH(log_discrete_packed_kernel, 4, false); break;
-      }
+    switch (d.n_outcomes) {
+      case 2: B200_LOG_LAUNCH(log_discrete_packed_kernel, 2, false); break;
+      case 3: B200_LOG_LAUNCH(log_discrete_packed_kernel, 3, false); break;
+      default: B200_LOG_LAUNCH(log_discrete_packed_kernel, 4, false); break;
     }
 #undef B200_EXTRA
 #define B200_EXTRA

@@ -181,6 +181,9 @@ tally_compact_kernel(TallyDev t, unsigned long long* __restrict__ ukeys, uint32_
   const uint64_t cap = t.mask + 1;
   const uint64_t base = (uint64_t)blockIdx.x * COMPACT_CHUNK;
   if (threadIdx.x == 0) n_s = 0;
+  // launched early (one GPU): the table is the count kernel's until it has completed
+  pdl_launch_dependents();
+  pdl_wait();
   __syncthreads();
   // all of a thread's slots (keys and counts) are requested before the first is looked at:
   // one round trip to memory per block, not one per occupied slot
@@ -569,6 +572,11 @@ tally_select_kernel(long long* __restrict__ header, const unsigned long long* __
   uint32_t* cc = reinterpret_cast<uint32_t*>(dyn) + SEL_CACHE; // [SEL_CACHE] their counts
   uint16_t* cb = reinterpret_cast<uint16_t*>(cc + SEL_CACHE);  // [SEL_CACHE] their log-wealth bins
   SelShared* L = cluster.map_shared_rank(&sh, 0);              // the leader's copy
+  // Launched early (one GPU, depth 1), the select waits here for the compaction's list and header; the next
+  // sweep's count kernel may then start on the SMs this grid leaves free (it waits for this grid before it
+  // touches the table).
+  pdl_launch_dependents();
+  pdl_wait();
 
   const int g = blockIdx.x / C;
   const long long B = header[TH_NBINS];
@@ -1119,10 +1127,11 @@ tally_select_kernel(long long* __restrict__ header, const unsigned long long* __
 
 // Cluster size and per-CTA shared-memory cache of the select kernel.  Defaults from measurement on
 // B200 (DESIGN.md): B200_SELECT_CLUSTER / B200_SELECT_CACHE override them for experiments.
-static void select_shape(int& cluster, int& cache) {
+static void select_shape(int& cluster, int& cache, bool early) {
   static int c = [] {
     const char* e = getenv("B200_SELECT_CLUSTER");
-    int x = e ? atoi(e) : 6;
+    if (e == nullptr) return 0;
+    const int x = atoi(e);
     return x < 1 ? 1 : x > SEL_MAX_CLUSTER ? SEL_MAX_CLUSTER : x;
   }();
   static int k = [] {
@@ -1130,19 +1139,22 @@ static void select_shape(int& cluster, int& cache) {
     int x = e ? atoi(e) : 16384;
     return x < 0 ? 0 : x > 20480 ? 20480 : x;
   }();
-  cluster = c;
+  // 0: six CTAs per grid point, three when the select is launched early - the next sweep then has the other
+  // 88 SMs (of 148) while the select runs, and 3 x 16 384 cached bins still hold the flagship's 45 561
+  cluster = c != 0 ? c : early ? 3 : 6;
   cache = k;
 }
 
 template <int K>
 static int launch_select_k(int n_grid, long long* header, const unsigned long long* ukeys, const uint32_t* ucnt,
                            float* wbuf, int64_t ldw, int32_t H, const LogTable& lf, double logV0, int64_t n_total,
-                           int64_t top, double* stats, bool beside_sweep, bool force_radix, cudaStream_t st) {
+                           int64_t top, double* stats, bool beside_sweep, bool force_radix, bool early,
+                           cudaStream_t st) {
   static bool attr_set[64] = {false};
   int dev = 0;
   B200_CUDA(cudaGetDevice(&dev));
   int C = 1, cache = 0;
-  select_shape(C, cache);
+  select_shape(C, cache, early);
   static const bool forced = getenv("B200_SELECT_CLUSTER") != nullptr;
   if (beside_sweep && !forced) C = 2;     // a small footprint beside a running sweep (B200_LEV_FLAG_BESIDE_SWEEP)
   const size_t dyn = (size_t)cache * 10;   // wealth, count and log-wealth bin of the cached bins
@@ -1157,13 +1169,14 @@ static int launch_select_k(int n_grid, long long* header, const unsigned long lo
   cfg.blockDim = dim3(SEL_THREADS);
   cfg.dynamicSmemBytes = dyn;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
+  cudaLaunchAttribute at[2];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = (unsigned)C;
   at[0].val.clusterDim.y = 1;
   at[0].val.clusterDim.z = 1;
+  set_pdl_attribute(at[1]);
   cfg.attrs = at;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = early ? 2 : 1;
   return check_cuda(cudaLaunchKernelEx(&cfg, tally_select_kernel<K>, header, ukeys, ucnt, wbuf, ldw, H, lf, logV0,
                                        n_total, top, stats, (int32_t)cache, (int32_t)force_radix),
                     "tally_select launch");
@@ -1216,8 +1229,18 @@ extern "C" int b200_tally_finalize(const b200_tally_plan* plan, void* workspace,
   const int cgrid = (int)((L.capA + COMPACT_CHUNK - 1) / COMPACT_CHUNK);
   if (plan->world == 1) {
     if (phase == 1) return 0;
-    tally_compact_kernel<false><<<cgrid, 256, 0, st>>>(t, L.ukeys, L.ucnt, std::min(plan->bins_cap, L.list_cap), P);
-    return check_cuda(cudaGetLastError(), "tally_compact launch");
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)cgrid);
+    cfg.blockDim = dim3(256);
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    set_pdl_attribute(at[0]);
+    cfg.attrs = at;
+    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    return check_cuda(cudaLaunchKernelEx(&cfg, tally_compact_kernel<false>, t, L.ukeys, L.ucnt,
+                                         (int64_t)std::min(plan->bins_cap, L.list_cap), P),
+                      "tally_compact launch");
   }
   B200_REQUIRE(peers != nullptr, "tally_finalize: peers is NULL with world > 1");
   B200_REQUIRE(peers->world == plan->world && peers->rank >= 0 && peers->rank < peers->world,
@@ -1276,9 +1299,11 @@ extern "C" int b200_tally_stats(const b200_tally_plan* plan, void* workspace, co
   const double logV0 = log((double)desc->value_0);
   const bool beside = (desc->flags & B200_LEV_FLAG_BESIDE_SWEEP) != 0;
   const bool radix = (desc->flags & B200_LEV_FLAG_RADIX_SELECT) != 0;
+  // one GPU, nothing beside it: the select starts under the compaction, and the next sweep under the select
+  const bool early = plan->world == 1 && !beside && pdl_enabled();
   switch (desc->n_outcomes) {
-    case 2: return launch_select_k<2>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
-    case 3: return launch_select_k<3>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
-    default: return launch_select_k<4>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, st);
+    case 2: return launch_select_k<2>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, early, st);
+    case 3: return launch_select_k<3>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, early, st);
+    default: return launch_select_k<4>(desc->n_grid, L.header, L.ukeys, L.ucnt, L.wbuf, L.ldw, desc->horizon, lf, logV0, n_total, top, stats, beside, radix, early, st);
   }
 }

@@ -694,6 +694,8 @@ class FinalSweepPipeline:
         self.count = 0
         self.last_sweep = None                # (start, end) events of the last sweep, when timing is on
         self.timing = False
+        self._timing_stream = None
+        self._sweep_opens = None              # depth 1, timing on: the next sweep's start event
 
     def submit(self, outcomes, factors: Optional[np.ndarray] = None) -> torch.Tensor:
         f = self.factors if factors is None else np.ascontiguousarray(factors, dtype=np.float32)
@@ -702,6 +704,14 @@ class FinalSweepPipeline:
         b = self.count % self.depth
         self.count += 1
         tally = self.statistics == "tally"
+        # Depth 1 on the tally path: count kernel, compaction and select follow each other on one stream with
+        # nothing between them but event waits and records without timing, so each kernel starts under the one before it
+        # (programmatic dependent launch, B200_LEV_FLAG_EARLY_START): the sweep of this step streams its rows on
+        # the SMs the previous step's select leaves free.  A record of a timing event would end that overlap,
+        # so the sweep's timing events are taken on a stream of their own (_stamp).
+        chain = tally and self.depth == 1
+        if not (self.timing and chain):
+            self._sweep_opens = None
         with torch.cuda.device(self.dev):
             cur = torch.cuda.current_stream()
             self.sweep_stream.wait_stream(cur)        # the caller produced `outcomes` on its stream
@@ -719,31 +729,47 @@ class FinalSweepPipeline:
                     self.data_T[b] = torch.empty((g, n), dtype=torch.float32, device=self.dev)
                     self.ws[b] = rowstats_workspace(g, self.dev)
                 if self.timing:
-                    t0 = torch.cuda.Event(enable_timing=True)
-                    t0.record(self.sweep_stream)
+                    t0 = self._sweep_opens if chain and self._sweep_opens is not None else self._stamp()
                 if tally:
-                    self.tallies[b].add(outcomes, f.shape[1])
+                    self.tallies[b].add(outcomes, f.shape[1], early_start=chain)
                 else:
                     lev_sweep(self.kind, f, self.value_0, outcomes=outcomes, mode="log", out_data_T=self.data_T[b])
-                swept = torch.cuda.Event(enable_timing=self.timing)
-                swept.record(self.sweep_stream)
                 if self.timing:
-                    self.last_sweep = (t0, swept)
+                    self.last_sweep = (t0, self._stamp())
             n_total = self.n_total if self.n_total is not None else n
             with torch.cuda.stream(self.stats_stream):
-                self.stats_stream.wait_event(swept)
+                if self.depth > 1:
+                    swept = torch.cuda.Event()
+                    swept.record(self.sweep_stream)
+                    self.stats_stream.wait_event(swept)
                 if tally:
                     self.tallies[b].finalize()
+                    if self.timing and chain:
+                        # the next step's sweep starts under this step's select: its window opens here
+                        self._sweep_opens = self._stamp()
                     stats = self.tallies[b].stats(f, self.value_0, h, n_total=n_total, top=self.top,
                                                   beside_sweep=self.depth > 1)
                 else:
                     stats = rowstats(self.data_T[b], self.top, n_total=self.n_total, group=self.group,
                                      workspace=self.ws[b])
-                done = torch.cuda.Event()
-                done.record(self.stats_stream)
-                self.free[b] = done
+                if self.depth > 1:
+                    done = torch.cuda.Event()
+                    done.record(self.stats_stream)
+                    self.free[b] = done
                 stats.record_stream(cur)
         return stats
+
+    def _stamp(self) -> torch.cuda.Event:
+        """A timing event that completes with the work enqueued so far on the sweep stream: recorded on a
+        stream of its own behind an event without timing, which leaves the sweep stream's kernels overlapping."""
+        if self._timing_stream is None:
+            self._timing_stream = torch.cuda.Stream(self.dev)
+        mark = torch.cuda.Event()
+        mark.record(self.sweep_stream)
+        self._timing_stream.wait_event(mark)
+        ev = torch.cuda.Event(enable_timing=True)
+        ev.record(self._timing_stream)
+        return ev
 
     def submit_philox(self, n_investors: int, horizon: int, *, seed: int, investor_offset: int = 0,
                       log_mean: float, sigma: float, growth_quantiles: Optional[Sequence[float]] = (0.05, 0.5)):
@@ -797,6 +823,8 @@ class FinalSweepPipeline:
     def synchronize(self) -> None:
         self.sweep_stream.synchronize()
         self.stats_stream.synchronize()
+        if self._timing_stream is not None:
+            self._timing_stream.synchronize()
         for t in self.tallies:
             if t is not None:
                 t.check()

@@ -143,11 +143,13 @@ class FinalTally:
         self.rows += n
 
     def add(self, outcomes, n_outcomes: int, *, counts: Optional[torch.Tensor] = None,
-            codes_out: Optional[torch.Tensor] = None) -> None:
+            codes_out: Optional[torch.Tensor] = None, early_start: bool = False) -> None:
         """
         Tallies the rows of `outcomes` (a CUDA tensor [N,H] in any accepted format, or
         PackedCodes) on the current stream.  `counts` (int32 [N,K]) and `codes_out`
         (uint8 [N, >=H], reference formats only) are optional extra sinks.
+        early_start: packed outcomes only - the count kernel may start while the stream's previous kernel
+        runs (B200_LEV_FLAG_EARLY_START); only when that kernel does not write the outcomes.
         """
         from .engine import PackedCodes
 
@@ -166,6 +168,7 @@ class FinalTally:
                 d.value_0 = 1.0
                 d.outcome_bits = outcomes.bits if packed else 8
                 d.ld_outcomes = data.stride(0) if n > 1 else data.shape[1]
+                d.flags = _lib.LEV_FLAG_EARLY_START if early_start else 0
                 check(lib.b200_lev_tally(C.byref(d), ptr(data), C.byref(self.plan), ptr(self.ws), ptr(counts),
                                          stream_ptr()))
                 return
