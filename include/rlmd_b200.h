@@ -324,6 +324,33 @@ int b200_rowstats(const float* values, int64_t rows, int64_t n, int64_t ld,
 int b200_rowstats_exchange(int32_t phase, int64_t out[5]);
 
 /* ------------------------------------------------------------------ *
+ * Float64 leverage sweeps (the reference run under
+ * torch.set_default_dtype(torch.float64): coin and GBM) - single GPU
+ * ------------------------------------------------------------------ */
+/* bytes of device workspace b200_rowstats_f64 needs for `rows` rows */
+int64_t b200_rowstats_f64_workspace_bytes(int64_t rows);
+
+/* The 12 statistics of b200_rowstats (same order and definitions) over double
+ * rows: values double [rows, ld], n >= 1 entries per row, 1 <= top <= n (top == n:
+ * the adj group is empty and its statistics are NaN, as torch's).  Exact order
+ * statistics (select on the fp64 bit pattern, NaN greatest), fp64 moments.
+ * stats double [rows, 12]. */
+int b200_rowstats_f64(const double* values, int64_t rows, int64_t n, int64_t ld,
+                      int64_t top, void* workspace, double* stats, void* stream);
+
+/* Steps [t_begin, t_end) of the exact fp64 chain value <- value * m_t
+ * (lev/lev_exp.py:160-212, :1042-1093).  desc: kind, n_investors, horizon,
+ * ld_outcomes, n_grid (<= B200_MAX_GRID), n_outcomes as for b200_lev_chunk;
+ * source must be B200_SRC_STREAM (value_0, seed and mode are not read).
+ *   discrete: outcomes uint8 codes [N, ld], factors_host double [G,K], m = factors[g][code]
+ *   GBM:      outcomes double x [N, ld],    factors_host double lev[G], m = exp(lev[g] * x)
+ * state : double [G,N] wealth, in/out (value_0 everywhere before step 0).
+ * dump  : double [G, t_end - t_begin, N] wealth after every step, or NULL. */
+int b200_lev_chunk_f64(const b200_lev_desc* desc, const void* outcomes,
+                       const double* factors_host, int32_t t_begin, int32_t t_end,
+                       double* state, double* dump, void* stream);
+
+/* ------------------------------------------------------------------ *
  * Batched multiplicative environment step (K4)
  *
  * Sits behind the gym.Env classes of envs/coin_flip_envs.py (Coin_Inv{A,B,C}

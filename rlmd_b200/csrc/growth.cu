@@ -18,13 +18,11 @@
 // log_w, so selecting on log_w selects g.  Six streaming passes of 8 B/element,
 // every cross-block quantity an 8-byte workspace word (summed across ranks by a
 // multi-GPU caller, like b200_rowstats).
-#include "common.cuh"
+#include "select64.cuh"
 
 namespace b200 {
 
 constexpr int GT = 8;                 // target ranks
-constexpr int GBITS = 11, GBINS = 1 << GBITS;
-constexpr int GLEVELS = 6;            // 11,11,11,11,11,9 bits
 constexpr int G_THREADS = 256;
 
 struct GrowthWS {
@@ -50,25 +48,6 @@ struct GrowthParams {
   int n_q;
 };
 
-__host__ __device__ __forceinline__ unsigned long long double_key(double x) {
-  unsigned long long b;
-#ifdef __CUDA_ARCH__
-  b = (unsigned long long)__double_as_longlong(x);
-#else
-  union { double d; unsigned long long u; } cv; cv.d = x; b = cv.u;
-#endif
-  if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) return ~0ull;  // NaN sorts last (numpy / torch)
-  return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-__device__ __forceinline__ double key_double(unsigned long long k) {
-  if (k == ~0ull) return __longlong_as_double(0x7ff8000000000000LL);
-  const unsigned long long b = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;
-  return __longlong_as_double((long long)b);
-}
-
-__host__ __device__ __forceinline__ int level_shift(int level) { return level < 5 ? 64 - GBITS * (level + 1) : 0; }
-__host__ __device__ __forceinline__ int level_bins(int level) { return level < 5 ? GBINS : 1 << 9; }
-
 // grid = (slices, rows)
 template <int LEVEL>
 __global__ void __launch_bounds__(G_THREADS)
@@ -82,14 +61,10 @@ growth_pass_kernel(const double* __restrict__ log_w, const float* __restrict__ d
   const float* __restrict__ w32 = data_T ? data_T + row * ld_T : nullptr;
   GrowthWS* w = ws + row;
   constexpr int NH = LEVEL == 0 ? 1 : GT;
-  const int bins = level_bins(LEVEL), shift = level_shift(LEVEL);
   for (int i = threadIdx.x; i < NH * GBINS; i += G_THREADS) g_hist[i] = 0;
   unsigned long long pfx[GT];
   double mean = 0.0;
-  if (LEVEL > 0) {
-#pragma unroll
-    for (int j = 0; j < GT; ++j) pfx[j] = w->prefix[j] >> (shift + (LEVEL < 5 ? GBITS : 9));
-  }
+  if (LEVEL > 0) select64_prefixes<LEVEL, GT>(w->prefix, pfx);
   if (LEVEL == 1) mean = w->mean;
   __syncthreads();
 
@@ -104,15 +79,11 @@ growth_pass_kernel(const double* __restrict__ log_w, const float* __restrict__ d
       if (has_x) ok = x > 0.0f && x < __int_as_float(0x7f800000);
       else ok = fabs(lw) < __longlong_as_double(0x7ff0000000000000LL);
       if (ok) { a1 += g; ++c0; }
-      atomicAdd(&g_hist[k >> shift], 1u);
-    } else {
-      if (LEVEL == 1) { const double d = (lw - p.log_v0) / p.h - mean; a0 += d * d; }
-      const unsigned long long hi = k >> (shift + (LEVEL < 5 ? GBITS : 9));
-      const unsigned int lo = (unsigned int)(k >> shift) & (unsigned int)(bins - 1);
-#pragma unroll
-      for (int j = 0; j < GT; ++j)
-        if (hi == pfx[j]) atomicAdd(&g_hist[j * GBINS + lo], 1u);
+    } else if (LEVEL == 1) {
+      const double d = (lw - p.log_v0) / p.h - mean;
+      a0 += d * d;
     }
+    select64_count<LEVEL, GT>(k, pfx, g_hist);
   };
   // four independent loads per thread are in flight before the first is used: with 64 KB of histograms a
   // block the SM holds few warps, so the passes were bound by one memory round trip per element per thread
@@ -155,38 +126,13 @@ __global__ void __launch_bounds__(256)
 growth_resolve_kernel(GrowthWS* __restrict__ ws, int level, int64_t n_total, const __grid_constant__ GrowthParams p,
                       double* __restrict__ out, int out_ld) {
   GrowthWS* w = ws + blockIdx.x;
-  const int bins = level_bins(level), shift = level_shift(level);
-  // warp j resolves target j (eight warps, eight targets, all at once): every lane sums a contiguous
-  // run of bins, a shuffle scan names the lane whose run holds the rank, that lane walks its run
+  // warp j resolves target j (eight warps, eight targets, all at once)
   {
-    const int j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int j = threadIdx.x >> 5;
     const long long* h = level == 0 ? w->hist[0] : w->hist[j];
     const long long rank = level == 0 ? p.rank[j] : w->rank[j];
-    const int per = bins / 32;   // 64 or 16
-    long long local = 0;
-    for (int i = 0; i < per; ++i) local += h[lane * per + i];
-    long long incl = local;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long up = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += up;
-    }
-    const long long excl = incl - local;
-    const long long total = __shfl_sync(0xffffffffu, incl, 31);
-    const bool owner = (rank >= excl && rank < incl) || (lane == 31 && rank >= total);
-    if (owner) {
-      long long r = rank - excl;
-      int b = lane * per;
-      for (int i = 0; i < per; ++i) {
-        const long long c = h[lane * per + i];
-        if (r < c || i == per - 1) { b = lane * per + i; break; }
-        r -= c;
-      }
-      const unsigned long long add = (unsigned long long)b << shift;
-      w->prefix[j] = (level == 0 ? 0ull : w->prefix[j]) | add;
-      w->rank[j] = r;
-      if (level == GLEVELS - 1) w->value[j] = (key_double(w->prefix[j]) - p.log_v0) / p.h;
-    }
+    if (select64_resolve(h, level, rank, &w->prefix[j], &w->rank[j]) && level == GLEVELS - 1)
+      w->value[j] = (key_double(w->prefix[j]) - p.log_v0) / p.h;
   }
   __threadfence_block();
   __syncthreads();

@@ -410,11 +410,14 @@ def lev_series(
     n_total: Optional[int] = None,
     group=None,
     device=None,
+    dtype: torch.dtype = torch.float32,
 ):
     """
     Per-step statistics of the whole grid (the *_smart_lev contract):
     returns data [G,13,H-1] fp32 (rows: the 12 statistics in the reference's
     order, then the leverage) and data_T [G,N] fp32 (wealth after step H-1).
+    dtype=torch.float64: the reference run under a float64 default dtype - see
+    lev_series_f64 (factors float64, data / data_T float64, one GPU).
 
     The horizon is walked in chunks: b200_lev_chunk dumps the wealth after every
     step of the chunk to a [G*steps, N] buffer, b200_rowstats reduces every row,
@@ -423,6 +426,15 @@ def lev_series(
     A chunk is up to `chunk_bytes` (8 GB of the 180) and 2048 rows: the statistics'
     launch and cross-GPU latencies (4 exchange steps per chunk) are paid once per chunk.
     """
+    if dtype == torch.float64:
+        if group is not None:
+            raise ValueError("float64 sweeps are single-GPU")
+        if n_total is not None and outcomes is not None and int(n_total) != outcomes.shape[0]:
+            raise ValueError("float64 sweeps are single-GPU: n_total must be the number of investors")
+        return lev_series_f64(kind, factors, lev_row, value_0, top, outcomes, chunk_steps=chunk_steps,
+                              chunk_bytes=chunk_bytes)
+    if dtype != torch.float32:
+        raise ValueError("dtype must be torch.float32 or torch.float64")
     require_cuda()
     f = np.ascontiguousarray(factors, dtype=np.float32)
     mode = "chain" if kind == "discrete" else "log"
@@ -470,6 +482,87 @@ def lev_series(
             torch.cuda.current_stream().synchronize()
             sharding.raise_if_peers_timed_out(group, dev)
     return data, data_T
+
+
+def _desc_f64(kind: str, factors, outcomes):
+    """The b200_lev_chunk_f64 descriptor and float64 factor table of a streamed sweep."""
+    want = {"discrete": torch.uint8, "gbm": torch.float64}.get(kind)
+    if want is None:
+        raise ValueError("kind must be 'discrete' or 'gbm'")
+    if not isinstance(outcomes, torch.Tensor) or not outcomes.is_cuda or outcomes.dtype != want \
+            or outcomes.dim() != 2 or outcomes.stride(1) != 1:
+        raise ValueError(f"float64 sweeps stream outcomes: a [N,H] {want} CUDA tensor with unit inner stride")
+    f = np.ascontiguousarray(factors, dtype=np.float64)
+    d = LevDesc()
+    if kind == "discrete":
+        if f.ndim != 2:
+            raise ValueError("factors must be [G,K]")
+        d.kind, d.n_outcomes = _lib.LEV_DISCRETE, f.shape[1]
+    else:
+        f = f.reshape(-1)
+        d.kind = _lib.LEV_GBM
+    g = f.shape[0]
+    if not 1 <= g <= _lib.MAX_GRID:
+        raise ValueError(f"float64 sweeps take 1..{_lib.MAX_GRID} grid points (got {g})")
+    n, h = outcomes.shape
+    d.n_grid, d.n_investors, d.horizon = g, n, h
+    d.source, d.mode = _lib.SRC_STREAM, _lib.MODE_CHAIN
+    d.ld_outcomes = outcomes.stride(0) if n > 1 else max(outcomes.stride(0), h)
+    return d, f, g, n, h
+
+
+def lev_series_f64(kind: str, factors, lev_row, value_0: float, top: int, outcomes: torch.Tensor, *,
+                   chunk_steps: Optional[int] = None, chunk_bytes: int = 8 << 30):
+    """
+    lev_series for the reference run under torch.set_default_dtype(torch.float64), on one GPU:
+    the exact fp64 chain value = value_0 * m_0, value = value * m_t (b200_lev_chunk_f64) and
+    the statistics of float64 rows (b200_rowstats_f64).
+    kind "discrete": outcomes uint8 codes [N,H], factors float64 [G,K];
+    kind "gbm": outcomes float64 x [N,H], factors = float64 lev [G] (m = exp(l x)).
+    Returns data [G,13,H-1] and data_T [G,N], float64 on the GPU.  A chunk is up to
+    `chunk_bytes` of 8-byte wealth and 2048 rows.
+    """
+    require_cuda()
+    d, f, g, n, h = _desc_f64(kind, factors, outcomes)
+    fptr = f.ctypes.data_as(C.POINTER(C.c_double))
+    dev = outcomes.device
+    with torch.cuda.device(dev):
+        data = torch.zeros((g, 13, max(h - 1, 0)), dtype=torch.float64, device=dev)
+        if h > 1:
+            data[:, 12, :] = torch.as_tensor(np.asarray(lev_row, dtype=np.float64), device=dev)[:, None]
+        state = torch.full((g, n), float(value_0), dtype=torch.float64, device=dev)
+        if chunk_steps is None:
+            chunk_steps = min(h, chunk_bytes // max(8 * g * n, 1), 2048 // g)
+        tc_max = max(1, min(int(chunk_steps), h))
+        chunk = torch.empty((g * tc_max * max(n, 1),), dtype=torch.float64, device=dev)
+        ws = rowstats_f64_workspace(g * tc_max, dev)
+        for t0 in range(0, h, tc_max):
+            t1 = min(h, t0 + tc_max)
+            tc = t1 - t0
+            dump = chunk[: g * tc * n].view(g * tc, n)
+            check(lib.b200_lev_chunk_f64(C.byref(d), ptr(outcomes), fptr, t0, t1, ptr(state), ptr(dump), stream_ptr()))
+            lo = max(t0, 1)
+            if n > 0 and t1 > lo:
+                st = rowstats(dump, top, workspace=ws[: g * tc]).view(g, tc, 12)
+                data[:, :12, lo - 1:t1 - 1] = st[:, lo - t0:, :].permute(0, 2, 1)
+    return data, state
+
+
+def lev_final_f64(kind: str, factors, value_0: float, top: int, outcomes: torch.Tensor):
+    """
+    The *_fixed_final_lev counterpart of lev_series_f64 (same inputs): the fp64 chain over the whole
+    horizon without a dump, then the statistics of the float64 rows.
+    Returns (stats [G,12], data_T [G,N]), float64 on the GPU.
+    """
+    require_cuda()
+    d, f, g, n, h = _desc_f64(kind, factors, outcomes)
+    dev = outcomes.device
+    with torch.cuda.device(dev):
+        data_T = torch.full((g, n), float(value_0), dtype=torch.float64, device=dev)
+        check(lib.b200_lev_chunk_f64(C.byref(d), ptr(outcomes), f.ctypes.data_as(C.POINTER(C.c_double)), 0, h,
+                                     ptr(data_T), None, stream_ptr()))
+        stats = rowstats(data_T, top) if n > 0 else torch.full((g, 12), float("nan"), dtype=torch.float64, device=dev)
+    return stats, data_T
 
 
 _copy_streams = {}
@@ -868,11 +961,38 @@ def rowstats_workspace(rows: int, device) -> torch.Tensor:
     return torch.empty((rows, nbytes // 8 // max(rows, 1)), dtype=torch.int64, device=device)
 
 
+def rowstats_f64_workspace(rows: int, device) -> torch.Tensor:
+    nbytes = lib.b200_rowstats_f64_workspace_bytes(rows)
+    return torch.empty((rows, nbytes // 8 // max(rows, 1)), dtype=torch.int64, device=device)
+
+
+def _rowstats_f64(values: torch.Tensor, top: int, n_total: Optional[int], workspace: Optional[torch.Tensor]):
+    require_cuda()
+    if values.dim() != 2 or not values.is_cuda or values.stride(1) != 1:
+        raise ValueError("values must be a [rows,n] float64 CUDA tensor with unit inner stride")
+    rows, n = values.shape
+    if n_total is not None and int(n_total) != n:
+        raise ValueError("float64 rows are single-GPU: n_total must equal the row length")
+    ld = values.stride(0) if rows > 1 else max(values.stride(0), n)
+    dev = values.device
+    stats = torch.empty((rows, 12), dtype=torch.float64, device=dev)
+    if rows == 0:
+        return stats
+    with torch.cuda.device(dev):
+        ws = workspace if workspace is not None else rowstats_f64_workspace(rows, dev)
+        check(lib.b200_rowstats_f64(ptr(values), rows, n, ld, int(top), ptr(ws), ptr(stats), stream_ptr()))
+    return stats
+
+
 def rowstats(values: torch.Tensor, top: int, *, n_total: Optional[int] = None, group=None,
              workspace: Optional[torch.Tensor] = None, exchange: Optional[str] = None) -> torch.Tensor:
     """
     The reference's 12 summary statistics for every row of `values` [rows, n]
     (fp32, CUDA, unit inner stride) -> float64 [rows, 12] (STAT_NAMES order).
+
+    float64 rows (one GPU; `workspace` from rowstats_f64_workspace) take b200_rowstats_f64: the
+    same statistics with exact fp64 order statistics, 1 <= top <= n (top == n: the adj group is
+    empty and its statistics are NaN, as torch's).
 
     With `group` (a torch.distributed process group) the rows are investor
     shards of a global vector of n_total entries and every rank returns the global
@@ -881,6 +1001,10 @@ def rowstats(values: torch.Tensor, top: int, *, n_total: Optional[int] = None, g
     NVLink (b200_rowstats_p2p, GPUs of one node); "nccl": one packed all-reduce per
     pass between the kernels.
     """
+    if values.dtype == torch.float64:
+        if group is not None:
+            raise ValueError("float64 rows are single-GPU")
+        return _rowstats_f64(values, top, n_total, workspace)
     require_cuda()
     if values.dim() != 2 or values.dtype != torch.float32 or not values.is_cuda or values.stride(1) != 1:
         raise ValueError("values must be a [rows,n] float32 CUDA tensor with unit inner stride")

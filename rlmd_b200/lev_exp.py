@@ -22,6 +22,13 @@ caller holds them, then weighted exact statistics of the distinct tuples), the
 GBM one the log-domain sum.  `outcomes` may live on the GPU or in host memory,
 in the reference's dtypes (fp32 {0,1}, int64 {0,1,2}, fp32 x) or the engine's
 (uint8 codes, engine.PackedCodes); host arrays are streamed in row chunks.
+
+Float64 default dtype (`torch.set_default_dtype(torch.float64)` before the reference's
+outcomes are drawn and its functions called): the coin functions, and the GBM ones
+when `outcomes` is float64 too, follow the reference's all-fp64 run - fp64 grid and
+factors, the exact fp64 chain, statistics of the fp64 wealth, float64 tensors back
+(engine.lev_series_f64 / lev_final_f64; one GPU).  Every other function and dtype
+combination runs as under the float32 default.
 """
 from __future__ import annotations
 
@@ -59,6 +66,20 @@ def _grid(lev_low, lev_high, lev_incr, up_r=None, down_r=None) -> np.ndarray:
     if up_r is not None and -down_r > up_r:
         g = -g
     return g
+
+
+def _grid64(lev_low, lev_high, lev_incr, up_r=None, down_r=None) -> np.ndarray:
+    """The grid of the float64 default: T.tensor(param_range(...)) holds the doubles, same negation rule."""
+    g = np.asarray(param_range(lev_low, lev_high, lev_incr), dtype=np.float64)
+    if up_r is not None and -down_r > up_r:
+        g = -g
+    return g
+
+
+def coin_factor_table64(lev: np.ndarray, up_r: float, down_r: float) -> np.ndarray:
+    """[G,2] float64: 1 + lev * r in double (lev/lev_exp.py:85 under a float64 default)."""
+    lev = np.asarray(lev, dtype=np.float64)
+    return np.stack([1.0 + lev * float(down_r), 1.0 + lev * float(up_r)], axis=1)
 
 
 def _lin(lev: np.ndarray, r: float) -> np.ndarray:
@@ -213,6 +234,34 @@ def _n_total(n_local: int, device) -> int:
     return n_local if _GROUP is None else sharding.global_count(n_local, _GROUP, device)
 
 
+def _fp64_coin() -> bool:
+    """The coin follows the all-fp64 run under a float64 default (its values depend on the outcomes only
+    through outcomes == 1, so their dtype does not matter)."""
+    return T.get_default_dtype() == T.float64
+
+
+def _fp64_gbm(outcomes) -> bool:
+    """GBM follows the all-fp64 run under a float64 default with float64 outcomes."""
+    if T.get_default_dtype() != T.float64:
+        return False
+    dt = getattr(outcomes, "dtype", None)
+    if isinstance(dt, T.dtype):
+        return dt == T.float64
+    return dt is not None and np.dtype(dt) == np.float64
+
+
+def _single_gpu_f64() -> None:
+    if _GROUP is not None:
+        raise ValueError("the float64 sweeps (float64 default dtype) run on one GPU: call set_process_group(None) "
+                         "or run under the float32 default")
+
+
+def _returns64(outcomes, device=None) -> T.Tensor:
+    t = T.as_tensor(outcomes)
+    dev = t.device if t.is_cuda else engine._cuda_device(device)
+    return t.to(device=dev, dtype=T.float64).contiguous()
+
+
 def _final_discrete(device, outcomes, table, top, value_0) -> np.ndarray:
     """Statistics [G,12] (in the reference's dtype) of a discrete final-time sweep: the tally path; inputs
     it cannot hold (more distinct count tuples than its plan, horizon >= 2^21) take the general path (LOG
@@ -241,6 +290,13 @@ def _final_discrete(device, outcomes, table, top, value_0) -> np.ndarray:
 # ----------------------------------------------------- fixed final leverage
 def coin_fixed_final_lev(device, outcomes, top, value_0, up_r, down_r, lev_low, lev_high, lev_incr):
     """lev/lev_exp.py:56-125 - prints the final-time statistics per leverage."""
+    if _fp64_coin():
+        _single_gpu_f64()
+        lev = _grid64(lev_low, lev_high, lev_incr, up_r, down_r)
+        stats, _ = engine.lev_final_f64("discrete", coin_factor_table64(lev, up_r, down_r), _as_float(value_0),
+                                        _as_int(top), _codes(outcomes, 2, device))
+        _print_final(lev, stats.cpu().numpy())
+        return
     lev = _grid(lev_low, lev_high, lev_incr, up_r, down_r)
     _print_final(lev, _final_discrete(device, outcomes, coin_factor_table(lev, up_r, down_r), top, value_0))
 
@@ -261,6 +317,12 @@ def dice_sh_fixed_final_lev(device, outcomes, top, value_0, up_r, down_r, mid_r,
 
 def gbm_fixed_final_lev(device, outcomes, top, value_0, lev_low, lev_high, lev_incr):
     """lev/lev_exp.py:935-1005 (no sign flip of the grid).  Host outcomes are streamed in row chunks."""
+    if _fp64_gbm(outcomes):
+        _single_gpu_f64()
+        lev = _grid64(lev_low, lev_high, lev_incr)
+        stats, _ = engine.lev_final_f64("gbm", lev, _as_float(value_0), _as_int(top), _returns64(outcomes, device))
+        _print_final(lev, stats.cpu().numpy())
+        return
     lev = _grid(lev_low, lev_high, lev_incr)
     t = T.as_tensor(outcomes)
     dev = t.device if t.is_cuda else engine._cuda_device(device)
@@ -278,16 +340,24 @@ def gbm_fixed_final_lev(device, outcomes, top, value_0, lev_low, lev_high, lev_i
 
 
 # ------------------------------------------------------------ smart leverage
-def _series(kind, outcomes, table, lev, investors, horizon, top, value_0) -> Tuple[T.Tensor, T.Tensor]:
+def _series(kind, outcomes, table, lev, investors, horizon, top, value_0, dtype=T.float32) -> Tuple[T.Tensor, T.Tensor]:
     n, h = outcomes.shape
     if (investors is not None and _as_int(investors) != n) or (horizon is not None and _as_int(horizon) != h):
         raise ValueError("investors/horizon do not match the shape of outcomes")
     return engine.lev_series(kind, table, lev, _as_float(value_0), int(top), outcomes=outcomes,
-                             n_total=_n_total(n, outcomes.device), group=_GROUP)
+                             n_total=_n_total(n, outcomes.device), group=_GROUP, dtype=dtype)
 
 
 def coin_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, down_r, lev_low, lev_high, lev_incr):
-    """lev/lev_exp.py:128-237 -> (data [L,13,H-1], data_T [L,N]), fp32 on the GPU."""
+    """lev/lev_exp.py:128-237 -> (data [L,13,H-1], data_T [L,N]), fp32 on the GPU (float64 under a float64
+    default dtype)."""
+    if _fp64_coin():
+        _single_gpu_f64()
+        lev = _grid64(lev_low, lev_high, lev_incr, up_r, down_r)
+        data, data_T = _series("discrete", _codes(outcomes, 2, device), coin_factor_table64(lev, up_r, down_r),
+                               lev, investors, horizon, top, value_0, T.float64)
+        _print_final(lev, data[:, :12, -1].cpu().numpy(), smart=True)
+        return data, data_T
     lev = _grid(lev_low, lev_high, lev_incr, up_r, down_r)
     data, data_T = _series("discrete", _codes(outcomes, 2, device), coin_factor_table(lev, up_r, down_r), lev, investors,
                            horizon, top, value_0)
@@ -316,7 +386,14 @@ def dice_sh_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, 
 
 
 def gbm_smart_lev(device, outcomes, investors, horizon, top, value_0, lev_low, lev_high, lev_incr):
-    """lev/lev_exp.py:1008-1118."""
+    """lev/lev_exp.py:1008-1118 (float64 under a float64 default dtype with float64 outcomes)."""
+    if _fp64_gbm(outcomes):
+        _single_gpu_f64()
+        lev = _grid64(lev_low, lev_high, lev_incr)
+        data, data_T = _series("gbm", _returns64(outcomes, device), lev, lev, investors, horizon, top, value_0,
+                               T.float64)
+        _print_final(lev, data[:, :12, -1].cpu().numpy())
+        return data, data_T
     lev = _grid(lev_low, lev_high, lev_incr)
     data, data_T = _series("gbm", _returns(outcomes, device), lev, lev, investors, horizon, top, value_0)
     _print_final(lev, data[:, :12, -1].double().cpu().numpy())

@@ -2,8 +2,9 @@
 The experiment section of the reference's `lev/*.py` scripts as callable
 functions: same defaults, same sequence of `lev_exp` calls, and the same
 on-disk contract - `<name>_inv1_val.npy`, `<name>_inv1_val_T.npy`,
-`<name>_inv{2,3}_val.npy`, `coin_inv4_lev.npy` with identical shapes and fp32
-dtype - so that the reference's plotting stage (`plotting/plots_multiverse.py`,
+`<name>_inv{2,3}_val.npy`, `coin_inv4_lev.npy` with identical shapes and the
+dtype of the tensors saved (fp32; the inv1 arrays of the float64 paths of
+`lev_exp` are float64) - so that the reference's plotting stage (`plotting/plots_multiverse.py`,
 `lev/coin_flip.py:244-283`) runs on the engine's output unchanged.
 
 Reference: lev/coin_flip.py:54-241, lev/dice_roll.py:54-218,
@@ -94,7 +95,10 @@ def _report(t0: float) -> None:
 @_reusing_codes
 def coin_flip(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
               galaxy: bool = True, **overrides) -> Dict[str, np.ndarray]:
-    """lev/coin_flip.py:154-241 -> coin_inv1_val[_T], coin_inv2_val, coin_inv3_val, coin_inv4_lev."""
+    """lev/coin_flip.py:154-241 -> coin_inv1_val[_T], coin_inv2_val, coin_inv3_val, coin_inv4_lev.
+
+    Under a float64 default dtype coin_inv1_val[_T] are float64, as the reference's np.save of its fp64
+    tensors (lev_exp's all-fp64 coin path); the big-brain and Kelly arrays stay fp32."""
     c = _cfg(COIN, overrides)
     dev = T.device("cuda")
     t0 = time.perf_counter()
@@ -167,7 +171,11 @@ def dice_roll_sh(path_results: Optional[str] = "./results/multiverse/", *, seed:
 
 def gbm(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
         **overrides) -> Dict[str, np.ndarray]:
-    """lev/gbm.py:112-157 -> {gbm_op,gbm_snp}_inv1_val[_T]; `outcomes` = one array per environment."""
+    """lev/gbm.py:112-157 -> {gbm_op,gbm_snp}_inv1_val[_T]; `outcomes` = one array per environment.
+
+    The engine's own draws (engine.lev_draw) are float32, so without `outcomes` the sweeps run the float32
+    path whatever the default dtype; float64 arrays injected under a float64 default take lev_exp's all-fp64
+    GBM path and the inv1 files are float64."""
     c = _cfg(GBM, overrides)
     dev = T.device("cuda")
     n, h = c["investors"], c["horizon"]
