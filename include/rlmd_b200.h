@@ -351,6 +351,47 @@ int b200_lev_chunk_f64(const b200_lev_desc* desc, const void* outcomes,
                        double* state, double* dump, void* stream);
 
 /* ------------------------------------------------------------------ *
+ * Per-step series of the coin from the up-move count lattice
+ *
+ * Sits behind coin_smart_lev (lev/lev_exp.py:128-237) when the caller opts in
+ * (method="counts"): after step t an investor with k_t up-moves in steps 0..t
+ * holds V0 u^k d^(t+1-k) at every leverage - monotone in k - so the 12
+ * statistics of every leverage at step t follow from one integer histogram
+ * hist[t][k].  The caller walks the horizon in chunks: count, then stats.
+ * ------------------------------------------------------------------ */
+/* One read of steps [t_begin, t_end) of the outcomes.
+ * outcomes : outcome_bits = 8: uint8 codes [N, ld] (up = code & 1, the column of
+ *            the factor table [G,2] = (down, up)); outcome_bits = 1: one bit per
+ *            flip (b200_lev_pack_bits' layout; ld in bytes, a multiple of 4).
+ * k_state  : int32 [N] up-moves in steps 0..t_begin-1 (ignored when t_begin == 0);
+ *            on return, in steps 0..t_end-1.
+ * hist     : int32 [t_end - t_begin, ld_hist], ld_hist >= horizon + 1, overwritten:
+ *            row i = investors per k after step t_begin + i.
+ * kmin/kmax: int32 [t_end - t_begin]: the occupied band of each row. */
+int b200_coin_lattice_count(const void* outcomes, int64_t n_investors, int32_t horizon,
+                            int64_t ld_outcomes, int32_t outcome_bits, int32_t t_begin,
+                            int32_t t_end, int32_t* k_state, int32_t* hist, int64_t ld_hist,
+                            int32_t* kmin, int32_t* kmax, void* stream);
+/* The 12 statistics (b200_rowstats order and definitions, torch's non-finite rules,
+ * 1 <= top <= n_investors; top == n_investors: the adj group is NaN) of every
+ * leverage g and step t_begin + i from b200_coin_lattice_count's rows for those steps:
+ * the wealth of bin k is exp(log_v0 + k log u + (t+1-k) log d) in fp64, rounded to
+ * fp32 when round_f32; exact ranks by the cumulative counts, fp64 moments.
+ * logs_host : HOST double [G,2] = (log d, log u) of each leverage (G <= B200_MAX_GRID).
+ * stats     : double [G, n_steps, 12].
+ * fails     : int32 [G], NOT cleared: += the steps at which leverage g fails the
+ *             route rule - an extreme path (kmin[t] or kmax[t]) not strictly inside
+ *             (FLT_MIN, FLT_MAX) (round_f32) / (DBL_MIN, DBL_MAX), with a margin of
+ *             1e-3 in log space, or a log that is not finite.  The chain saturates
+ *             path by path (inf and 0 absorb), the lattice does not: only a leverage
+ *             that never fails may take the lattice's statistics. */
+int b200_coin_lattice_stats(const int32_t* hist, int64_t ld_hist, const int32_t* kmin,
+                            const int32_t* kmax, int32_t t_begin, int32_t n_steps,
+                            const double* logs_host, int32_t n_grid, double log_v0,
+                            int32_t round_f32, int64_t n_investors, int64_t top,
+                            double* stats, int32_t* fails, void* stream);
+
+/* ------------------------------------------------------------------ *
  * Batched multiplicative environment step (K4)
  *
  * Sits behind the gym.Env classes of envs/coin_flip_envs.py (Coin_Inv{A,B,C}

@@ -249,6 +249,9 @@ _SIGNATURES = {
     "b200_rowstats_f64_workspace_bytes": (_i64, [_i64]),
     "b200_rowstats_f64": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp]),
     "b200_lev_chunk_f64": (C.c_int, [C.POINTER(LevDesc), _vp, C.POINTER(C.c_double), _i32, _i32, _vp, _vp, _vp]),
+    "b200_coin_lattice_count": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _i32, _i32, _vp, _vp, _i64, _vp, _vp, _vp]),
+    "b200_coin_lattice_stats": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, C.POINTER(C.c_double), _i32, C.c_double,
+                                          _i32, _i64, _i64, _vp, _vp, _vp]),
 }
 # extended below as entry points are added; tests/test_cabi.py checks that every
 # symbol declared in include/rlmd_b200.h is listed here and exported.

@@ -411,6 +411,7 @@ def lev_series(
     group=None,
     device=None,
     dtype: torch.dtype = torch.float32,
+    method: str = "chain",
 ):
     """
     Per-step statistics of the whole grid (the *_smart_lev contract):
@@ -425,7 +426,19 @@ def lev_series(
     With `group`, the rows are investor shards and the statistics are global.
     A chunk is up to `chunk_bytes` (8 GB of the 180) and 2048 rows: the statistics'
     launch and cross-GPU latencies (4 exchange steps per chunk) are paid once per chunk.
+    method="counts": the two-outcome gamble (factors [G,2], streamed uint8 codes, one GPU) from the
+    up-move count lattice - coin_series_counts; `chunk_steps` is then its histogram chunk.
     """
+    if method == "counts":
+        f = np.asarray(factors)
+        if kind != "discrete" or f.ndim != 2 or f.shape[1] != 2 or not isinstance(outcomes, torch.Tensor):
+            raise ValueError('method="counts" is the two-outcome discrete gamble\'s, from streamed uint8 codes')
+        if group is not None or (n_total is not None and int(n_total) != outcomes.shape[0]):
+            raise ValueError('method="counts" runs on one GPU')
+        data, data_T, _ = coin_series_counts(f, lev_row, value_0, top, outcomes, dtype=dtype, chunk_steps=chunk_steps)
+        return data, data_T
+    if method != "chain":
+        raise ValueError("method must be 'chain' or 'counts'")
     if dtype == torch.float64:
         if group is not None:
             raise ValueError("float64 sweeps are single-GPU")
@@ -563,6 +576,156 @@ def lev_final_f64(kind: str, factors, value_0: float, top: int, outcomes: torch.
                                      ptr(data_T), None, stream_ptr()))
         stats = rowstats(data_T, top) if n > 0 else torch.full((g, 12), float("nan"), dtype=torch.float64, device=dev)
     return stats, data_T
+
+
+def coin_lattice_count(outcomes, t_begin: int, t_end: int, k_state: torch.Tensor, *,
+                       hist: Optional[torch.Tensor] = None, kmin: Optional[torch.Tensor] = None,
+                       kmax: Optional[torch.Tensor] = None):
+    """
+    Steps [t_begin, t_end) of a coin's up-move count lattice (b200_coin_lattice_count): one read of the
+    outcomes - uint8 codes [N,H] (up = code & 1) or PackedCodes with bits = 1 - into hist int32
+    [t_end - t_begin, H + 1] (row i: investors per up-move count k after step t_begin + i) and the occupied
+    band kmin / kmax int32 [t_end - t_begin].  k_state int32 [N] carries each investor's count from one call
+    to the next (read when t_begin > 0, updated in place).  hist / kmin / kmax may be passed to reuse buffers
+    (at least that many rows).  Returns (hist, kmin, kmax) views of exactly t_end - t_begin rows.
+    """
+    require_cuda()
+    packed = isinstance(outcomes, PackedCodes)
+    data = outcomes.data if packed else outcomes
+    if packed and outcomes.bits != 1:
+        raise ValueError("the lattice reads uint8 codes or one-bit PackedCodes")
+    if not packed and (not outcomes.is_cuda or outcomes.dtype != torch.uint8 or outcomes.dim() != 2
+                       or outcomes.stride(1) != 1):
+        raise ValueError("outcomes must be a [N,H] uint8 CUDA tensor with unit inner stride (or one-bit PackedCodes)")
+    n, h = outcomes.shape
+    steps = int(t_end) - int(t_begin)
+    dev = data.device
+    if tuple(k_state.shape) != (n,) or k_state.dtype != torch.int32 or not k_state.is_contiguous():
+        raise ValueError("k_state must be a contiguous int32 [N] tensor")
+    with torch.cuda.device(dev):
+        if hist is None:
+            hist = torch.empty((max(steps, 1), h + 1), dtype=torch.int32, device=dev)
+        if kmin is None:
+            kmin = torch.empty(max(steps, 1), dtype=torch.int32, device=dev)
+        if kmax is None:
+            kmax = torch.empty(max(steps, 1), dtype=torch.int32, device=dev)
+        if hist.dim() != 2 or hist.shape[0] < steps or hist.shape[1] < h + 1 or hist.dtype != torch.int32 \
+                or hist.stride(1) != 1 or kmin.shape[0] < steps or kmax.shape[0] < steps:
+            raise ValueError("hist must be int32 [>= steps, >= H + 1] with unit inner stride, kmin / kmax [>= steps]")
+        ld = data.stride(0) if n > 1 else data.shape[1]
+        check(lib.b200_coin_lattice_count(ptr(data), n, h, ld, 1 if packed else 8, int(t_begin), int(t_end),
+                                          ptr(k_state), ptr(hist), hist.stride(0), ptr(kmin), ptr(kmax), stream_ptr()))
+    return hist[:steps], kmin[:steps], kmax[:steps]
+
+
+def coin_lattice_logs(factors, value_0: float, dtype: torch.dtype = torch.float32):
+    """(log V0, logs [G,2] = (log d, log u)) of the factor table [G,2] = (down, up) as the series holds it (fp32
+    values in fp32 mode, with the fp32 V0); nan for a factor <= 0 (such a leverage never takes the lattice)."""
+    f = np.asarray(factors, dtype=np.float32 if dtype == torch.float32 else np.float64).astype(np.float64)
+    v0 = float(np.float32(value_0)) if dtype == torch.float32 else float(value_0)
+    logs = np.array([[math.log(x) if x > 0 else math.nan for x in row] for row in f], dtype=np.float64)
+    return math.log(v0), np.ascontiguousarray(logs.reshape(-1, 2))
+
+
+def coin_lattice_stats(hist: torch.Tensor, kmin: torch.Tensor, kmax: torch.Tensor, t_begin: int, factors,
+                       value_0: float, top: int, n_investors: int, *, dtype: torch.dtype = torch.float32,
+                       fails: Optional[torch.Tensor] = None):
+    """
+    The 12 statistics (rowstats' order and definitions) of every leverage at steps t_begin .. t_begin + T - 1
+    from coin_lattice_count's rows for those steps (b200_coin_lattice_stats): float64 [G, T, 12].  The lattice
+    value is fl32-rounded when dtype is float32.  `fails` int32 [G] (created zeroed when None) is incremented
+    at every step where a leverage fails the route rule (an extreme path outside the dtype's normal range);
+    returns (stats, fails).
+    """
+    require_cuda()
+    lv0, logs = coin_lattice_logs(factors, value_0, dtype)
+    g = logs.shape[0]
+    steps = hist.shape[0]
+    dev = hist.device
+    with torch.cuda.device(dev):
+        if fails is None:
+            fails = torch.zeros(g, dtype=torch.int32, device=dev)
+        stats = torch.empty((g, steps, 12), dtype=torch.float64, device=dev)
+        check(lib.b200_coin_lattice_stats(ptr(hist), hist.stride(0), ptr(kmin), ptr(kmax), int(t_begin), steps,
+                                          logs.ctypes.data_as(C.POINTER(C.c_double)), g, lv0,
+                                          int(dtype == torch.float32), int(n_investors), int(top), ptr(stats),
+                                          ptr(fails), stream_ptr()))
+    return stats, fails
+
+
+def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: torch.Tensor, *,
+                       dtype: torch.dtype = torch.float32, chunk_steps: Optional[int] = None,
+                       chunk_bytes: int = 256 << 20):
+    """
+    lev_series of the coin (factors [G,2] = (down, up), uint8 codes [N,H] on the GPU) from the up-move count
+    lattice: returns (data [G,13,H-1], data_T [G,N], routed bool [G]) with lev_series' layout and dtype
+    (float32, or float64 = lev_series_f64's all-fp64 run).
+
+    Wealth after step t is V0 u^k d^(t+1-k), so every leverage's statistics at step t follow from one
+    histogram of k (coin_lattice_count, walked in chunks of `chunk_steps` steps - by default as many as fit
+    `chunk_bytes` of histogram - then coin_lattice_stats) instead of a dump of every investor's wealth.
+    A leverage is routed - its columns 0..H-3 come from the lattice - when its factors are > 0 and both
+    extreme paths stay inside the dtype's normal range at every step (the chain saturates path by path, the
+    closed form does not); the others take lev_series on their sub-grid.  data_T of every leverage is the
+    exact chain (lev_sweep "chain" / lev_final_f64), and the last column is its row statistics: both are
+    bit-identical to lev_series'.
+    """
+    require_cuda()
+    if dtype not in (torch.float32, torch.float64):
+        raise ValueError("dtype must be torch.float32 or torch.float64")
+    fp64 = dtype == torch.float64
+    f = np.ascontiguousarray(factors, dtype=np.float64 if fp64 else np.float32)
+    if f.ndim != 2 or f.shape[1] != 2:
+        raise ValueError("the lattice is the two-outcome gamble's: factors [G,2] = (down, up)")
+    if not isinstance(outcomes, torch.Tensor) or not outcomes.is_cuda or outcomes.dtype != torch.uint8 \
+            or outcomes.dim() != 2 or outcomes.stride(1) != 1:
+        raise ValueError("outcomes must be a [N,H] uint8 CUDA tensor with unit inner stride (engine.encode_codes)")
+    lev_row = np.asarray(lev_row, dtype=np.float64 if fp64 else np.float32)
+    g = f.shape[0]
+    n, h = outcomes.shape
+    dev = outcomes.device
+    if n == 0:
+        data, data_T = lev_series("discrete", f, lev_row, value_0, top, outcomes=outcomes, dtype=dtype)
+        return data, data_T, np.zeros(g, dtype=bool)
+    with torch.cuda.device(dev):
+        if fp64:
+            last, data_T = lev_final_f64("discrete", f, value_0, top, outcomes)
+        else:
+            data_T = lev_sweep("discrete", f, value_0, outcomes=outcomes, mode="chain")["data_T"]
+            last = stats_to_reference_dtype(rowstats(data_T, top), n, top)
+        data = torch.zeros((g, 13, max(h - 1, 0)), dtype=dtype, device=dev)
+        if h > 1:
+            data[:, 12, :] = torch.as_tensor(lev_row, device=dev)[:, None]
+        routed = (f > 0).all(axis=1)
+        lat = np.flatnonzero(routed)
+        if lat.size:
+            if chunk_steps is None:
+                chunk_steps = chunk_bytes // (4 * (h + 1))
+            tc = max(1, min(int(chunk_steps), h))
+            k_state = torch.empty(n, dtype=torch.int32, device=dev)
+            hist = torch.empty((tc, h + 1), dtype=torch.int32, device=dev)
+            kmin = torch.empty(tc, dtype=torch.int32, device=dev)
+            kmax = torch.empty(tc, dtype=torch.int32, device=dev)
+            fails = torch.zeros(lat.size, dtype=torch.int32, device=dev)
+            sel = torch.as_tensor(lat, device=dev)
+            for t0 in range(0, h, tc):          # every step: a saturation at any step decides the route
+                t1 = min(h, t0 + tc)
+                hs, lo, hi = coin_lattice_count(outcomes, t0, t1, k_state, hist=hist, kmin=kmin, kmax=kmax)
+                st, _ = coin_lattice_stats(hs, lo, hi, t0, f[lat], value_0, top, n, dtype=dtype, fails=fails)
+                c0, c1 = max(t0, 1), min(t1, h - 1)      # steps 1..H-2 -> columns 0..H-3
+                if c1 > c0:
+                    st = st[:, c0 - t0:c1 - t0]
+                    if not fp64:
+                        st = stats_to_reference_dtype(st, n, top)
+                    data[sel, :12, c0 - 1:c1 - 1] = st.permute(0, 2, 1)
+            routed[lat] = fails.cpu().numpy() == 0
+        rest = np.flatnonzero(~routed)
+        if rest.size:
+            sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes, dtype=dtype)
+            data[torch.as_tensor(rest, device=dev)] = sub
+        if h > 1:
+            data[:, :12, h - 2] = last
+    return data, data_T, routed
 
 
 _copy_streams = {}

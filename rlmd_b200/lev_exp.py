@@ -340,27 +340,70 @@ def gbm_fixed_final_lev(device, outcomes, top, value_0, lev_low, lev_high, lev_i
 
 
 # ------------------------------------------------------------ smart leverage
-def _series(kind, outcomes, table, lev, investors, horizon, top, value_0, dtype=T.float32) -> Tuple[T.Tensor, T.Tensor]:
+def _series(kind, outcomes, table, lev, investors, horizon, top, value_0, dtype=T.float32,
+            method="chain") -> Tuple[T.Tensor, T.Tensor]:
     n, h = outcomes.shape
     if (investors is not None and _as_int(investors) != n) or (horizon is not None and _as_int(horizon) != h):
         raise ValueError("investors/horizon do not match the shape of outcomes")
+    if method == "counts":
+        return engine.lev_series(kind, table, lev, _as_float(value_0), int(top), outcomes=outcomes, dtype=dtype,
+                                 method="counts")
     return engine.lev_series(kind, table, lev, _as_float(value_0), int(top), outcomes=outcomes,
                              n_total=_n_total(n, outcomes.device), group=_GROUP, dtype=dtype)
 
 
-def coin_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, down_r, lev_low, lev_high, lev_incr):
+_SERIES_METHOD = ["chain"]
+
+
+class series_method:
+    """
+    `with lev_exp.series_method("counts"):` - inside the block coin_smart_lev computes its per-step statistics
+    from the up-move count lattice (engine.coin_series_counts) unless a call passes `method` itself, so an
+    unmodified script that reaches this module through sys.modules opts in without a change.  "chain" (the
+    default outside any block) is the reference's sequential product for every column.  Blocks nest.
+    """
+
+    def __init__(self, method: str):
+        self.method = _series_method(method)
+
+    def __enter__(self):
+        _SERIES_METHOD.append(self.method)
+        return self
+
+    def __exit__(self, *exc):
+        _SERIES_METHOD.pop()
+        return False
+
+
+def _series_method(method) -> str:
+    if method not in ("chain", "counts"):
+        raise ValueError("method must be 'chain' or 'counts'")
+    return method
+
+
+def coin_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, down_r, lev_low, lev_high, lev_incr, *,
+                   method=None):
     """lev/lev_exp.py:128-237 -> (data [L,13,H-1], data_T [L,N]), fp32 on the GPU (float64 under a float64
-    default dtype)."""
+    default dtype).
+
+    method "chain" (default; see series_method): the exact sequential product for every column.  "counts": the
+    columns of every leverage whose paths stay inside the dtype's normal range come from the up-move count
+    lattice (engine.coin_series_counts: the same statistics of the closed-form wealth V0 u^k d^(t+1-k), within
+    rounding of the chain's, without a pass over every investor's wealth per step); data_T, the last column and
+    the printed text are the chain's, bit for bit.  One GPU: ValueError under set_process_group."""
+    method = _series_method(_SERIES_METHOD[-1] if method is None else method)
+    if method == "counts" and _GROUP is not None:
+        raise ValueError('method="counts" runs on one GPU: call set_process_group(None) or use method="chain"')
     if _fp64_coin():
         _single_gpu_f64()
         lev = _grid64(lev_low, lev_high, lev_incr, up_r, down_r)
         data, data_T = _series("discrete", _codes(outcomes, 2, device), coin_factor_table64(lev, up_r, down_r),
-                               lev, investors, horizon, top, value_0, T.float64)
+                               lev, investors, horizon, top, value_0, T.float64, method)
         _print_final(lev, data[:, :12, -1].cpu().numpy(), smart=True)
         return data, data_T
     lev = _grid(lev_low, lev_high, lev_incr, up_r, down_r)
     data, data_T = _series("discrete", _codes(outcomes, 2, device), coin_factor_table(lev, up_r, down_r), lev, investors,
-                           horizon, top, value_0)
+                           horizon, top, value_0, method=method)
     _print_final(lev, data[:, :12, -1].double().cpu().numpy(), smart=True)
     return data, data_T
 

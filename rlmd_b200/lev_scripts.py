@@ -94,11 +94,12 @@ def _report(t0: float) -> None:
 
 @_reusing_codes
 def coin_flip(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
-              galaxy: bool = True, **overrides) -> Dict[str, np.ndarray]:
+              galaxy: bool = True, series: str = "chain", **overrides) -> Dict[str, np.ndarray]:
     """lev/coin_flip.py:154-241 -> coin_inv1_val[_T], coin_inv2_val, coin_inv3_val, coin_inv4_lev.
 
     Under a float64 default dtype coin_inv1_val[_T] are float64, as the reference's np.save of its fp64
-    tensors (lev_exp's all-fp64 coin path); the big-brain and Kelly arrays stay fp32."""
+    tensors (lev_exp's all-fp64 coin path); the big-brain and Kelly arrays stay fp32.
+    series: coin_smart_lev's method ("chain" or "counts", the up-move count lattice)."""
     c = _cfg(COIN, overrides)
     dev = T.device("cuda")
     t0 = time.perf_counter()
@@ -108,7 +109,8 @@ def coin_flip(path_results: Optional[str] = "./results/multiverse/", *, seed: in
     out: Dict[str, np.ndarray] = {}
     lf = _lev_factor(c["up_r"], c["down_r"], c["asym_lim"])
     lev_exp.coin_fixed_final_lev(dev, outcomes, c["top"], c["value_0"], c["up_r"], c["down_r"], *c["l0"])
-    d, dT = lev_exp.coin_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], c["up_r"], c["down_r"], *c["l1"])
+    d, dT = lev_exp.coin_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], c["up_r"], c["down_r"], *c["l1"],
+                                   method=series)
     _save(path_results, "coin_inv1_val", d, out)
     _save(path_results, "coin_inv1_val_T", dT, out)
     for tag, s, r in (("coin_inv2_val", c["s2"], c["r2"]), ("coin_inv3_val", c["s3"], c["r3"])):
