@@ -392,6 +392,41 @@ int b200_coin_lattice_stats(const int32_t* hist, int64_t ld_hist, const int32_t*
                             double* stats, int32_t* fails, void* stream);
 
 /* ------------------------------------------------------------------ *
+ * Per-step series of GBM from the running log-return sum
+ *
+ * Sits behind gbm_smart_lev (lev/lev_exp.py:1012-1120) when the caller opts in
+ * (method="sum"): log wealth after step t is log V0 + l S_t at every leverage l,
+ * S_t the running sum of the investor's log-returns, so one exact select on S_t
+ * gives the order statistics of every leverage (the order reverses for l < 0)
+ * and two passes over S_t its moments.  The caller walks the horizon in chunks:
+ * S rows, then stats.
+ * ------------------------------------------------------------------ */
+/* Steps [t_begin, t_end) of x [N, ld_x] (x_f64 = 0: float, 1: double) into
+ * S double [t_end - t_begin, ld_S] (row i = S after step t_begin + i).
+ * state : double [3,N] = S, its running max and min (0 before step 0 counts),
+ *         in/out (ignored as input when t_begin == 0).
+ * float x: S is b200_lev_chunk's (32 steps in fp32 on the fp64 base, folded
+ * when (t & 31) == 31), bit for bit; t_begin must be a multiple of 32.
+ * double x: the sequential fp64 sum.  S may be NULL: advance the state only. */
+int b200_gbm_sum_chunk(const void* x, int32_t x_f64, int64_t n_investors, int32_t horizon,
+                       int64_t ld_x, int32_t t_begin, int32_t t_end, double* state, double* S,
+                       int64_t ld_S, void* stream);
+/* bytes of device workspace b200_gbm_sum_stats needs */
+int64_t b200_gbm_sum_stats_workspace_bytes(int64_t rows, int64_t n, int32_t n_grid);
+/* The 12 statistics (b200_rowstats order and definitions, torch's non-finite rules,
+ * 1 <= top <= n; top == n: the adj group is NaN) of the wealth
+ * w = exp(log_v0 + l * S) (rounded to fp32 when round_f32: gbm_smart_lev's chain
+ * wealth bit for bit) of every leverage l and every row of S double [rows, ld].
+ * Exact order statistics (select on S at the ranks and, for a grid with an l < 0,
+ * their mirrors), fp64 moments; the same statistics however the rows are chunked.
+ * lev_host : HOST double [n_grid] (n_grid <= B200_MAX_GRID).
+ * stats    : double [n_grid, rows, 12]. */
+int b200_gbm_sum_stats(const double* S, int64_t rows, int64_t n, int64_t ld,
+                       const double* lev_host, int32_t n_grid, double log_v0,
+                       int32_t round_f32, int64_t top, void* workspace, double* stats,
+                       void* stream);
+
+/* ------------------------------------------------------------------ *
  * Batched multiplicative environment step (K4)
  *
  * Sits behind the gym.Env classes of envs/coin_flip_envs.py (Coin_Inv{A,B,C}

@@ -472,4 +472,31 @@ static int chain_launch_all(const ChainLaunch& a0) {
   return dump ? chain_launch_gt<K, V_FSEL, true>(a) : chain_launch_gt<K, V_FSEL, false>(a);
 }
 
+// GBM: the running sum S of the log-returns, 32 steps in fp32 relative to the fp64 base, then
+// folded into the base.  The LOG sweep, the series chunks (lev_sweep.cu) and the sum route
+// (gbm_sum.cu) all accumulate through this one struct, so their S agree bit for bit.
+struct GbmAcc {
+  double S = 0.0, Smax = 0.0, Smin = 0.0;  // running sum and its extremes (t >= 0; start value 0)
+  float p = 0.f, pmax = -3.0e38f, pmin = 3.0e38f;
+  __device__ __forceinline__ void step(float x) {
+    p += x;
+    pmax = fmaxf(pmax, p);
+    pmin = fminf(pmin, p);
+  }
+  // two steps: the running extremes take both partial sums in ONE three-input min / max each
+  // (FMNMX3, sm_100) - 4 instructions per pair instead of 6, the same values bit for bit
+  __device__ __forceinline__ void step2(float x0, float x1) {
+    const float p1 = p + x0;
+    p = p1 + x1;
+    asm("max.f32 %0, %0, %1, %2;" : "+f"(pmax) : "f"(p1), "f"(p));
+    asm("min.f32 %0, %0, %1, %2;" : "+f"(pmin) : "f"(p1), "f"(p));
+  }
+  __device__ __forceinline__ void fold() {
+    Smax = fmax(Smax, S + (double)pmax);
+    Smin = fmin(Smin, S + (double)pmin);
+    S += (double)p;
+    p = 0.f; pmax = -3.0e38f; pmin = 3.0e38f;
+  }
+};
+
 }  // namespace b200

@@ -451,31 +451,6 @@ __device__ __forceinline__ void gbm_finish(double S, double Smax, double Smin, i
   }
 }
 
-// 32 steps in fp32 relative to the fp64 base, then fold into the base.
-struct GbmAcc {
-  double S = 0.0, Smax = 0.0, Smin = 0.0;  // running sum and its extremes (t >= 0; start value 0)
-  float p = 0.f, pmax = -3.0e38f, pmin = 3.0e38f;
-  __device__ __forceinline__ void step(float x) {
-    p += x;
-    pmax = fmaxf(pmax, p);
-    pmin = fminf(pmin, p);
-  }
-  // two steps: the running extremes take both partial sums in ONE three-input min / max each
-  // (FMNMX3, sm_100) - 4 instructions per pair instead of 6, the same values bit for bit
-  __device__ __forceinline__ void step2(float x0, float x1) {
-    const float p1 = p + x0;
-    p = p1 + x1;
-    asm("max.f32 %0, %0, %1, %2;" : "+f"(pmax) : "f"(p1), "f"(p));
-    asm("min.f32 %0, %0, %1, %2;" : "+f"(pmin) : "f"(p1), "f"(p));
-  }
-  __device__ __forceinline__ void fold() {
-    Smax = fmax(Smax, S + (double)pmax);
-    Smin = fmin(Smin, S + (double)pmin);
-    S += (double)p;
-    p = 0.f; pmax = -3.0e38f; pmin = 3.0e38f;
-  }
-};
-
 template <bool USE_TMA>
 __global__ void __launch_bounds__(TILE_ROWS)
 log_gbm_stream_kernel(const __grid_constant__ CUtensorMap tmap, const float* __restrict__ x, int64_t ld,

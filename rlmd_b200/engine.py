@@ -9,6 +9,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+import sys
 from typing import Optional, Sequence
 
 import numpy as np
@@ -428,6 +429,8 @@ def lev_series(
     launch and cross-GPU latencies (4 exchange steps per chunk) are paid once per chunk.
     method="counts": the two-outcome gamble (factors [G,2], streamed uint8 codes, one GPU) from the
     up-move count lattice - coin_series_counts; `chunk_steps` is then its histogram chunk.
+    method="sum": GBM (streamed log-returns, one GPU) from the running log-return sum -
+    gbm_series_sum; `chunk_steps` is then its S chunk.
     """
     if method == "counts":
         f = np.asarray(factors)
@@ -437,8 +440,15 @@ def lev_series(
             raise ValueError('method="counts" runs on one GPU')
         data, data_T, _ = coin_series_counts(f, lev_row, value_0, top, outcomes, dtype=dtype, chunk_steps=chunk_steps)
         return data, data_T
+    if method == "sum":
+        if kind != "gbm" or not isinstance(outcomes, torch.Tensor):
+            raise ValueError('method="sum" is GBM\'s, from streamed log-returns')
+        if group is not None or (n_total is not None and int(n_total) != outcomes.shape[0]):
+            raise ValueError('method="sum" runs on one GPU')
+        data, data_T, _ = gbm_series_sum(factors, lev_row, value_0, top, outcomes, dtype=dtype, chunk_steps=chunk_steps)
+        return data, data_T
     if method != "chain":
-        raise ValueError("method must be 'chain' or 'counts'")
+        raise ValueError("method must be 'chain', 'counts' or 'sum'")
     if dtype == torch.float64:
         if group is not None:
             raise ValueError("float64 sweeps are single-GPU")
@@ -723,6 +733,213 @@ def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: tor
         if rest.size:
             sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes, dtype=dtype)
             data[torch.as_tensor(rest, device=dev)] = sub
+        if h > 1:
+            data[:, :12, h - 2] = last
+    return data, data_T, routed
+
+
+# lev_sweep.cu's saturation bounds of the fp32 chain: inf above ln FLT_MAX, 0 below ln 2^-150
+_LOG_FLT_MAX = 88.72283905206835
+_LOG_FLT_ZERO = -103.97207708399179
+
+
+def gbm_sum_chunk(x: torch.Tensor, t_begin: int, t_end: int, state: torch.Tensor, *,
+                  out: Optional[torch.Tensor] = None, state_only: bool = False) -> Optional[torch.Tensor]:
+    """
+    Steps [t_begin, t_end) of the running log-return sum S (b200_gbm_sum_chunk): x float32 or float64 [N,H] on
+    the GPU -> float64 [t_end - t_begin, N] (row i: S after step t_begin + i).  float32 x: the S of the series
+    chain (b200_lev_chunk) bit for bit, t_begin a multiple of 32; float64 x: the sequential fp64 sum.
+    state float64 [3,N] = (S, running max, running min) carries from one call to the next (read when
+    t_begin > 0, updated in place).  `out` may be passed to reuse a buffer (at least that many rows).
+    state_only: advance the state without writing S rows (returns None).
+    """
+    require_cuda()
+    if not isinstance(x, torch.Tensor) or not x.is_cuda or x.dtype not in (torch.float32, torch.float64) \
+            or x.dim() != 2 or x.stride(1) != 1:
+        raise ValueError("x must be a [N,H] float32 / float64 CUDA tensor with unit inner stride")
+    n, h = x.shape
+    steps = int(t_end) - int(t_begin)
+    if tuple(state.shape) != (3, n) or state.dtype != torch.float64 or not state.is_contiguous():
+        raise ValueError("state must be a contiguous float64 [3,N] tensor")
+    with torch.cuda.device(x.device):
+        ld = x.stride(0) if n > 1 else max(x.stride(0), h)
+        if state_only:
+            check(lib.b200_gbm_sum_chunk(ptr(x), int(x.dtype == torch.float64), n, h, ld, int(t_begin), int(t_end),
+                                         ptr(state), None, max(n, 1), stream_ptr()))
+            return None
+        if out is None:
+            out = torch.empty((max(steps, 1), max(n, 1)), dtype=torch.float64, device=x.device)
+        if out.dim() != 2 or out.dtype != torch.float64 or out.shape[0] < steps or out.shape[1] < n \
+                or out.stride(1) != 1:
+            raise ValueError("out must be float64 [>= steps, >= N] with unit inner stride")
+        check(lib.b200_gbm_sum_chunk(ptr(x), int(x.dtype == torch.float64), n, h, ld, int(t_begin), int(t_end),
+                                     ptr(state), ptr(out), out.stride(0), stream_ptr()))
+    return out[:steps, :n]
+
+
+_GBM_SUM_MAX_ROWS = 2048
+
+
+def gbm_sum_chunk_steps(n: int, n_grid: int, h: int, chunk_steps: Optional[int] = None,
+                        chunk_bytes: int = 256 << 20) -> int:
+    """
+    Steps per chunk of gbm_series_sum: a multiple of 32 (fp32 chunks start where the partial sums fold), at most
+    2048 rows (the chain series' cap: a row of the statistics' workspace costs its select histograms whatever N
+    is) and at most the steps the route covers (H - 1, rounded up to 32).  By default as many as fit `chunk_bytes`
+    of S rows plus workspace; an explicit `chunk_steps` is rounded down to 32 and capped the same way.
+    """
+    if chunk_steps is None:
+        per_row = 8 * max(n, 1) + lib.b200_gbm_sum_stats_workspace_bytes(1, max(n, 1), int(n_grid))
+        chunk_steps = chunk_bytes // per_row
+    tc = max(32, int(chunk_steps) // 32 * 32)
+    return min(tc, _GBM_SUM_MAX_ROWS, _round_up(max(h - 1, 1), 32))
+
+
+def gbm_sum_workspace(rows: int, n: int, n_grid: int, device) -> torch.Tensor:
+    nbytes = lib.b200_gbm_sum_stats_workspace_bytes(int(rows), int(n), int(n_grid))
+    return torch.empty((max(nbytes // 8, 1),), dtype=torch.int64, device=device)
+
+
+def _gbm_log_v0(value_0: float, dtype: torch.dtype) -> float:
+    """log V0 as the chain forms it: of the fp32 V0 in fp32 mode (b200_lev_chunk), of the double in fp64 mode."""
+    return math.log(float(np.float32(value_0)) if dtype == torch.float32 else float(value_0))
+
+
+def gbm_sum_stats(S: torch.Tensor, lev, value_0: float, top: int, *, dtype: torch.dtype = torch.float32,
+                  workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """
+    The 12 statistics (rowstats' order and definitions) of the wealth exp(log V0 + l S) of every leverage l at
+    every row of S float64 [T,N] (b200_gbm_sum_stats): float64 [G, T, 12].  dtype float32: the wealth is rounded
+    to fp32 as the series chain rounds it (lev fp32, V0 fp32), so a leverage whose chain never saturates gets the
+    chain's order statistics bit for bit; float64: the fp64 wealth.  1 <= top <= N (top == N: adj is NaN).
+    """
+    require_cuda()
+    if dtype not in (torch.float32, torch.float64):
+        raise ValueError("dtype must be torch.float32 or torch.float64")
+    if S.dim() != 2 or S.dtype != torch.float64 or not S.is_cuda or S.stride(1) != 1:
+        raise ValueError("S must be a [T,N] float64 CUDA tensor with unit inner stride")
+    lv = np.ascontiguousarray(np.asarray(lev, dtype=np.float32 if dtype == torch.float32 else np.float64)
+                              .reshape(-1), dtype=np.float64)
+    g = lv.shape[0]
+    rows, n = S.shape
+    dev = S.device
+    with torch.cuda.device(dev):
+        stats = torch.empty((g, rows, 12), dtype=torch.float64, device=dev)
+        if rows == 0:
+            return stats
+        ws = workspace if workspace is not None else gbm_sum_workspace(rows, n, g, dev)
+        if ws.numel() * ws.element_size() < lib.b200_gbm_sum_stats_workspace_bytes(rows, n, g):
+            raise ValueError("workspace too small (gbm_sum_workspace)")
+        ld = S.stride(0) if rows > 1 else max(S.stride(0), n)
+        check(lib.b200_gbm_sum_stats(ptr(S), rows, n, ld, lv.ctypes.data_as(C.POINTER(C.c_double)), g,
+                                     _gbm_log_v0(value_0, dtype), int(dtype == torch.float32), int(top), ptr(ws),
+                                     ptr(stats), stream_ptr()))
+    return stats
+
+
+def gbm_sum_routed(state: torch.Tensor, lev, value_0: float, dtype: torch.dtype = torch.float32) -> np.ndarray:
+    """
+    Which leverages may take the running-sum statistics, from state float64 [3,N] = (S, running max, running
+    min) over the steps the statistics cover: every entry finite and, for the global extremes,
+    float32: log V0 + l max S <= ln FLT_MAX and log V0 + l min S >= ln 2^-150 (swapped for l < 0) - the same
+    double arithmetic in which the series chain saturates, so this holds iff no investor's chain saturates;
+    float64: both extreme paths strictly inside (DBL_MIN, DBL_MAX) with a margin of 1e-3 in log space (the fp64
+    chain is a sequential product, not the closed form).
+    """
+    f32 = dtype == torch.float32
+    lv = np.asarray(lev, dtype=np.float32 if f32 else np.float64).reshape(-1)
+    ext = torch.stack([state[1].max(), state[2].min(), torch.isfinite(state).all().to(torch.float64)]).cpu()
+    smax, smin, finite = float(ext[0]), float(ext[1]), bool(ext[2])
+    if not finite:
+        return np.zeros(lv.shape[0], dtype=bool)
+    lv0 = _gbm_log_v0(value_0, dtype)
+    out = np.zeros(lv.shape[0], dtype=bool)
+    for i, l in enumerate(lv):
+        l = float(l)
+        hi = lv0 + (l * smax if l >= 0 else l * smin)
+        lo = lv0 + (l * smin if l >= 0 else l * smax)
+        if f32:
+            out[i] = not (hi > _LOG_FLT_MAX) and not (lo < _LOG_FLT_ZERO)
+        else:
+            out[i] = lo > math.log(sys.float_info.min) + 1e-3 and hi < math.log(sys.float_info.max) - 1e-3
+    return out
+
+
+def gbm_series_sum(lev, lev_row, value_0: float, top: int, x: torch.Tensor, *, dtype: torch.dtype = torch.float32,
+                   chunk_steps: Optional[int] = None, chunk_bytes: int = 256 << 20):
+    """
+    lev_series of GBM (lev [G], log-returns x [N,H] on the GPU: float32, or float64 with dtype float64) from the
+    running log-return sum: returns (data [G,13,H-1], data_T [G,N], routed bool [G]) with lev_series' layout
+    and dtype (float32, or float64 = lev_series_f64's all-fp64 run).
+
+    Log wealth after step t is log V0 + l S_t at every leverage, so the statistics of every leverage at step t
+    follow from S_t alone (gbm_sum_chunk, walked in chunks of gbm_sum_chunk_steps steps - by default as many as
+    fit `chunk_bytes` of S rows and statistics workspace, a multiple of 32, at most 2048 - then gbm_sum_stats) instead of a dump of every investor's wealth.
+    A leverage is routed - its columns 0..H-3 come from S - by gbm_sum_routed: float32, iff its chain never
+    saturates (decided from lev_sweep's LOG state before the walk; its order statistics are then the chain's bit
+    for bit, its moments differ in fp64 summation order); float64, iff its extreme paths stay inside the normal
+    range (decided from a state-only pass over x before the walk).  A horizon of H <= 2 routes nothing: column
+    H-2 is always the chain's.  The others take lev_series on their sub-grid.  data_T is the chain's
+    (float32: the LOG sweep's, which equals it when nothing saturates, and the sub-grid's otherwise; float64:
+    lev_final_f64), and the last column is its row statistics.
+    """
+    require_cuda()
+    if dtype not in (torch.float32, torch.float64):
+        raise ValueError("dtype must be torch.float32 or torch.float64")
+    fp64 = dtype == torch.float64
+    if not isinstance(x, torch.Tensor) or not x.is_cuda or x.dtype != dtype or x.dim() != 2 or x.stride(1) != 1:
+        raise ValueError(f"x must be a [N,H] {dtype} CUDA tensor with unit inner stride")
+    lv = np.ascontiguousarray(lev, dtype=np.float64 if fp64 else np.float32).reshape(-1)
+    lev_row = np.asarray(lev_row, dtype=np.float64 if fp64 else np.float32)
+    g = lv.shape[0]
+    n, h = x.shape
+    dev = x.device
+    if n == 0:
+        data, data_T = lev_series("gbm", lv, lev_row, value_0, top, outcomes=x, dtype=dtype)
+        return data, data_T, np.zeros(g, dtype=bool)
+    hw = h - 1                                  # steps 0..H-2: column H-2 is the last one, from data_T
+    with torch.cuda.device(dev):
+        state = torch.empty((3, n), dtype=torch.float64, device=dev)
+        if fp64:
+            last, data_T = lev_final_f64("gbm", lv, value_0, top, x)
+            if hw > 0:                          # the extremes of S over the steps the route covers, first
+                gbm_sum_chunk(x, 0, hw, state, out=None, state_only=True)
+                routed = gbm_sum_routed(state, lv, value_0, dtype)
+            else:
+                routed = np.zeros(g, dtype=bool)
+        else:
+            res = lev_sweep("gbm", lv, value_0, outcomes=x, mode="log", want_state=True)
+            data_T = res["data_T"]
+            routed = gbm_sum_routed(res["state"], lv, value_0, dtype)
+        if h <= 2:
+            routed[:] = False                   # no column comes from the route
+        data = torch.zeros((g, 13, max(h - 1, 0)), dtype=dtype, device=dev)
+        if h > 1:
+            data[:, 12, :] = torch.as_tensor(lev_row, device=dev)[:, None]
+        sel = np.flatnonzero(routed)
+        if sel.size:
+            tc = gbm_sum_chunk_steps(n, sel.size, h, chunk_steps, chunk_bytes)
+            buf = torch.empty((tc, n), dtype=torch.float64, device=dev)
+            ws = gbm_sum_workspace(tc, n, sel.size, dev)
+            idx = torch.as_tensor(sel, device=dev)
+            for t0 in range(0, hw, tc):
+                t1 = min(hw, t0 + tc)
+                rows = gbm_sum_chunk(x, t0, t1, state, out=buf)
+                c0 = max(t0, 1)                 # steps 1..H-2 -> columns 0..H-3
+                if t1 > c0:
+                    st = gbm_sum_stats(rows[c0 - t0:], lv[sel], value_0, top, dtype=dtype, workspace=ws)
+                    if not fp64:
+                        st = stats_to_reference_dtype(st, n, top)
+                    data[idx, :12, c0 - 1:t1 - 1] = st.permute(0, 2, 1)
+        rest = np.flatnonzero(~routed)
+        if rest.size:
+            sub, sub_T = lev_series("gbm", lv[rest], lev_row[rest], value_0, top, outcomes=x, dtype=dtype)
+            ridx = torch.as_tensor(rest, device=dev)
+            data[ridx] = sub
+            if not fp64:
+                data_T[ridx] = sub_T
+        if not fp64:
+            last = stats_to_reference_dtype(rowstats(data_T, top), n, top)
         if h > 1:
             data[:, :12, h - 2] = last
     return data, data_T, routed

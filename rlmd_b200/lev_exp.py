@@ -345,9 +345,9 @@ def _series(kind, outcomes, table, lev, investors, horizon, top, value_0, dtype=
     n, h = outcomes.shape
     if (investors is not None and _as_int(investors) != n) or (horizon is not None and _as_int(horizon) != h):
         raise ValueError("investors/horizon do not match the shape of outcomes")
-    if method == "counts":
+    if method != "chain":
         return engine.lev_series(kind, table, lev, _as_float(value_0), int(top), outcomes=outcomes, dtype=dtype,
-                                 method="counts")
+                                 method=method)
     return engine.lev_series(kind, table, lev, _as_float(value_0), int(top), outcomes=outcomes,
                              n_total=_n_total(n, outcomes.device), group=_GROUP, dtype=dtype)
 
@@ -359,8 +359,11 @@ class series_method:
     """
     `with lev_exp.series_method("counts"):` - inside the block coin_smart_lev computes its per-step statistics
     from the up-move count lattice (engine.coin_series_counts) unless a call passes `method` itself, so an
-    unmodified script that reaches this module through sys.modules opts in without a change.  "chain" (the
-    default outside any block) is the reference's sequential product for every column.  Blocks nest.
+    unmodified script that reaches this module through sys.modules opts in without a change.  "sum" does the
+    same for gbm_smart_lev (the running log-return sum, engine.gbm_series_sum).  Each function takes the
+    innermost block's method only when it is its own ("counts" for the coin, "sum" for GBM) and "chain"
+    otherwise.  "chain" (the default outside any block) is the reference's sequential product for every
+    column.  Blocks nest.
     """
 
     def __init__(self, method: str):
@@ -376,8 +379,18 @@ class series_method:
 
 
 def _series_method(method) -> str:
-    if method not in ("chain", "counts"):
-        raise ValueError("method must be 'chain' or 'counts'")
+    if method not in ("chain", "counts", "sum"):
+        raise ValueError("method must be 'chain', 'counts' or 'sum'")
+    return method
+
+
+def _call_method(method, own: str) -> str:
+    """The method of one *_smart_lev call whose alternative route is `own`: its `method` ("chain" or `own`),
+    else the innermost series_method block's when that is `own`, else "chain"."""
+    if method is None:
+        return own if _SERIES_METHOD[-1] == own else "chain"
+    if method not in ("chain", own):
+        raise ValueError(f"method must be 'chain' or '{own}'")
     return method
 
 
@@ -391,7 +404,7 @@ def coin_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, dow
     lattice (engine.coin_series_counts: the same statistics of the closed-form wealth V0 u^k d^(t+1-k), within
     rounding of the chain's, without a pass over every investor's wealth per step); data_T, the last column and
     the printed text are the chain's, bit for bit.  One GPU: ValueError under set_process_group."""
-    method = _series_method(_SERIES_METHOD[-1] if method is None else method)
+    method = _call_method(method, "counts")
     if method == "counts" and _GROUP is not None:
         raise ValueError('method="counts" runs on one GPU: call set_process_group(None) or use method="chain"')
     if _fp64_coin():
@@ -428,17 +441,28 @@ def dice_sh_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, 
     return data, data_T
 
 
-def gbm_smart_lev(device, outcomes, investors, horizon, top, value_0, lev_low, lev_high, lev_incr):
-    """lev/lev_exp.py:1008-1118 (float64 under a float64 default dtype with float64 outcomes)."""
+def gbm_smart_lev(device, outcomes, investors, horizon, top, value_0, lev_low, lev_high, lev_incr, *, method=None):
+    """lev/lev_exp.py:1008-1118 (float64 under a float64 default dtype with float64 outcomes).
+
+    method "chain" (default; see series_method): the sequential chain for every column.  "sum": the columns of
+    every leverage whose chain never saturates (float64: whose extreme paths stay inside the normal range) come
+    from the running log-return sum S (engine.gbm_series_sum: log wealth is log V0 + l S, so one select on S per
+    step serves every leverage, without a pass over every investor's wealth per step) - in float32 the order
+    statistics are the chain's bit for bit and the moments differ in fp64 summation order; data_T, the last
+    column and the printed text are the chain's.  One GPU: ValueError under set_process_group."""
+    method = _call_method(method, "sum")
+    if method == "sum" and _GROUP is not None:
+        raise ValueError('method="sum" runs on one GPU: call set_process_group(None) or use method="chain"')
     if _fp64_gbm(outcomes):
         _single_gpu_f64()
         lev = _grid64(lev_low, lev_high, lev_incr)
         data, data_T = _series("gbm", _returns64(outcomes, device), lev, lev, investors, horizon, top, value_0,
-                               T.float64)
+                               T.float64, method)
         _print_final(lev, data[:, :12, -1].cpu().numpy())
         return data, data_T
     lev = _grid(lev_low, lev_high, lev_incr)
-    data, data_T = _series("gbm", _returns(outcomes, device), lev, lev, investors, horizon, top, value_0)
+    data, data_T = _series("gbm", _returns(outcomes, device), lev, lev, investors, horizon, top, value_0,
+                           method=method)
     _print_final(lev, data[:, :12, -1].double().cpu().numpy())
     return data, data_T
 

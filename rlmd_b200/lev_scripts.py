@@ -172,12 +172,13 @@ def dice_roll_sh(path_results: Optional[str] = "./results/multiverse/", *, seed:
 
 
 def gbm(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
-        **overrides) -> Dict[str, np.ndarray]:
+        series: str = "chain", **overrides) -> Dict[str, np.ndarray]:
     """lev/gbm.py:112-157 -> {gbm_op,gbm_snp}_inv1_val[_T]; `outcomes` = one array per environment.
 
     The engine's own draws (engine.lev_draw) are float32, so without `outcomes` the sweeps run the float32
     path whatever the default dtype; float64 arrays injected under a float64 default take lev_exp's all-fp64
-    GBM path and the inv1 files are float64."""
+    GBM path and the inv1 files are float64.
+    series: gbm_smart_lev's method ("chain" or "sum", the running log-return sum)."""
     c = _cfg(GBM, overrides)
     dev = T.device("cuda")
     n, h = c["investors"], c["horizon"]
@@ -190,7 +191,7 @@ def gbm(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 42
                                                                       sigma=vol)
         lev_exp.gbm_fixed_final_lev(dev, oc, c["top"], c["value_0"], c["l0_l"][x], c["l0_h"][x], c["l0_i"][x])
         d, dT = lev_exp.gbm_smart_lev(dev, oc, n, h, c["top"], c["value_0"], c["l1_l"][x], c["l1_h"][x],
-                                      c["l1_i"][x])
+                                      c["l1_i"][x], method=series)
         _save(path_results, c["name"][x] + "_inv1_val", d, out)
         _save(path_results, c["name"][x] + "_inv1_val_T", dT, out)
         del oc
