@@ -392,6 +392,55 @@ int b200_coin_lattice_stats(const int32_t* hist, int64_t ld_hist, const int32_t*
                             double* stats, int32_t* fails, void* stream);
 
 /* ------------------------------------------------------------------ *
+ * Per-step series of the three-outcome gamble from the count-tuple lattice
+ *
+ * Sits behind dice_smart_lev / dice_sh_smart_lev (lev/lev_exp.py:586-701,
+ * :1209-1334) when the caller opts in (method="tuples"): after step t an
+ * investor with a up-moves, b down-moves and c = t+1-a-b mid-moves holds
+ * V0 u^a d^b m^c at every leverage, so the 12 statistics of every leverage at
+ * step t follow from one integer histogram over the occupied (a, b) cells.
+ * The caller walks the codes once for the bounds, lays every step's box out
+ * flat, then walks them again in chunks: count, then stats.
+ * outcomes: uint8 codes [N, ld] (0 up, 1 down, 2 mid: the columns of the factor
+ * table [G,3]), unit inner stride, any ld >= horizon.
+ * ab_state: int32 [2,N] = each investor's (a, b) over steps 0..t_begin-1 (ignored
+ * when t_begin == 0); on return, over steps 0..t_end-1.
+ * bounds  : int32 [4, ld_bounds] = amin, amax, bmin, bmax; column i = step
+ *           t_begin + i.
+ * ------------------------------------------------------------------ */
+/* One read of steps [t_begin, t_end): the occupied bounds of every step. */
+int b200_dice_lattice_bounds(const void* outcomes, int64_t n_investors, int32_t horizon,
+                             int64_t ld_outcomes, int32_t t_begin, int32_t t_end,
+                             int32_t* ab_state, int32_t* bounds, int64_t ld_bounds, void* stream);
+/* One read of steps [t_begin, t_end) into hist int32 [hist_cells] (cleared first):
+ * cell (a, b) of step t_begin + i is hist[offsets[i] + (a - amin) * (bmax - bmin + 1)
+ * + (b - bmin)], bounds as b200_dice_lattice_bounds wrote them for those steps. */
+int b200_dice_lattice_count(const void* outcomes, int64_t n_investors, int32_t horizon,
+                            int64_t ld_outcomes, int32_t t_begin, int32_t t_end,
+                            int32_t* ab_state, const int32_t* bounds, int64_t ld_bounds,
+                            const int64_t* offsets, int32_t* hist, int64_t hist_cells,
+                            void* stream);
+/* The 12 statistics (b200_rowstats order and definitions, torch's non-finite rules,
+ * 1 <= top <= n_investors; top == n_investors: the adj group is NaN) of every
+ * leverage g and step t_begin + i from b200_dice_lattice_count's histogram of those
+ * steps: the wealth of cell (a, b) is fl32(exp(log_v0 + a log u + b log d + c log m)),
+ * evaluated in fp64 left to right; exact ranks by a select on that log value weighted
+ * by the counts, fp64 moments summed in an order fixed by the step's box alone.
+ * logs_host : HOST double [G,3] = (log u, log d, log m) of each leverage (G <= B200_MAX_GRID).
+ * stats     : double [G, n_steps, 12].
+ * fails     : int32 [G], NOT cleared: += the steps at which leverage g fails the
+ *             route rule - the min or the max of the log value over the step's occupied
+ *             cells not strictly inside (log FLT_MIN, log FLT_MAX) with a margin of 1e-3,
+ *             a log that is not finite, or a select that cannot finish exactly (that
+ *             step's statistics are then NaN).  Only a leverage that never fails may take
+ *             the lattice's statistics. */
+int b200_dice_lattice_stats(const int32_t* hist, const int32_t* bounds, int64_t ld_bounds,
+                            const int64_t* offsets, int32_t t_begin, int32_t n_steps,
+                            const double* logs_host, int32_t n_grid, double log_v0,
+                            int64_t n_investors, int64_t top, double* stats, int32_t* fails,
+                            void* stream);
+
+/* ------------------------------------------------------------------ *
  * Per-step series of GBM from the running log-return sum
  *
  * Sits behind gbm_smart_lev (lev/lev_exp.py:1012-1120) when the caller opts in

@@ -252,6 +252,10 @@ _SIGNATURES = {
     "b200_coin_lattice_count": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _i32, _i32, _vp, _vp, _i64, _vp, _vp, _vp]),
     "b200_coin_lattice_stats": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, C.POINTER(C.c_double), _i32, C.c_double,
                                           _i32, _i64, _i64, _vp, _vp, _vp]),
+    "b200_dice_lattice_bounds": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _i32, _vp, _vp, _i64, _vp]),
+    "b200_dice_lattice_count": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _i32, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
+    "b200_dice_lattice_stats": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _i32, C.POINTER(C.c_double), _i32, C.c_double,
+                                          _i64, _i64, _vp, _vp, _vp]),
     "b200_gbm_sum_chunk": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _i32, _i32, _vp, _vp, _i64, _vp]),
     "b200_gbm_sum_stats_workspace_bytes": (_i64, [_i64, _i64, _i32]),
     "b200_gbm_sum_stats": (C.c_int, [_vp, _i64, _i64, _i64, C.POINTER(C.c_double), _i32, C.c_double, _i32, _i64,

@@ -431,6 +431,8 @@ def lev_series(
     up-move count lattice - coin_series_counts; `chunk_steps` is then its histogram chunk.
     method="sum": GBM (streamed log-returns, one GPU) from the running log-return sum -
     gbm_series_sum; `chunk_steps` is then its S chunk.
+    method="tuples": the three-outcome gamble (factors [G,3], streamed uint8 codes, fp32, one GPU) from the
+    count-tuple lattice - dice_series_tuples, with its default histogram chunk.
     """
     if method == "counts":
         f = np.asarray(factors)
@@ -447,8 +449,18 @@ def lev_series(
             raise ValueError('method="sum" runs on one GPU')
         data, data_T, _ = gbm_series_sum(factors, lev_row, value_0, top, outcomes, dtype=dtype, chunk_steps=chunk_steps)
         return data, data_T
+    if method == "tuples":
+        f = np.asarray(factors)
+        if kind != "discrete" or f.ndim != 2 or f.shape[1] != 3 or not isinstance(outcomes, torch.Tensor):
+            raise ValueError('method="tuples" is the three-outcome discrete gamble\'s, from streamed uint8 codes')
+        if dtype != torch.float32:
+            raise ValueError('method="tuples" runs in float32')
+        if group is not None or (n_total is not None and int(n_total) != outcomes.shape[0]):
+            raise ValueError('method="tuples" runs on one GPU')
+        data, data_T, _ = dice_series_tuples(f, lev_row, value_0, top, outcomes)
+        return data, data_T
     if method != "chain":
-        raise ValueError("method must be 'chain', 'counts' or 'sum'")
+        raise ValueError("method must be 'chain', 'counts', 'sum' or 'tuples'")
     if dtype == torch.float64:
         if group is not None:
             raise ValueError("float64 sweeps are single-GPU")
@@ -735,6 +747,195 @@ def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: tor
             data[torch.as_tensor(rest, device=dev)] = sub
         if h > 1:
             data[:, :12, h - 2] = last
+    return data, data_T, routed
+
+
+def _dice_codes(outcomes) -> None:
+    if not isinstance(outcomes, torch.Tensor) or not outcomes.is_cuda or outcomes.dtype != torch.uint8 \
+            or outcomes.dim() != 2 or outcomes.stride(1) != 1:
+        raise ValueError("outcomes must be a [N,H] uint8 CUDA tensor with unit inner stride (engine.encode_codes)")
+
+
+def _dice_ld(outcomes: torch.Tensor) -> int:
+    return outcomes.stride(0) if outcomes.shape[0] > 1 else outcomes.shape[1]
+
+
+def dice_lattice_bounds(outcomes: torch.Tensor, t_begin: int, t_end: int, ab_state: torch.Tensor, *,
+                        bounds: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """
+    Steps [t_begin, t_end) of a three-outcome gamble's count-tuple lattice (b200_dice_lattice_bounds): one read
+    of the uint8 codes [N,H] (0 up, 1 down, 2 mid) into the occupied bounds int32 [4, t_end - t_begin] = (amin,
+    amax, bmin, bmax) of every step, a = up-moves and b = down-moves in steps 0..t.  ab_state int32 [2,N] carries
+    each investor's (a, b) from one call to the next (read when t_begin > 0, updated in place).  `bounds` may be
+    passed to reuse a buffer ([4, >= steps]).  Returns a view of exactly t_end - t_begin columns.
+    """
+    require_cuda()
+    _dice_codes(outcomes)
+    n, h = outcomes.shape
+    steps = int(t_end) - int(t_begin)
+    if tuple(ab_state.shape) != (2, n) or ab_state.dtype != torch.int32 or not ab_state.is_contiguous():
+        raise ValueError("ab_state must be a contiguous int32 [2,N] tensor")
+    with torch.cuda.device(outcomes.device):
+        if bounds is None:
+            bounds = torch.empty((4, max(steps, 1)), dtype=torch.int32, device=outcomes.device)
+        if bounds.dim() != 2 or bounds.shape[0] != 4 or bounds.shape[1] < steps or bounds.dtype != torch.int32 \
+                or bounds.stride(1) != 1:
+            raise ValueError("bounds must be int32 [4, >= steps] with unit inner stride")
+        check(lib.b200_dice_lattice_bounds(ptr(outcomes), n, h, _dice_ld(outcomes), int(t_begin), int(t_end),
+                                           ptr(ab_state), ptr(bounds), bounds.stride(0), stream_ptr()))
+    return bounds[:, :steps]
+
+
+def dice_lattice_plan(bounds: np.ndarray, chunk_bytes: int):
+    """
+    The flat layout of the steps' boxes (host): bounds [4,T] = (amin, amax, bmin, bmax) of steps t0 .. t0 + T - 1
+    -> (offsets int64 [T], chunks [(i0, i1, cells)]): the steps i0 .. i1 - 1 of a chunk hold `cells` int32 cells
+    in all, at most chunk_bytes, and step i's box [amax-amin+1][bmax-bmin+1] starts at offsets[i] of its chunk.
+    None when one step's box alone exceeds chunk_bytes.
+    """
+    b = np.asarray(bounds, dtype=np.int64)
+    area = (b[1] - b[0] + 1) * (b[3] - b[2] + 1)
+    budget = min(int(chunk_bytes) // 4, 2 ** 31 - 1)
+    if area.size == 0 or area.max() > budget:
+        return None
+    offsets = np.empty(area.size, dtype=np.int64)
+    chunks = []
+    i0, cells = 0, 0
+    for i, c in enumerate(area.tolist()):
+        if cells + c > budget:
+            chunks.append((i0, i, cells))
+            i0, cells = i, 0
+        offsets[i] = cells
+        cells += c
+    chunks.append((i0, area.size, cells))
+    return offsets, chunks
+
+
+def dice_lattice_count(outcomes: torch.Tensor, t_begin: int, t_end: int, ab_state: torch.Tensor,
+                       bounds: torch.Tensor, offsets: torch.Tensor, cells: int, *,
+                       hist: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """
+    Steps [t_begin, t_end) of the count-tuple lattice (b200_dice_lattice_count): a second read of the codes into
+    hist int32 [cells], cell (a, b) of step t_begin + i at offsets[i] + (a - amin) * (bmax - bmin + 1) + (b - bmin).
+    bounds int32 [4, >= steps] and offsets int64 [>= steps] (CUDA) describe those steps (column 0 = t_begin), as
+    dice_lattice_bounds and dice_lattice_plan give them; ab_state as in dice_lattice_bounds (its own copy: the
+    count walk carries its own).  Returns hist[:cells].
+    """
+    require_cuda()
+    _dice_codes(outcomes)
+    n, h = outcomes.shape
+    steps = int(t_end) - int(t_begin)
+    if tuple(ab_state.shape) != (2, n) or ab_state.dtype != torch.int32 or not ab_state.is_contiguous():
+        raise ValueError("ab_state must be a contiguous int32 [2,N] tensor")
+    if bounds.dtype != torch.int32 or bounds.shape[0] != 4 or bounds.shape[1] < steps or bounds.stride(1) != 1 \
+            or offsets.dtype != torch.int64 or offsets.shape[0] < steps or offsets.stride(0) != 1:
+        raise ValueError("bounds must be int32 [4, >= steps] and offsets int64 [>= steps], unit inner stride")
+    with torch.cuda.device(outcomes.device):
+        if hist is None:
+            hist = torch.empty(max(int(cells), 1), dtype=torch.int32, device=outcomes.device)
+        if hist.dtype != torch.int32 or hist.numel() < cells or not hist.is_contiguous():
+            raise ValueError("hist must be a contiguous int32 tensor of >= cells elements")
+        check(lib.b200_dice_lattice_count(ptr(outcomes), n, h, _dice_ld(outcomes), int(t_begin), int(t_end),
+                                          ptr(ab_state), ptr(bounds), bounds.stride(0), ptr(offsets), ptr(hist),
+                                          int(cells), stream_ptr()))
+    return hist[:cells]
+
+
+def dice_lattice_logs(factors, value_0: float):
+    """(log V0, logs [G,3] = (log u, log d, log m)) of the fp32 factor table [G,3] (columns = codes 0 up, 1 down,
+    2 mid) and the fp32 V0; nan for a factor <= 0 (such a leverage never takes the lattice)."""
+    f = np.asarray(factors, dtype=np.float32).astype(np.float64)
+    logs = np.array([[math.log(x) if x > 0 else math.nan for x in row] for row in f], dtype=np.float64)
+    return math.log(float(np.float32(value_0))), np.ascontiguousarray(logs.reshape(-1, 3))
+
+
+def dice_lattice_stats(hist: torch.Tensor, bounds: torch.Tensor, offsets: torch.Tensor, t_begin: int, factors,
+                       value_0: float, top: int, n_investors: int, *, fails: Optional[torch.Tensor] = None):
+    """
+    The 12 statistics (rowstats' order and definitions) of every leverage at steps t_begin .. t_begin + T - 1
+    (T = bounds.shape[1]) from dice_lattice_count's histogram of those steps (b200_dice_lattice_stats): float64
+    [G, T, 12] of the fp32 wealth fl32(exp(log V0 + a log u + b log d + c log m)).  `fails` int32 [G] (created
+    zeroed when None) is incremented at every step where a leverage fails the route rule (the extreme occupied
+    cells outside fp32's normal range, or a select that cannot finish exactly); returns (stats, fails).
+    """
+    require_cuda()
+    lv0, logs = dice_lattice_logs(factors, value_0)
+    g = logs.shape[0]
+    steps = bounds.shape[1]
+    dev = hist.device
+    with torch.cuda.device(dev):
+        if fails is None:
+            fails = torch.zeros(g, dtype=torch.int32, device=dev)
+        stats = torch.empty((g, steps, 12), dtype=torch.float64, device=dev)
+        check(lib.b200_dice_lattice_stats(ptr(hist), ptr(bounds), bounds.stride(0), ptr(offsets), int(t_begin), steps,
+                                          logs.ctypes.data_as(C.POINTER(C.c_double)), g, lv0, int(n_investors),
+                                          int(top), ptr(stats), ptr(fails), stream_ptr()))
+    return stats, fails
+
+
+def dice_series_tuples(factors, lev_row, value_0: float, top: int, outcomes: torch.Tensor, *,
+                       chunk_bytes: int = 256 << 20):
+    """
+    lev_series of the three-outcome gamble (factors fp32 [G,3], columns = codes 0 up, 1 down, 2 mid; uint8 codes
+    [N,H] on the GPU) from the count-tuple lattice: returns (data [G,13,H-1] fp32, data_T [G,N] fp32, routed bool
+    [G]) with lev_series' layout.
+
+    Wealth after step t is V0 u^a d^b m^(t+1-a-b), so every leverage's statistics at step t follow from one
+    histogram over the occupied (a, b) cells instead of a dump of every investor's wealth: one read of the codes
+    for every step's bounds (dice_lattice_bounds), a flat layout of the steps' boxes in chunks of at most
+    `chunk_bytes` (dice_lattice_plan), then per chunk a second read into the histogram (dice_lattice_count) and
+    the statistics (dice_lattice_stats).  A leverage is routed - its columns 0..H-3 come from the lattice - when
+    its factors are > 0 and, at every step, the occupied cells' log wealth stays inside fp32's normal range (the
+    chain saturates path by path, the closed form does not) and the select finished exactly; the others take
+    lev_series on their sub-grid.  When one step's box alone exceeds `chunk_bytes`, or H <= 2, nothing is routed.
+    data_T of every leverage is the exact chain (lev_sweep "chain") and the last column is its row statistics:
+    both are bit-identical to lev_series'.
+    """
+    require_cuda()
+    f = np.ascontiguousarray(factors, dtype=np.float32)
+    if f.ndim != 2 or f.shape[1] != 3:
+        raise ValueError("the count-tuple lattice is the three-outcome gamble's: factors [G,3] = (up, down, mid)")
+    _dice_codes(outcomes)
+    lev_row = np.asarray(lev_row, dtype=np.float32)
+    g = f.shape[0]
+    n, h = outcomes.shape
+    dev = outcomes.device
+    routed = np.zeros(g, dtype=bool)
+    if n == 0 or h <= 2:
+        data, data_T = lev_series("discrete", f, lev_row, value_0, top, outcomes=outcomes)
+        return data, data_T, routed
+
+    with torch.cuda.device(dev):
+        data_T = lev_sweep("discrete", f, value_0, outcomes=outcomes, mode="chain")["data_T"]
+        last = stats_to_reference_dtype(rowstats(data_T, top), n, top)
+        data = torch.zeros((g, 13, h - 1), dtype=torch.float32, device=dev)
+        data[:, 12, :] = torch.as_tensor(lev_row, device=dev)[:, None]
+        lat = np.flatnonzero((f > 0).all(axis=1))
+        plan = None
+        if lat.size:
+            ab = torch.empty((2, n), dtype=torch.int32, device=dev)
+            bounds = dice_lattice_bounds(outcomes, 0, h, ab)
+            plan = dice_lattice_plan(bounds.cpu().numpy(), chunk_bytes)
+        if plan is not None:
+            offsets, chunks = plan
+            off_dev = torch.as_tensor(offsets, device=dev)
+            hist = torch.empty(max(c for _, _, c in chunks), dtype=torch.int32, device=dev)
+            fails = torch.zeros(lat.size, dtype=torch.int32, device=dev)
+            sel = torch.as_tensor(lat, device=dev)
+            for t0, t1, cells in chunks:      # every step: a saturation at any step decides the route
+                hs = dice_lattice_count(outcomes, t0, t1, ab, bounds[:, t0:t1], off_dev[t0:t1], cells, hist=hist)
+                st, _ = dice_lattice_stats(hs, bounds[:, t0:t1], off_dev[t0:t1], t0, f[lat], value_0, top, n,
+                                           fails=fails)
+                c0, c1 = max(t0, 1), min(t1, h - 1)      # steps 1..H-2 -> columns 0..H-3
+                if c1 > c0:
+                    data[sel, :12, c0 - 1:c1 - 1] = stats_to_reference_dtype(st[:, c0 - t0:c1 - t0], n,
+                                                                             top).permute(0, 2, 1)
+            routed[lat] = fails.cpu().numpy() == 0
+        rest = np.flatnonzero(~routed)
+        if rest.size:
+            sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes)
+            data[torch.as_tensor(rest, device=dev)] = sub
+        data[:, :12, h - 2] = last
     return data, data_T, routed
 
 

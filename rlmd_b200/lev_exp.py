@@ -360,9 +360,10 @@ class series_method:
     `with lev_exp.series_method("counts"):` - inside the block coin_smart_lev computes its per-step statistics
     from the up-move count lattice (engine.coin_series_counts) unless a call passes `method` itself, so an
     unmodified script that reaches this module through sys.modules opts in without a change.  "sum" does the
-    same for gbm_smart_lev (the running log-return sum, engine.gbm_series_sum).  Each function takes the
-    innermost block's method only when it is its own ("counts" for the coin, "sum" for GBM) and "chain"
-    otherwise.  "chain" (the default outside any block) is the reference's sequential product for every
+    same for gbm_smart_lev (the running log-return sum, engine.gbm_series_sum), "tuples" for dice_smart_lev and
+    dice_sh_smart_lev (the count-tuple lattice, engine.dice_series_tuples).  Each function takes the innermost
+    block's method only when it is its own ("counts" for the coin, "sum" for GBM, "tuples" for the dice) and
+    "chain" otherwise.  "chain" (the default outside any block) is the reference's sequential product for every
     column.  Blocks nest.
     """
 
@@ -379,8 +380,8 @@ class series_method:
 
 
 def _series_method(method) -> str:
-    if method not in ("chain", "counts", "sum"):
-        raise ValueError("method must be 'chain', 'counts' or 'sum'")
+    if method not in ("chain", "counts", "sum", "tuples"):
+        raise ValueError("method must be 'chain', 'counts', 'sum' or 'tuples'")
     return method
 
 
@@ -421,22 +422,38 @@ def coin_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, dow
     return data, data_T
 
 
+def _dice_method(method) -> str:
+    method = _call_method(method, "tuples")
+    if method == "tuples" and _GROUP is not None:
+        raise ValueError('method="tuples" runs on one GPU: call set_process_group(None) or use method="chain"')
+    return method
+
+
 def dice_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, down_r, mid_r, lev_low, lev_high,
-                   lev_incr):
-    """lev/lev_exp.py:586-701."""
+                   lev_incr, *, method=None):
+    """lev/lev_exp.py:586-701.
+
+    method "chain" (default; see series_method): the exact sequential product for every column.  "tuples": the
+    columns of every leverage whose occupied cells stay inside fp32's normal range come from the count-tuple
+    lattice (engine.dice_series_tuples: the same statistics of the closed-form wealth V0 u^a d^b m^c, within
+    rounding of the chain's, without a pass over every investor's wealth per step); data_T, the last column and
+    the printed text are the chain's, bit for bit.  One GPU: ValueError under set_process_group."""
+    method = _dice_method(method)
     lev = _grid(lev_low, lev_high, lev_incr, up_r, down_r)
     data, data_T = _series("discrete", _codes(outcomes, 3, device), dice_factor_table(lev, up_r, down_r, mid_r), lev, investors,
-                           horizon, top, value_0)
+                           horizon, top, value_0, method=method)
     _print_final(lev, data[:, :12, -1].double().cpu().numpy())
     return data, data_T
 
 
 def dice_sh_smart_lev(device, outcomes, investors, horizon, top, value_0, up_r, down_r, mid_r, sh_up_r, sh_down_r,
-                      sh_mid_r, lev_low, lev_high, lev_incr):
-    """lev/lev_exp.py:1209-1334."""
+                      sh_mid_r, lev_low, lev_high, lev_incr, *, method=None):
+    """lev/lev_exp.py:1209-1334.  method: as dice_smart_lev's ("chain" or "tuples")."""
+    method = _dice_method(method)
     lev = _grid(lev_low, lev_high, lev_incr, up_r, down_r)
     table = dice_sh_factor_table(lev, up_r, down_r, mid_r, sh_up_r, sh_down_r, sh_mid_r)
-    data, data_T = _series("discrete", _codes(outcomes, 3, device), table, lev, investors, horizon, top, value_0)
+    data, data_T = _series("discrete", _codes(outcomes, 3, device), table, lev, investors, horizon, top, value_0,
+                           method=method)
     _print_final(lev, data[:, :12, -1].double().cpu().numpy())
     return data, data_T
 

@@ -126,8 +126,9 @@ def coin_flip(path_results: Optional[str] = "./results/multiverse/", *, seed: in
 
 @_reusing_codes
 def dice_roll(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
-              **overrides) -> Dict[str, np.ndarray]:
-    """lev/dice_roll.py:143-218 -> dice_inv1_val[_T], dice_inv2_val, dice_inv3_val."""
+              series: str = "chain", **overrides) -> Dict[str, np.ndarray]:
+    """lev/dice_roll.py:143-218 -> dice_inv1_val[_T], dice_inv2_val, dice_inv3_val.
+    series: dice_smart_lev's method ("chain" or "tuples", the count-tuple lattice)."""
     c = _cfg(DICE, overrides)
     dev = T.device("cuda")
     t0 = time.perf_counter()
@@ -139,7 +140,7 @@ def dice_roll(path_results: Optional[str] = "./results/multiverse/", *, seed: in
     lf = _lev_factor(c["up_r"], c["down_r"], c["asym_lim"])
     rets = (c["up_r"], c["down_r"], c["mid_r"])
     lev_exp.dice_fixed_final_lev(dev, outcomes, c["top"], c["value_0"], *rets, *c["l0"])
-    d, dT = lev_exp.dice_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], *rets, *c["l1"])
+    d, dT = lev_exp.dice_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], *rets, *c["l1"], method=series)
     _save(path_results, "dice_inv1_val", d, out)
     _save(path_results, "dice_inv1_val_T", dT, out)
     for tag, s, r in (("dice_inv2_val", c["s2"], c["r2"]), ("dice_inv3_val", c["s3"], c["r3"])):
@@ -152,8 +153,9 @@ def dice_roll(path_results: Optional[str] = "./results/multiverse/", *, seed: in
 
 @_reusing_codes
 def dice_roll_sh(path_results: Optional[str] = "./results/multiverse/", *, seed: int = 420, outcomes=None,
-                 **overrides) -> Dict[str, np.ndarray]:
-    """lev/dice_roll_sh.py:122-161 -> dice_sh_inv1_val[_T]."""
+                 series: str = "chain", **overrides) -> Dict[str, np.ndarray]:
+    """lev/dice_roll_sh.py:122-161 -> dice_sh_inv1_val[_T].
+    series: dice_sh_smart_lev's method ("chain" or "tuples", the count-tuple lattice)."""
     c = _cfg(DICE_SH, overrides)
     dev = T.device("cuda")
     t0 = time.perf_counter()
@@ -164,7 +166,7 @@ def dice_roll_sh(path_results: Optional[str] = "./results/multiverse/", *, seed:
     out: Dict[str, np.ndarray] = {}
     rets = (c["up_r"], c["down_r"], c["mid_r"], c["sh_up_r"], c["sh_down_r"], c["sh_mid_r"])
     lev_exp.dice_sh_fixed_final_lev(dev, outcomes, c["top"], c["value_0"], *rets, *c["l0"])
-    d, dT = lev_exp.dice_sh_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], *rets, *c["l1"])
+    d, dT = lev_exp.dice_sh_smart_lev(dev, outcomes, n, h, c["top"], c["value_0"], *rets, *c["l1"], method=series)
     _save(path_results, "dice_sh_inv1_val", d, out)
     _save(path_results, "dice_sh_inv1_val_T", dT, out)
     _report(t0)
