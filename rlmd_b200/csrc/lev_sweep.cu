@@ -9,6 +9,7 @@
 //   TMA-staged fp32 tiles, or Philox + Box-Muller draws in registers.
 // CHAIN mode kernels live in lev_kernels.cuh / lev_chain_k*.cu.
 #include <cstdlib>
+#include <type_traits>
 
 #include "lev_kernels.cuh"
 #include "tally.cuh"
@@ -248,10 +249,10 @@ log_discrete_stream_kernel(const uint8_t* __restrict__ outcomes, int64_t ld, int
 }
 
 // ------------------------------------------ LOG, discrete: packed 2-bit codes
-// Same contract as log_discrete_stream_kernel on a quarter of the bytes.  The
-// masks of a code's low / high bit occupy the even bit positions only, so the
-// masks of TWO words share one popc: per 32 codes 2 shifts, 2 LOP3, 2 POPC and
-// 2 adds (POPC issues at 16 lanes/clk/SM: ~1/3 of its rate at the HBM rate).
+// Same contract as log_discrete_stream_kernel on a quarter of the bytes.  Rows off
+// 16-byte alignment count word pairs here: the masks of a code's low / high bit
+// occupy the even bit positions only, so the masks of TWO words share one popc.
+// Aligned rows take the bit-sliced tree below.
 template <int K, int BITS = 2>
 __device__ __forceinline__ void count_pair(uint32_t a, uint32_t b, uint32_t& s1, uint32_t& s2, uint32_t& s3) {
   if (BITS == 1) { s1 += __popc(a) + __popc(b); return; }     // one bit per flip: the ones ARE the up moves
@@ -263,10 +264,80 @@ __device__ __forceinline__ void count_pair(uint32_t a, uint32_t b, uint32_t& s1,
 
 // Rows that start on a 16-byte boundary (every row of pack_codes / lev_draw) are
 // read as whole 16-byte vectors, PACKED_U per lane per iteration, all issued
-// before the first is consumed: a 1e4-step row (2500 bytes) is ONE round trip to
-// DRAM per warp.  The last vector may reach into the row's pad bytes (ld is a
-// multiple of 16 there): the lane that holds it masks the codes of steps >= H.
-constexpr int PACKED_U = 6;
+// before the first is consumed: a 1e4-step row (2500 bytes, 157 vectors) is ONE
+// round trip to DRAM per warp and fills every slot of that round.  The last vector
+// may reach into the row's pad bytes (ld is a multiple of 16 there): the lane that
+// holds it masks the codes of steps >= H.
+constexpr int PACKED_U = 5;
+
+// Bit-sliced counting of those vectors (carry-save / Harley-Seal): the words of a
+// lane's vectors go through a tree of full adders, each two LOP3s (a^b^c, maj(a,b,c)),
+// into counters c1/c2/c4/c8 that hold, bit for bit, the weight-1/2/4/8 digit of how
+// many of the lane's words have that bit set; what carries out at weight 16 is
+// POPC'd at once.  The row's sums are POPCs of the four counters at its end: the low
+// code bits sit in the even positions and the high ones in the odd positions, so one
+// tree serves n1 and n2 (and all 32 positions are flips at BITS = 1).  Per 32-bit
+// word that is ~2 LOP3s where the pairwise POPC path (count_pair) spent ~6
+// instructions; a lane's 20 words of a 1e4-step row take 12 POPCs instead of 24.
+__device__ __forceinline__ uint32_t full_add(uint32_t& acc, uint32_t a, uint32_t b) {   // acc += a + b, returns the carry
+  const uint32_t carry = (acc & a) | (acc & b) | (a & b);
+  acc ^= a ^ b;
+  return carry;
+}
+__device__ __forceinline__ uint32_t half_add(uint32_t& acc, uint32_t a) {
+  const uint32_t carry = acc & a;
+  acc ^= a;
+  return carry;
+}
+// adds N words of one weight into that weight's counter; the carries (next weight) go to out
+template <int N>
+__device__ __forceinline__ void add_level(uint32_t& acc, const uint32_t (&in)[N], uint32_t (&out)[(N + 1) / 2]) {
+#pragma unroll
+  for (int j = 0; j + 1 < N; j += 2) out[j / 2] = full_add(acc, in[j], in[j + 1]);
+  if (N & 1) out[N / 2] = half_add(acc, in[N - 1]);
+}
+
+template <int K, int BITS>
+struct SliceCounter {
+  static constexpr uint32_t EVEN = 0x55555555u;
+  uint32_t c1 = 0, c2 = 0, c4 = 0, c8 = 0;
+  uint32_t hi_e = 0, hi_t = 0;   // weight-16 carries: set bits in the even positions / in all positions
+  uint32_t s3 = 0;               // K = 4: codes 3 (low AND high bit), counted per word pair
+
+  template <int U>
+  __device__ __forceinline__ void add(const uint4 (&v)[U]) {
+    uint32_t w[4 * U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      w[4 * u] = v[u].x; w[4 * u + 1] = v[u].y; w[4 * u + 2] = v[u].z; w[4 * u + 3] = v[u].w;
+      if (K >= 4 && BITS == 2) {   // a & (a >> 1) in the even bits, b & (b << 1) in the odd bits: one POPC
+        s3 += __popc(((v[u].x & (v[u].x >> 1)) & EVEN) | ((v[u].y & (v[u].y << 1)) & ~EVEN));
+        s3 += __popc(((v[u].z & (v[u].z >> 1)) & EVEN) | ((v[u].w & (v[u].w << 1)) & ~EVEN));
+      }
+    }
+    uint32_t x2[2 * U], x4[U], x8[(U + 1) / 2], x16[(U + 3) / 4];
+    add_level(c1, w, x2);
+    add_level(c2, x2, x4);
+    add_level(c4, x4, x8);
+    add_level(c8, x8, x16);
+#pragma unroll
+    for (int j = 0; j < (U + 3) / 4; ++j) {
+      if (BITS == 2) hi_e += __popc(x16[j] & EVEN);
+      if (BITS == 1 || K >= 3) hi_t += __popc(x16[j]);
+    }
+  }
+  // this lane's sums: s1 = set low bits (all bits at BITS = 1), s2 = set high bits
+  __device__ __forceinline__ void sums(uint32_t& s1, uint32_t& s2) const {
+    if (BITS == 2)
+      s1 = __popc(c1 & EVEN) + (__popc(c2 & EVEN) << 1) + (__popc(c4 & EVEN) << 2) + (__popc(c8 & EVEN) << 3) +
+           (hi_e << 4);
+    if (BITS == 1 || K >= 3) {
+      const uint32_t t = __popc(c1) + (__popc(c2) << 1) + (__popc(c4) << 2) + (__popc(c8) << 3) + (hi_t << 4);
+      if (BITS == 1) s1 = t;
+      else s2 = t - s1;
+    }
+  }
+};
 
 template <int BITS>
 __device__ __forceinline__ uint32_t word_mask(int valid) {   // low BITS*valid bits, valid clamped to 0..32/BITS
@@ -322,102 +393,100 @@ log_discrete_packed_kernel(const uint8_t* __restrict__ outcomes, int64_t ldb, in
     if (K >= 3) s2 += __popc((c >> 1) & 0x55u);
     if (K >= 4) s3 += __popc(c & (c >> 1) & 0x55u);
   };
-  for (int64_t row0 = warp_global * task_rows; row0 < N; row0 += nwarps * task_rows) {
-    const int nr = (int)min((int64_t)task_rows, N - row0);
-    uint32_t m1 = 0, m2 = 0, m3 = 0;   // sums of row (row0 + lane)
-    for (int r = 0; r < nr; ++r) {
-      const uint8_t* __restrict__ p = outcomes + (row0 + r) * ldb;
-      uint32_t s1 = 0, s2 = 0, s3 = 0;
-      // the next row's lines start their way from DRAM to L2 while this row is counted
-      if (r + 1 < nr)
-        for (int b = lane * 128; b < nbytes; b += 32 * 128)
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(p + ldb + b));
-      if (vec_rows && (((uintptr_t)p) & 15) == 0) {
-        const uint4* __restrict__ q = reinterpret_cast<const uint4*>(p) + lane;
-        // full iterations: PACKED_U vectors per lane, no predicates
-        for (int it = 0; it + 1 < iters; ++it, q += 32 * PACKED_U) {
+  // Rows on 16-byte boundaries take the vector walk.  With ldb a multiple of 16 that is every row or none, so
+  // it is decided once and the row loop carries one path (not the other path's address arithmetic as well).
+  auto sweep = [&](auto vec) {
+    for (int64_t row0 = warp_global * task_rows; row0 < N; row0 += nwarps * task_rows) {
+      const int nr = (int)min((int64_t)task_rows, N - row0);
+      uint32_t m1 = 0, m2 = 0, m3 = 0;   // sums of row (row0 + lane)
+      for (int r = 0; r < nr; ++r) {
+        const uint8_t* __restrict__ p = outcomes + (row0 + r) * ldb;
+        uint32_t s1 = 0, s2 = 0, s3 = 0;
+        // the next row's lines start their way from DRAM to L2 while this row is counted
+        if (r + 1 < nr)
+#pragma unroll 1
+          for (int b = lane * 128; b < nbytes; b += 32 * 128)
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(p + ldb + b));
+        if constexpr (decltype(vec)::value) {
+          const uint4* __restrict__ q = reinterpret_cast<const uint4*>(p) + lane;
+          SliceCounter<K, BITS> acc;
+          // full iterations: PACKED_U vectors per lane, no predicates
+          for (int it = 0; it + 1 < iters; ++it, q += 32 * PACKED_U) {
+            uint4 v[PACKED_U];
+#pragma unroll
+            for (int u = 0; u < PACKED_U; ++u) v[u] = __ldcs(q + u * 32);
+            acc.add(v);
+          }
+          // the row's last `rem` vectors: slots below tail_slots-1 are full, slot
+          // tail_slots-1 ends at lane tail_lanes-1, whose vector reaches into the pad
+          // (everything here but the loaded data was worked out before the row loop).
+          // Slots the row does not reach enter the tree as zeros; the partly filled
+          // last slot, masked, takes the array's last place.
           uint4 v[PACKED_U];
 #pragma unroll
-          for (int u = 0; u < PACKED_U; ++u) v[u] = __ldcs(q + u * 32);
-#pragma unroll
-          for (int u = 0; u < PACKED_U; ++u) {
-            count_pair<K, BITS>(v[u].x, v[u].y, s1, s2, s3);
-            count_pair<K, BITS>(v[u].z, v[u].w, s1, s2, s3);
+          for (int u = 0; u < PACKED_U - 1; ++u)
+            v[u] = u < tail_slots - 1 ? __ldcs(q + u * 32) : make_uint4(0u, 0u, 0u, 0u);
+          uint4 vl = make_uint4(0u, 0u, 0u, 0u);
+          if (in_tail) vl = __ldcs(q + (tail_slots - 1) * 32);
+          v[PACKED_U - 1] = make_uint4(vl.x & wm.x, vl.y & wm.y, vl.z & wm.z, vl.w & wm.w);
+          acc.add(v);
+          acc.sums(s1, s2);
+          s3 = acc.s3;
+        } else {
+          // any alignment: head bytes up to 16-byte alignment, body in uint4 (full bytes only), tail bytes
+          const uintptr_t addr = (uintptr_t)p;
+          int head = (int)((16 - (addr & 15)) & 15);
+          if (head > full) head = full;
+          const int body = (full - head) >> 4;
+          const int tail0 = head + (body << 4);
+          for (int t = lane; t < head; t += 32) count_byte(t, s1, s2, s3, p);
+          const uint4* __restrict__ q = reinterpret_cast<const uint4*>(p + head);
+          for (int i = lane; i < body; i += 32) {
+            const uint4 a = __ldcs(q + i);
+            count_pair<K, BITS>(a.x, a.y, s1, s2, s3); count_pair<K, BITS>(a.z, a.w, s1, s2, s3);
           }
+          for (int t = tail0 + lane; t < nbytes; t += 32) count_byte(t, s1, s2, s3, p);
         }
-        // the row's last `rem` vectors: slots below tail_slots-1 are full, slot
-        // tail_slots-1 ends at lane tail_lanes-1, whose vector reaches into the pad
-        // (everything here but the loaded data was worked out before the row loop)
-        uint4 vl = make_uint4(0u, 0u, 0u, 0u);   // the partly filled last slot, kept apart from the array
-        if (in_tail) vl = __ldcs(q + (tail_slots - 1) * 32);
-        uint4 v[PACKED_U - 1];
+        // row sums across the warp: one REDUX per value
+        s1 = __reduce_add_sync(0xffffffffu, s1);
+        if (K >= 3) s2 = __reduce_add_sync(0xffffffffu, s2);
+        if (K >= 4) s3 = __reduce_add_sync(0xffffffffu, s3);
+        if (lane == r) { m1 = s1; m2 = s2; m3 = s3; }
+      }
+      // ---- epilogue: one row per lane
+      // Launched early (B200_LEV_FLAG_EARLY_START), the kernel has only read the outcomes so far; the table and
+      // `counts` belong to the previous kernel (the last step's statistics) until it has completed.
+      if (TALLY) pdl_wait();
+      if (lane < nr) {
+        const int64_t row = row0 + lane;
+        int n[4];
+        if (K == 2) { n[1] = (int)m1; n[0] = H - n[1]; n[2] = n[3] = 0; }
+        else if (K == 3) { n[1] = (int)m1; n[2] = (int)m2; n[0] = H - n[1] - n[2]; n[3] = 0; }
+        else { n[3] = (int)m3; n[1] = (int)(m1 - m3); n[2] = (int)(m2 - m3); n[0] = H - n[1] - n[2] - n[3]; }
+        if (counts != nullptr) {
 #pragma unroll
-        for (int u = 0; u < PACKED_U - 1; ++u)
-          if (u < tail_slots - 1) v[u] = __ldcs(q + u * 32);
-        vl.x &= wm.x; vl.y &= wm.y; vl.z &= wm.z; vl.w &= wm.w;
-        count_pair<K, BITS>(vl.x, vl.y, s1, s2, s3);
-        count_pair<K, BITS>(vl.z, vl.w, s1, s2, s3);
-#pragma unroll
-        for (int u = 0; u < PACKED_U - 1; ++u) {
-          if (u < tail_slots - 1) {
-            count_pair<K, BITS>(v[u].x, v[u].y, s1, s2, s3);
-            count_pair<K, BITS>(v[u].z, v[u].w, s1, s2, s3);
-          }
+          for (int k = 0; k < K; ++k) counts[row * K + k] = n[k];
         }
-      } else {
-        // any alignment: head bytes up to 16-byte alignment, body in uint4 (full bytes only), tail bytes
-        const uintptr_t addr = (uintptr_t)p;
-        int head = (int)((16 - (addr & 15)) & 15);
-        if (head > full) head = full;
-        const int body = (full - head) >> 4;
-        const int tail0 = head + (body << 4);
-        for (int t = lane; t < head; t += 32) count_byte(t, s1, s2, s3, p);
-        const uint4* __restrict__ q = reinterpret_cast<const uint4*>(p + head);
-        for (int i = lane; i < body; i += 32) {
-          const uint4 a = __ldcs(q + i);
-          count_pair<K, BITS>(a.x, a.y, s1, s2, s3); count_pair<K, BITS>(a.z, a.w, s1, s2, s3);
+        if (TALLY) {
+          tally_insert(tally, tally_key(n[1], n[2], n[3]), 1u);
+          continue;
         }
-        for (int t = tail0 + lane; t < nbytes; t += 32) count_byte(t, s1, s2, s3, p);
-      }
+        double nd[K];
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-        if (K >= 3) s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-        if (K >= 4) s3 += __shfl_xor_sync(0xffffffffu, s3, o);
-      }
-      if (lane == r) { m1 = s1; m2 = s2; m3 = s3; }
-    }
-    // ---- epilogue: one row per lane
-    // Launched early (B200_LEV_FLAG_EARLY_START), the kernel has only read the outcomes so far; the table and
-    // `counts` belong to the previous kernel (the last step's statistics) until it has completed.
-    if (TALLY) pdl_wait();
-    if (lane < nr) {
-      const int64_t row = row0 + lane;
-      int n[4];
-      if (K == 2) { n[1] = (int)m1; n[0] = H - n[1]; n[2] = n[3] = 0; }
-      else if (K == 3) { n[1] = (int)m1; n[2] = (int)m2; n[0] = H - n[1] - n[2]; n[3] = 0; }
-      else { n[3] = (int)m3; n[1] = (int)(m1 - m3); n[2] = (int)(m2 - m3); n[0] = H - n[1] - n[2] - n[3]; }
-      if (counts != nullptr) {
+        for (int k = 0; k < K; ++k) nd[k] = (double)n[k];
+        for (int g = 0; g < G; ++g) {
+          double lw = logV0;
 #pragma unroll
-        for (int k = 0; k < K; ++k) counts[row * K + k] = n[k];
-      }
-      if (TALLY) {
-        tally_insert(tally, tally_key(n[1], n[2], n[3]), 1u);
-        continue;
-      }
-      double nd[K];
-#pragma unroll
-      for (int k = 0; k < K; ++k) nd[k] = (double)n[k];
-      for (int g = 0; g < G; ++g) {
-        double lw = logV0;
-#pragma unroll
-        for (int k = 0; k < K; ++k)
-          if (n[k] > 0) lw += nd[k] * lf.lm[k][g];
-        if (log_w != nullptr) log_w[(int64_t)g * ldT + row] = lw;
-        if (data_T != nullptr) data_T[(int64_t)g * ldT + row] = (float)exp(lw);
+          for (int k = 0; k < K; ++k)
+            if (n[k] > 0) lw += nd[k] * lf.lm[k][g];
+          if (log_w != nullptr) log_w[(int64_t)g * ldT + row] = lw;
+          if (data_T != nullptr) data_T[(int64_t)g * ldT + row] = (float)exp(lw);
+        }
       }
     }
-  }
+  };
+  if (vec_rows && (((uintptr_t)outcomes) & 15) == 0) sweep(std::true_type());
+  else sweep(std::false_type());
 }
 
 // ----------------------------------------------------------- LOG, GBM
