@@ -677,7 +677,7 @@ def coin_lattice_stats(hist: torch.Tensor, kmin: torch.Tensor, kmax: torch.Tenso
 
 def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: torch.Tensor, *,
                        dtype: torch.dtype = torch.float32, chunk_steps: Optional[int] = None,
-                       chunk_bytes: int = 256 << 20):
+                       chunk_bytes: int = 256 << 20, group=None):
     """
     lev_series of the coin (factors [G,2] = (down, up), uint8 codes [N,H] on the GPU) from the up-move count
     lattice: returns (data [G,13,H-1], data_T [G,N], routed bool [G]) with lev_series' layout and dtype
@@ -691,18 +691,21 @@ def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: tor
     closed form does not); the others take lev_series on their sub-grid.  data_T of every leverage is the
     exact chain (lev_sweep "chain" / lev_final_f64), and the last column is its row statistics: both are
     bit-identical to lev_series'.
+
+    With `group` (a torch.distributed process group; float32 only) `outcomes` is this rank's investor shard
+    (N may be 0) and every rank returns the one-GPU result on the ranks' concatenated codes: `data` and `routed`
+    the same on every rank, `data_T` this rank's columns.  The ranks' histograms are summed (an all-reduce per
+    chunk), each rank computes the statistics of its slice of the chunk's steps and the slices are all-gathered;
+    unrouted leverages take the sharded lev_series, the last column the sharded rowstats (DESIGN.md section 6.9).
     """
     require_cuda()
+    if group is not None:
+        return _coin_series_counts_sharded(factors, lev_row, value_0, top, outcomes, dtype, chunk_steps,
+                                           chunk_bytes, group)
     if dtype not in (torch.float32, torch.float64):
         raise ValueError("dtype must be torch.float32 or torch.float64")
     fp64 = dtype == torch.float64
-    f = np.ascontiguousarray(factors, dtype=np.float64 if fp64 else np.float32)
-    if f.ndim != 2 or f.shape[1] != 2:
-        raise ValueError("the lattice is the two-outcome gamble's: factors [G,2] = (down, up)")
-    if not isinstance(outcomes, torch.Tensor) or not outcomes.is_cuda or outcomes.dtype != torch.uint8 \
-            or outcomes.dim() != 2 or outcomes.stride(1) != 1:
-        raise ValueError("outcomes must be a [N,H] uint8 CUDA tensor with unit inner stride (engine.encode_codes)")
-    lev_row = np.asarray(lev_row, dtype=np.float64 if fp64 else np.float32)
+    f, lev_row = _coin_inputs(factors, lev_row, outcomes, fp64)
     g = f.shape[0]
     n, h = outcomes.shape
     dev = outcomes.device
@@ -747,6 +750,118 @@ def coin_series_counts(factors, lev_row, value_0: float, top: int, outcomes: tor
             data[torch.as_tensor(rest, device=dev)] = sub
         if h > 1:
             data[:, :12, h - 2] = last
+    return data, data_T, routed
+
+
+def _coin_inputs(factors, lev_row, outcomes, fp64: bool):
+    """coin_series_counts' argument checks: (factors [G,2], lev_row) in the series' dtype."""
+    f = np.ascontiguousarray(factors, dtype=np.float64 if fp64 else np.float32)
+    if f.ndim != 2 or f.shape[1] != 2:
+        raise ValueError("the lattice is the two-outcome gamble's: factors [G,2] = (down, up)")
+    if not isinstance(outcomes, torch.Tensor) or not outcomes.is_cuda or outcomes.dtype != torch.uint8 \
+            or outcomes.dim() != 2 or outcomes.stride(1) != 1:
+        raise ValueError("outcomes must be a [N,H] uint8 CUDA tensor with unit inner stride (engine.encode_codes)")
+    return f, np.asarray(lev_row, dtype=np.float64 if fp64 else np.float32)
+
+
+_INT32_MAX = 2 ** 31 - 1
+
+
+def _lattice_agree(check_inputs, outcomes, sizes, group):
+    """
+    The sharded lattice series' first collective: `check_inputs()` validates this rank's arguments (returning
+    (factors, lev_row)); every rank then compares its sizes and a checksum of the factors, lev_row and V0 with
+    the others', so that a refusal or a mismatch on one rank raises ValueError on all of them.
+    Returns (factors, lev_row, device).
+    """
+    import zlib
+
+    from . import sharding
+
+    f = lev_row = None
+    refused = ""
+    try:
+        f, lev_row = check_inputs()
+    except ValueError as exc:
+        refused = str(exc)
+    dev = outcomes.device if isinstance(outcomes, torch.Tensor) and outcomes.is_cuda \
+        else torch.device("cuda", torch.cuda.current_device())
+    values = [-1] * (len(sizes) + 3)
+    if not refused:
+        values = [outcomes.shape[1], f.shape[0], zlib.crc32(f.tobytes() + lev_row.tobytes())] + list(sizes)
+    with torch.cuda.device(dev):
+        sharding.agree(values, group, dev, refused)
+    return f, lev_row, dev
+
+
+def _coin_series_counts_sharded(factors, lev_row, value_0, top, outcomes, dtype, chunk_steps, chunk_bytes, group):
+    """coin_series_counts(..., group=): see there and DESIGN.md section 6.9."""
+    import torch.distributed as dist
+
+    from . import sharding
+
+    if dtype != torch.float32:
+        raise ValueError("coin_series_counts with a process group runs in float32 (the float64 last column's row "
+                         "statistics run on one GPU)")
+    sizes = (top, -1 if chunk_steps is None else int(chunk_steps), chunk_bytes, np.float64(value_0).view(np.int64))
+    f, lev_row, dev = _lattice_agree(lambda: _coin_inputs(factors, lev_row, outcomes, False), outcomes, sizes, group)
+    g = f.shape[0]
+    n, h = outcomes.shape
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    with torch.cuda.device(dev):
+        n_total = sharding.global_count(n, group, dev)
+        if n_total == 0:        # the one-GPU call on no investors: no statistics, nothing to exchange
+            return coin_series_counts(f, lev_row, value_0, top, outcomes, chunk_steps=chunk_steps,
+                                      chunk_bytes=chunk_bytes)
+        data_T = lev_sweep("discrete", f, value_0, outcomes=outcomes, mode="chain")["data_T"]
+        last = stats_to_reference_dtype(rowstats(data_T, top, n_total=n_total, group=group), n_total, top)
+        data = torch.zeros((g, 13, max(h - 1, 0)), dtype=torch.float32, device=dev)
+        if h > 1:
+            data[:, 12, :] = torch.as_tensor(lev_row, device=dev)[:, None]
+        routed = (f > 0).all(axis=1)
+        lat = np.flatnonzero(routed)
+        if lat.size:
+            if chunk_steps is None:
+                chunk_steps = chunk_bytes // (4 * (h + 1))      # H and the budget only: every rank walks these chunks
+            tc = max(1, min(int(chunk_steps), h))
+            k_state = torch.empty(n, dtype=torch.int32, device=dev)
+            hist = torch.empty((tc, h + 1), dtype=torch.int32, device=dev)
+            kmin = torch.empty(tc, dtype=torch.int32, device=dev)
+            kmax = torch.empty(tc, dtype=torch.int32, device=dev)
+            fails = torch.zeros(lat.size, dtype=torch.int32, device=dev)
+            sel = torch.as_tensor(lat, device=dev)
+            for t0 in range(0, h, tc):
+                t1 = min(h, t0 + tc)
+                if n > 0:
+                    hs, lo, hi = coin_lattice_count(outcomes, t0, t1, k_state, hist=hist, kmin=kmin, kmax=kmax)
+                else:           # an empty shard: no counts, and a band that leaves the other ranks' as it is
+                    hs, lo, hi = hist[:t1 - t0].zero_(), kmin[:t1 - t0].fill_(_INT32_MAX), kmax[:t1 - t0].fill_(-1)
+                # the global histogram and band: exactly the one-GPU count of the concatenated codes
+                dist.all_reduce(hs, group=group)
+                dist.all_reduce(lo, op=dist.ReduceOp.MIN, group=group)
+                dist.all_reduce(hi, op=dist.ReduceOp.MAX, group=group)
+                s0, cnt = sharding.shard_range(t1 - t0, world, rank)        # this rank's slice of the steps
+                if cnt:
+                    mine, _ = coin_lattice_stats(hs[s0:s0 + cnt], lo[s0:s0 + cnt], hi[s0:s0 + cnt], t0 + s0, f[lat],
+                                                 value_0, top, n_total, fails=fails)
+                else:
+                    mine = torch.empty((lat.size, 0, 12), dtype=torch.float64, device=dev)
+                st = sharding.gather_steps(mine, t1 - t0, group)
+                c0, c1 = max(t0, 1), min(t1, h - 1)      # steps 1..H-2 -> columns 0..H-3
+                if c1 > c0:
+                    data[sel, :12, c0 - 1:c1 - 1] = stats_to_reference_dtype(st[:, c0 - t0:c1 - t0], n_total,
+                                                                             top).permute(0, 2, 1)
+            dist.all_reduce(fails, group=group)          # each rank counted the route failures of its steps
+            routed[lat] = fails.cpu().numpy() == 0
+        rest = np.flatnonzero(~routed)
+        if rest.size:
+            sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes, n_total=n_total,
+                                group=group)
+            data[torch.as_tensor(rest, device=dev)] = sub
+        if h > 1:
+            data[:, :12, h - 2] = last
+        torch.cuda.current_stream().synchronize()
+        sharding.raise_if_peers_timed_out(group, dev)
     return data, data_T, routed
 
 
@@ -874,7 +989,7 @@ def dice_lattice_stats(hist: torch.Tensor, bounds: torch.Tensor, offsets: torch.
 
 
 def dice_series_tuples(factors, lev_row, value_0: float, top: int, outcomes: torch.Tensor, *,
-                       chunk_bytes: int = 256 << 20):
+                       chunk_bytes: int = 256 << 20, group=None):
     """
     lev_series of the three-outcome gamble (factors fp32 [G,3], columns = codes 0 up, 1 down, 2 mid; uint8 codes
     [N,H] on the GPU) from the count-tuple lattice: returns (data [G,13,H-1] fp32, data_T [G,N] fp32, routed bool
@@ -890,13 +1005,18 @@ def dice_series_tuples(factors, lev_row, value_0: float, top: int, outcomes: tor
     lev_series on their sub-grid.  When one step's box alone exceeds `chunk_bytes`, or H <= 2, nothing is routed.
     data_T of every leverage is the exact chain (lev_sweep "chain") and the last column is its row statistics:
     both are bit-identical to lev_series'.
+
+    With `group` (a torch.distributed process group) `outcomes` is this rank's investor shard (N may be 0) and
+    every rank returns the one-GPU result on the ranks' concatenated codes: `data` and `routed` the same on every
+    rank, `data_T` this rank's columns.  The ranks' bounds are reduced before the plan and their histograms
+    summed per chunk; each rank computes the statistics of its slice of the chunk's steps and the slices are
+    all-gathered; unrouted leverages take the sharded lev_series, the last column the sharded rowstats
+    (DESIGN.md section 6.11).
     """
     require_cuda()
-    f = np.ascontiguousarray(factors, dtype=np.float32)
-    if f.ndim != 2 or f.shape[1] != 3:
-        raise ValueError("the count-tuple lattice is the three-outcome gamble's: factors [G,3] = (up, down, mid)")
-    _dice_codes(outcomes)
-    lev_row = np.asarray(lev_row, dtype=np.float32)
+    if group is not None:
+        return _dice_series_tuples_sharded(factors, lev_row, value_0, top, outcomes, chunk_bytes, group)
+    f, lev_row = _dice_inputs(factors, lev_row, outcomes)
     g = f.shape[0]
     n, h = outcomes.shape
     dev = outcomes.device
@@ -936,6 +1056,91 @@ def dice_series_tuples(factors, lev_row, value_0: float, top: int, outcomes: tor
             sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes)
             data[torch.as_tensor(rest, device=dev)] = sub
         data[:, :12, h - 2] = last
+    return data, data_T, routed
+
+
+def _dice_inputs(factors, lev_row, outcomes):
+    """dice_series_tuples' argument checks: (factors fp32 [G,3], lev_row fp32)."""
+    f = np.ascontiguousarray(factors, dtype=np.float32)
+    if f.ndim != 2 or f.shape[1] != 3:
+        raise ValueError("the count-tuple lattice is the three-outcome gamble's: factors [G,3] = (up, down, mid)")
+    _dice_codes(outcomes)
+    return f, np.asarray(lev_row, dtype=np.float32)
+
+
+def _dice_series_tuples_sharded(factors, lev_row, value_0, top, outcomes, chunk_bytes, group):
+    """dice_series_tuples(..., group=): see there and DESIGN.md section 6.11."""
+    import torch.distributed as dist
+
+    from . import sharding
+
+    sizes = (top, chunk_bytes, np.float64(value_0).view(np.int64))
+    f, lev_row, dev = _lattice_agree(lambda: _dice_inputs(factors, lev_row, outcomes), outcomes, sizes, group)
+    g = f.shape[0]
+    n, h = outcomes.shape
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    routed = np.zeros(g, dtype=bool)
+    with torch.cuda.device(dev):
+        n_total = sharding.global_count(n, group, dev)
+        if n_total == 0:        # the one-GPU call on no investors: no statistics, nothing to exchange
+            return dice_series_tuples(f, lev_row, value_0, top, outcomes, chunk_bytes=chunk_bytes)
+        if h <= 2:
+            data, data_T = lev_series("discrete", f, lev_row, value_0, top, outcomes=outcomes, n_total=n_total,
+                                      group=group)
+            return data, data_T, routed
+        data_T = lev_sweep("discrete", f, value_0, outcomes=outcomes, mode="chain")["data_T"]
+        last = stats_to_reference_dtype(rowstats(data_T, top, n_total=n_total, group=group), n_total, top)
+        data = torch.zeros((g, 13, h - 1), dtype=torch.float32, device=dev)
+        data[:, 12, :] = torch.as_tensor(lev_row, device=dev)[:, None]
+        lat = np.flatnonzero((f > 0).all(axis=1))
+        plan = None
+        if lat.size:
+            ab = torch.empty((2, n), dtype=torch.int32, device=dev)
+            if n > 0:
+                bounds = dice_lattice_bounds(outcomes, 0, h, ab)
+            else:               # an empty shard: bounds that leave the other ranks' as they are
+                bounds = torch.tensor([[_INT32_MAX], [-1], [_INT32_MAX], [-1]], dtype=torch.int32,
+                                      device=dev).expand(4, h)
+            # the global box of every step (each rank's cells lie inside it): the same plan on every rank
+            lo, hi = bounds[0::2].contiguous(), bounds[1::2].contiguous()
+            dist.all_reduce(lo, op=dist.ReduceOp.MIN, group=group)
+            dist.all_reduce(hi, op=dist.ReduceOp.MAX, group=group)
+            bounds = torch.stack([lo[0], hi[0], lo[1], hi[1]])
+            plan = dice_lattice_plan(bounds.cpu().numpy(), chunk_bytes)
+        if plan is not None:
+            offsets, chunks = plan
+            off_dev = torch.as_tensor(offsets, device=dev)
+            hist = torch.empty(max(c for _, _, c in chunks), dtype=torch.int32, device=dev)
+            fails = torch.zeros(lat.size, dtype=torch.int32, device=dev)
+            sel = torch.as_tensor(lat, device=dev)
+            for t0, t1, cells in chunks:
+                if n > 0:
+                    hs = dice_lattice_count(outcomes, t0, t1, ab, bounds[:, t0:t1], off_dev[t0:t1], cells, hist=hist)
+                else:
+                    hs = hist[:cells].zero_()
+                dist.all_reduce(hs, group=group)        # exactly the one-GPU histogram of the concatenated codes
+                s0, cnt = sharding.shard_range(t1 - t0, world, rank)        # this rank's slice of the steps
+                a = t0 + s0
+                if cnt:
+                    mine, _ = dice_lattice_stats(hs, bounds[:, a:a + cnt], off_dev[a:a + cnt], a, f[lat], value_0, top,
+                                                 n_total, fails=fails)
+                else:
+                    mine = torch.empty((lat.size, 0, 12), dtype=torch.float64, device=dev)
+                st = sharding.gather_steps(mine, t1 - t0, group)
+                c0, c1 = max(t0, 1), min(t1, h - 1)      # steps 1..H-2 -> columns 0..H-3
+                if c1 > c0:
+                    data[sel, :12, c0 - 1:c1 - 1] = stats_to_reference_dtype(st[:, c0 - t0:c1 - t0], n_total,
+                                                                             top).permute(0, 2, 1)
+            dist.all_reduce(fails, group=group)          # each rank counted the route failures of its steps
+            routed[lat] = fails.cpu().numpy() == 0
+        rest = np.flatnonzero(~routed)
+        if rest.size:
+            sub, _ = lev_series("discrete", f[rest], lev_row[rest], value_0, top, outcomes=outcomes, n_total=n_total,
+                                group=group)
+            data[torch.as_tensor(rest, device=dev)] = sub
+        data[:, :12, h - 2] = last
+        torch.cuda.current_stream().synchronize()
+        sharding.raise_if_peers_timed_out(group, dev)
     return data, data_T, routed
 
 

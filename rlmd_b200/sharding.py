@@ -4,7 +4,9 @@ by INVESTOR - one process per GPU, every rank holds the whole leverage grid and 
 contiguous block of investor rows, Philox counters carry the global investor id -
 so there is no data-path collective.  The only exchange is inside the
 cross-investor statistics: after each pass of b200_rowstats the per-row partial
-sums and radix histograms named by b200_rowstats_exchange are summed over ranks.
+sums and radix histograms named by b200_rowstats_exchange are summed over ranks
+(and, for the count-lattice series, the integer histograms themselves: `agree`
+and `gather_steps` are that walk's helpers - engine.coin_series_counts).
 
 Nothing here launches a kernel, so the module is exercised on CPU with the gloo
 backend (tests/test_sharding_gloo.py) as well as with NCCL on the GPUs.
@@ -46,6 +48,44 @@ def global_count(n_local: int, group, device) -> int:
     t = torch.tensor([int(n_local)], dtype=torch.int64, device=device)
     dist.all_reduce(t, group=group)
     return int(t.item())
+
+
+def agree(values, group, device, refused: str = "") -> None:
+    """
+    Collective check that every rank of `group` called with the same `values` (integers: sizes, flags, checksums
+    of the arguments).  `refused` is this rank's own ValueError message when its local inputs failed validation;
+    it still takes part, so that every rank raises together instead of one waiting in a later collective.
+    """
+    import torch.distributed as dist
+
+    v = torch.tensor([0 if refused else 1] + [int(x) for x in values], dtype=torch.int64, device=device)
+    both = torch.cat([v, -v])            # one MAX all-reduce: the maxima, then minus the minima
+    dist.all_reduce(both, op=dist.ReduceOp.MAX, group=group)
+    hi, lo = both[:v.numel()].tolist(), (-both[v.numel():]).tolist()
+    if refused:
+        raise ValueError(refused)
+    if lo[0] == 0:
+        raise ValueError("rlmd_b200: another rank's inputs were refused (see that rank's error)")
+    if hi != lo:
+        raise ValueError("rlmd_b200: the ranks disagree on the call's shape or arguments (horizon, grid, top, "
+                         "factors, chunking)")
+
+
+def gather_steps(block: torch.Tensor, steps: int, group) -> torch.Tensor:
+    """
+    The all-gather of per-step results split by shard_range over the steps: `block` [G, count, ...] holds this
+    rank's steps; returns [G, steps, ...] of every rank's blocks in rank order (identical on every rank).
+    The blocks travel padded to the largest count.
+    """
+    import torch.distributed as dist
+
+    world = dist.get_world_size(group)
+    per = (steps + world - 1) // world
+    pad = block.new_zeros((block.shape[0], per) + tuple(block.shape[2:]))
+    pad[:, :block.shape[1]] = block
+    parts = [torch.empty_like(pad) for _ in range(world)]
+    dist.all_gather(parts, pad, group=group)
+    return torch.cat([p[:, :shard_range(steps, world, r)[1]] for r, p in enumerate(parts)], dim=1)
 
 
 class PeerWorkspace:
